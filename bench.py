@@ -22,6 +22,12 @@ GPUs (strong scaling), device-timed and end to end.
 `--impl reference` times the reference alone on the host cores (rank 0 only): exactly --warmup + --steps steps, each
 step a bounded sample of the workload sized from a calibration run so the whole command takes a few minutes; the
 line reports the sample, the steps actually run and the measured ms per (sample) step, with "impl": "reference".
+
+`--dump-outputs DIR` (our arm, rank 0) writes what the last timed step returned to its caller as DIR/<name>.npy, so
+that two builds can be compared output for output on the same seeded inputs: `out.npy` (float32) for a solve;
+`loss.npy`, `grad_lmbda.npy`, `grad_rho.npy` for the cfg4 training step.  An output larger than 64 MB is stored as a
+fixed sample of 8 Mi elements (flat indices drawn with torch.Generator seed 0, sorted; the same for every run with
+the same arguments).
 """
 from __future__ import annotations
 
@@ -81,6 +87,26 @@ def make_inputs_torch(shape, kind, k, sigma, seed=1234):
     blurred = torch.fft.irfft2(torch.fft.rfft2(sharp) * torch.fft.rfft2(pad), s=(H, W))
     blurred = torch.roll(blurred, (-s, -s), dims=(-2, -1)) + 0.01 * torch.randn(B, C, H, W, generator=g)
     return blurred.float().contiguous(), psf.float()[None, None].contiguous()
+
+
+DUMP_MAX_BYTES = 64 << 20
+DUMP_SAMPLE = 8 << 20
+
+
+def dump_array(t):
+    """`t` on the host as numpy (float32 / float64); beyond DUMP_MAX_BYTES a fixed seeded sample of its flat elements."""
+    import torch
+    t = t.detach()
+    if t.numel() * t.element_size() > DUMP_MAX_BYTES:
+        idx = torch.randint(0, t.numel(), (DUMP_SAMPLE,), generator=torch.Generator().manual_seed(0)).sort().values
+        t = t.reshape(-1)[idx.to(t.device)]
+    return t.cpu().numpy()
+
+
+def write_dump(path, arrays):
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 # ------------------------------------------------------------------------------------------ clocks
@@ -314,13 +340,17 @@ def bench_train(args, rank, world, local_rank, config):
     e0 = torch.cuda.Event(enable_timing=True); e1 = torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
-        step(x_dev)
+        loss = step(x_dev)
     reducer.wait()
     e1.record()
     barrier()
     ms_total = e0.elapsed_time(e1)
     clocks = sampler.stop() if sampler else None
     launches = _lib.launch_count() - n0
+    dump = None
+    if args.dump_outputs and rank == 0:
+        dump = {"loss": dump_array(loss.reshape(1)), "grad_lmbda": dump_array(model.lmbda.grad),
+                "grad_rho": dump_array(model.rho.grad)}
     # e2e: every step's batch comes from pinned host memory; like a prefetching data loader, the copy of step i+1 runs on
     # a side stream while step i computes (two device buffers), and loss + gradients go back to the host every step
     cur = torch.cuda.current_stream()
@@ -352,6 +382,8 @@ def bench_train(args, rank, world, local_rank, config):
         ms_total, ms_e2e = float(t[0]), float(t[1])
     if rank != 0:
         return
+    if dump is not None:
+        write_dump(args.dump_outputs, dump)
     units = world * B * H * W * maxit * args.steps
     peak, peak_src = measured_peak()
     elems = B * C * H * W
@@ -407,9 +439,9 @@ def cpu_baseline_block(workload):
     return block
 
 
-def bench_cfg5_strong(rank, world, dev, barrier):
+def bench_cfg5_strong(rank, world, dev, barrier, steps):
     """BASELINE configs[4]: 4096 synthetic 256 x 256 RGB patches, 15 x 15 Gaussian PSF, 50 iterations, split over the N GPUs
-    of the job (STRONG scaling: 4096 / N images per rank, contiguous batch split, no collective).  Device-timed with the
+    of the job (STRONG scaling: 4096 / N images per rank, contiguous batch split, no collective), `steps` timed steps.  Device-timed with the
     whole shard resident (one fft_admm_tv call per step), and end to end through HostPipeline in chunks of 512 images from
     pinned host memory.  Returns the block on rank 0 (max over ranks)."""
     import torch
@@ -432,7 +464,7 @@ def bench_cfg5_strong(rank, world, dev, barrier):
     outs = [torch.empty(chunk, C, H, W).pin_memory() for _ in range(2)]
     kern = psf.to(dev)
     lam = torch.tensor([LAMBDA], device=dev); rho = torch.tensor([RHO], device=dev)
-    steps, warm = 3, 1
+    warm = 1
     for _ in range(warm):
         fft_admm_tv(x_dev, lam, rho, kern, False, maxit)
     barrier()
@@ -488,7 +520,10 @@ def main():
     ap.add_argument("--workload", default="cfg2", choices=sorted(WORKLOADS))
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-cfg5", action="store_true", help="skip the scaling_cfg5 block (4096 images over the N GPUs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -628,29 +663,35 @@ def main():
     barrier()
 
     def timed_pass():
+        """Returns (ms, output of the last step); every other step's output is released before the next step runs."""
+        out = None
         if flush is None:
             e0 = torch.cuda.Event(enable_timing=True); e1 = torch.cuda.Event(enable_timing=True)
             e0.record()
             for _ in range(args.steps):
-                step_resident()
+                out = None
+                out = step_resident()
             e1.record()
             barrier()
-            return e0.elapsed_time(e1)
+            return e0.elapsed_time(e1), out
         # small working set: L2 is flushed between steps and the flush is kept OUT of the timed intervals
         evs = []
         for _ in range(args.steps):
+            out = None
             flush.fill_(1)
             a0 = torch.cuda.Event(enable_timing=True); a1 = torch.cuda.Event(enable_timing=True)
             a0.record()
-            fft_admm_tv(x_dev, lam, rho, kern, False, maxit)
+            out = fft_admm_tv(x_dev, lam, rho, kern, False, maxit)
             a1.record()
             evs.append((a0, a1))
         barrier()
-        return sum(a.elapsed_time(b) for a, b in evs)
+        return sum(a.elapsed_time(b) for a, b in evs), out
 
-    ms_total = timed_pass()
+    ms_total, out = timed_pass()
     clocks = sampler.stop() if sampler else None
     launches = _lib.launch_count()
+    dump = {"out": dump_array(out)} if args.dump_outputs and rank == 0 else None
+    del out
     # ---- second pass with CUDA events around every kernel launch -> per-kernel times for `roofline`.  The kernels are
     # timed one at a time on ONE stream (the public call overlaps the two halves of the batch on two streams, which would
     # make the events of one half include the other half's kernels)
@@ -659,7 +700,7 @@ def main():
     _deconv.SPLIT_STREAMS = 1
     _lib.set_option("profile", 1)
     _lib.profile_reset()
-    ms_profiled = timed_pass()
+    ms_profiled = timed_pass()[0]
     prof = {kname: _lib.profile_read(kid) for kid, kname in enumerate(("rows", "cols", "other"))}
     _lib.set_option("profile", 0)
     _deconv.SPLIT_STREAMS = split
@@ -685,9 +726,11 @@ def main():
 
     cfg5 = None
     if args.workload == "cfg2" and not args.no_cfg5:
-        cfg5 = bench_cfg5_strong(rank, world, dev, barrier)
+        cfg5 = bench_cfg5_strong(rank, world, dev, barrier, args.steps)
 
     if rank == 0:
+        if dump is not None:
+            write_dump(args.dump_outputs, dump)
         units = world * B * H * W * maxit * args.steps            # pixel-iterations of the whole job
         value = units / (ms_total * 1e-3) / 1e6
         e2e_val = units / (ms_e2e * 1e-3) / 1e6

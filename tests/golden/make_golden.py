@@ -80,9 +80,10 @@ def main():
     # cfg1 of BASELINE.json, in full: single 256x256 grayscale, 15x15 Gaussian, 50 iterations
     psf = make_psf("gauss", 15, 2.5)
     save_case("cfg1_256_gauss15_n50", make_blurred((1, 1, 256, 256), psf), psf, 0.02, 0.04, False, 50)
-    # cfg2 reduced (same PSF family, 31-tap motion blur), small enough for a fixture
+    # cfg2 reduced (same PSF family, 31-tap motion blur), small enough for a fixture: the first image of a seeded pair
+    # (planes are independent for iso=False; one image keeps the file under 1 MB)
     psf = make_psf("motion", 31)
-    save_case("cfg2r_128_motion31_n30", make_blurred((2, 3, 128, 128), psf, seed=11), psf, 0.02, 0.04, False, 30)
+    save_case("cfg2r_128_motion31_n30", make_blurred((2, 3, 128, 128), psf, seed=11)[:1], psf, 0.02, 0.04, False, 30)
     # D5 pins: asymmetric odd and even kernels
     k7 = rng.random((7, 7)); k7 /= k7.sum()
     save_case("asym7_32x48_n20", make_blurred((2, 3, 32, 48), k7.astype(np.float32), seed=12), k7, 0.02, 0.04, False, 20)

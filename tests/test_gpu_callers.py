@@ -99,6 +99,34 @@ def test_admmfusion_matches_reference_fixture():
     assert y.shape == d["out32"].shape and e < TOL
 
 
+def test_admmfusion_solvers_match_reference_fixture():
+    """The solver part of the reference ADMMFusion (fixture fanout_fusion, with_admms=True: the output ends with the
+    concatenated solver results) without the reference's pooling block: the fixture's state dict loads with strict=True
+    and the solver channels match the reference's within 1e-4."""
+    from test_host_api import keyed_module
+    from torch_admm_deconv_b200 import ADMMFusion
+    d = golden("fanout_fusion")
+    sd = _sd(d)
+
+    class Pooling(torch.nn.Module):                      # keys of the reference's AttentionChannelPooling; 3 zero channels out
+        def __init__(self):
+            super().__init__()
+            self.cwa = keyed_module({k[8:]: v for k, v in sd.items() if k.startswith("acp.cwa.")}).to(_dev())
+
+        def forward(self, x):
+            return torch.zeros_like(x[:, :3])
+    f = ADMMFusion(FANOUT_CFGS, in_channels=3, with_admms=True, acp=Pooling())
+    f.load_state_dict(sd, strict=True)
+    f = f.to(_dev()).eval()
+    x = torch.from_numpy(d["x"]).to(_dev())
+    with torch.inference_mode():
+        y = f(x)
+    want = d["out32"][:, 3:]
+    e = O.rel_err(y[:, 3:].cpu().numpy(), want)
+    print("ADMMFusion solver channels vs reference: %.2e" % e)
+    assert y.shape == d["out32"].shape and e < TOL
+
+
 def test_fused_activation_and_uint8_input_match_reference_fixture():
     """activation(x + b) applied by the last kernel (admmdeconv.py:64) and a uint8 image read as x / 255 by the first
     (etransforms.py:29-31, dataload.py:31): against the reference's outputs, and bit-identical to the float path."""
@@ -196,6 +224,28 @@ def test_restorer_end_to_end_with_solver_dropped_in():
     # input perturbation to ~4e-3 at its output (measured with the reference itself on the CPU), so the end-to-end gate is
     # relative to the reference's own device-to-device deviation on the same weights
     assert e < max(3.0 * e_ref, 1e-3)
+
+
+def test_restorer_solver_branches_match_reference_fixture():
+    """The two ADMMDeconv branches of the reference's DivergentRestorer (fixture restorer_e2e: kern_size=(), 100
+    iterations, iso=True, learnable lmbda / rho drawn from the seeded init) on the fixture's input, against the branch
+    outputs of the reference's CPU run.  The scalar parameters are read back from the fixture's per-tensor sums."""
+    from torch_admm_deconv_b200 import ADMMDeconv
+    d = golden("restorer_e2e")
+    dev = _dev()
+    sums = dict(zip(d["sd_keys"].tolist(), d["sd_sums"].tolist()))
+    x = torch.from_numpy(d["x"]).to(dev)
+    for i in range(2):
+        pre = "blocks.0.admms.%d." % i
+        assert sums[pre + "w"] == 0.0 and sums[pre + "b"] == 0.0
+        m = ADMMDeconv((), max_iters=100, iso=True).to(dev)
+        with torch.no_grad():
+            m.lmbda.fill_(sums[pre + "lmbda"]); m.rho.fill_(sums[pre + "rho"])
+        with torch.inference_mode():
+            y = m(x)
+        e = O.rel_err(y.cpu().numpy(), d["admm%d" % i])
+        print("DivergentRestorer ADMM branch %d vs reference: %.2e" % (i, e))
+        assert e < TOL
 
 
 def test_cast_shim_for_float64_inputs():

@@ -127,12 +127,43 @@ def _ref_path():
         sys.path.insert(0, ref)
 
 
+def _reference_classes():
+    """Stand-ins for the reference's `ADMMDeconv` (elayers/admmdeconv.py:6-64) and `MultiADMM` (modelbuild/blocks.py:252-261),
+    which `use_b200_admm` meets inside reference models: a class of its own named ADMMDeconv with the reference's
+    attributes, parameter-vs-buffer status, state-dict keys and RNG draw order (checked against the reference's recorded
+    construction, fixture module_k5_bias), and a container holding the layers in `admms`."""
+    from torch_admm_deconv_b200 import ADMMDeconv as Ours
+
+    class ADMMDeconv(torch.nn.Module):
+        def __init__(self, *args, **kwargs):
+            super().__init__()
+            src = Ours(*args, **kwargs)
+            for name in ("w", "lmbda", "rho", "b"):
+                t = getattr(src, name)
+                if isinstance(t, torch.nn.Parameter):
+                    self.register_parameter(name, t)
+                else:
+                    self.register_buffer(name, t)
+            self.max_iters, self.iso, self.activation = src.max_iters, src.iso, src.activation
+
+    class MultiADMM(torch.nn.Module):
+        def __init__(self, admm_dicts):
+            super().__init__()
+            self.admms = torch.nn.ModuleList(ADMMDeconv(**d) for d in admm_dicts)
+
+    d = golden("module_k5_bias")
+    torch.manual_seed(1234)
+    ref = ADMMDeconv((5, 5), max_iters=8, lmbda=None, rho=None, iso=False, bias=True)
+    assert list(ref.state_dict().keys()) == ["w", "lmbda", "rho", "b"]
+    assert all(np.array_equal(v.numpy(), d["init_" + k]) for k, v in ref.state_dict().items())
+    assert [isinstance(getattr(ref, n), torch.nn.Parameter) for n in ("w", "lmbda", "rho", "b")] == list(d["is_param"])
+    return MultiADMM, ADMMDeconv
+
+
 def test_drop_in_conversion_shares_parameters_and_keys():
     """use_b200_admm swaps the reference's ADMMDeconv layers inside the reference's own model, keeping the very same
     Parameter objects (optimizers, clippers that reach into .lmbda/.rho/.w, checkpoints: scripts/train.py:27-38,75-78)."""
-    _ref_path()
-    from admmtor.modelbuild.blocks import MultiADMM as RefMulti
-    from admmtor.elayers.admmdeconv import ADMMDeconv as RefLayer
+    RefMulti, RefLayer = _reference_classes()
     from torch_admm_deconv_b200 import use_b200_admm, ADMMDeconv
     cfgs = [dict(kern_size=(3, 3), max_iters=4, lmbda=None, rho=0.1, iso=False, bias=True, activation=torch.relu),
             dict(kern_size=(), max_iters=7)]
@@ -159,3 +190,42 @@ def test_admmfusion_state_dict_matches_reference():
     assert list(rs.keys()) == list(os_.keys())
     assert all(torch.equal(rs[k], os_[k]) for k in rs)                   # same RNG draw order as the reference
     o.load_state_dict(rs, strict=True)
+
+
+FANOUT_CFGS = [dict(kern_size=(), max_iters=12, lmbda=0.02, rho=0.04, iso=True),
+               dict(kern_size=(5, 5), max_iters=8, lmbda=None, rho=None, iso=False),
+               dict(kern_size=(), max_iters=10, lmbda=None, rho=None, iso=False, bias=True)]
+
+
+def keyed_module(sd):
+    """A module holding zero parameters under the keys of the state dict `sd` (stands in for a block that is not part of
+    this package, so that a state dict containing it loads with strict=True)."""
+    root = torch.nn.Module()
+    for key, v in sd.items():
+        *path, leaf = key.split(".")
+        m = root
+        for p in path:
+            if not hasattr(m, p):
+                m.add_module(p, torch.nn.Module())
+            m = getattr(m, p)
+        m.register_parameter(leaf, torch.nn.Parameter(torch.zeros(v.shape)))
+    return root
+
+
+def test_admmfusion_solver_state_dict_matches_reference_fixture():
+    """The solver part of ADMMFusion against the reference's ADMMFusion(FANOUT_CFGS, in_channels=3) built after
+    torch.manual_seed(12) (fixture fanout_fusion; the reference then replaced the 5 x 5 `w` by a Gaussian): same keys in
+    the same order, same RNG draws, and the reference state dict loads with strict=True.  The pooling block `acp` is
+    reference code, given here as a module with its keys."""
+    from torch_admm_deconv_b200 import ADMMFusion
+    d = golden("fanout_fusion")
+    sd = {k[3:]: torch.from_numpy(d[k]) for k in d.files if k.startswith("sd.")}
+    acp = keyed_module({k[4:]: v for k, v in sd.items() if k.startswith("acp.")})
+    torch.manual_seed(12)
+    o = ADMMFusion(FANOUT_CFGS, in_channels=3, with_admms=True, acp=acp)
+    os_ = o.state_dict()
+    assert list(os_.keys()) == list(sd.keys())
+    for k, v in sd.items():
+        if k.startswith("admms.") and k != "admms.1.w":
+            assert torch.equal(os_[k], v), k
+    o.load_state_dict(sd, strict=True)
