@@ -11,7 +11,8 @@
  *
  * Conventions
  *   - every pointer is a DEVICE pointer unless the name starts with `host_`;
- *   - image fields are fp32, contiguous NCHW; a "plane" is one (b, c) image, planes = B*C;
+ *   - image fields are fp32, contiguous NCHW; a "plane" is one (b, c) image, planes = B*C (the *_f64 calls: fp64
+ *     everywhere, see "float64 solve" below);
  *   - lmbd / rho are device pointers to ONE float each (learnable parameters: never read on host);
  *   - kern is (ksize x ksize) fp32 row-major, or NULL with ksize == 0 for the TV-denoise branch
  *     (deconv.py:46-47, 86-87);
@@ -30,7 +31,7 @@
 extern "C" {
 #endif
 
-#define ADMM_B200_VERSION 200   /* major*10000 + minor*100 + patch */
+#define ADMM_B200_VERSION 300   /* major*10000 + minor*100 + patch */
 
 /* error codes */
 #define ADMM_OK                0
@@ -132,6 +133,25 @@ int admm_tv_backward_ex(const float* y, const float* grad_out,
                         void* workspace, size_t workspace_bytes,
                         float* grad_y, float* grad_kern, float* grad_lmbd, float* grad_rho,
                         void* stream, int ckpt_interval);
+
+/* ---- float64 solve.  The reference computes in xin.dtype (deconv.py:50-67); these calls are the float32 ones above with
+ * double in place of float for every tensor (y, out, kern, lmbd, rho, saved state, gradients), same conventions, error
+ * codes and semantics (iso, empty PSF, negative tau, maxit = 0 / 1).  They run on the generic (any H, W) kernels
+ * instantiated for double.  Shared memory bounds the size: the column pass needs H <= 4842, the row pass W <= 2905 for
+ * iso = 0 with maxit >= 2 (two halo rows) and W <= 4842 otherwise; a larger frame returns ADMM_ERR_UNSUPPORTED before
+ * anything is launched.  No bias, activation, uint8 input, shared spectrum or checkpointing.
+ * Saved state: [slot][q_x, q_y][all planes] for slots 0 .. maxit-2, then for iso = 1 the maxit-1 pairs of H x W pixel-norm
+ * maps, in double (admm_query_saved_f64 = 2 x admm_query_saved - 256: both include one 256-byte pad). */
+size_t admm_query_workspace_f64(int planes, int H, int W, int ksize, int iso, int maxit);
+size_t admm_query_workspace_backward_f64(int planes, int H, int W, int ksize, int iso, int maxit);
+size_t admm_query_saved_f64(int planes, int H, int W, int ksize, int iso, int maxit);
+int admm_tv_forward_f64(const double* y, double* out, const double* kern, int ksize,
+                        const double* lmbd, const double* rho, int B, int C, int H, int W, int iso, int maxit,
+                        void* workspace, size_t workspace_bytes, void* saved, size_t saved_bytes, void* stream);
+int admm_tv_backward_f64(const double* y, const double* grad_out, const double* kern, int ksize,
+                         const double* lmbd, const double* rho, int B, int C, int H, int W, int iso, int maxit,
+                         const void* saved, size_t saved_bytes, void* workspace, size_t workspace_bytes,
+                         double* grad_y, double* grad_kern, double* grad_lmbd, double* grad_rho, void* stream);
 
 /* ---- measurement hooks (bench.py): per-kernel-class device time from CUDA events recorded on the launch
  * stream when option "profile" is 1, and the number of kernels launched since the last reset.

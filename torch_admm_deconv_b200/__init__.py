@@ -10,11 +10,11 @@
 The arithmetic runs in hand-written sm_100a CUDA kernels reached through the C ABI of
 include/admm_b200.h; there is no CPU or PyTorch fallback.
 """
-from .eops.deconv import fft_admm_tv, identity, soft_thresh, block_thresh, pixelnorm, hard_thresh, torch_abs2
+from .eops.deconv import fft_admm_tv, fft_admm_tv_f64, identity, soft_thresh, block_thresh, pixelnorm, hard_thresh, torch_abs2
 from .elayers.admmdeconv import ADMMDeconv
 from .elayers.multiadmm import MultiADMM, Deconvs, ADMMFusion
 from .dropin import use_b200_admm
 
-__all__ = ["fft_admm_tv", "ADMMDeconv", "MultiADMM", "Deconvs", "ADMMFusion", "use_b200_admm", "identity", "soft_thresh", "block_thresh", "pixelnorm", "hard_thresh",
+__all__ = ["fft_admm_tv", "fft_admm_tv_f64", "ADMMDeconv", "MultiADMM", "Deconvs", "ADMMFusion", "use_b200_admm", "identity", "soft_thresh", "block_thresh", "pixelnorm", "hard_thresh",
            "torch_abs2"]
 __version__ = "0.2.0"

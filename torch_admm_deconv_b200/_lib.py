@@ -49,6 +49,12 @@ SIGNATURES["admm_query_workspace_backward_ex"] = (_sz, [_i] * 7)
 SIGNATURES["admm_tv_backward_ex"] = (_i, SIGNATURES["admm_tv_backward"][1] + [_i])
 SIGNATURES["admm_spectrum_forward"] = (_i, [_vp, _i, _vp, _i, _i, _i, _vp, _sz, _vp])
 SIGNATURES["admm_tv_forward_ex"] = (_i, SIGNATURES["admm_tv_forward"][1] + [ctypes.POINTER(AdmmExt)])
+# float64 solve: the float32 calls with double tensors (admm_tv_forward_f64 has no bias argument)
+SIGNATURES["admm_query_workspace_f64"] = (_sz, [_i] * 6)
+SIGNATURES["admm_query_workspace_backward_f64"] = (_sz, [_i] * 6)
+SIGNATURES["admm_query_saved_f64"] = (_sz, [_i] * 6)
+SIGNATURES["admm_tv_forward_f64"] = (_i, [_vp, _vp, _vp, _i, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _sz, _vp, _sz, _vp])
+SIGNATURES["admm_tv_backward_f64"] = SIGNATURES["admm_tv_backward"]
 
 _lib = None
 

@@ -32,9 +32,26 @@ int launch_twiddles(float2* tw, double2* twd, int N, cudaStream_t st) {
     return 0;
 }
 
+// the float64 solve keeps the double table only (same values as k_twiddles' twd)
+__global__ void k_twiddles_f64(double2* __restrict__ twd, int N) {
+    int n = blockIdx.x * blockDim.x + threadIdx.x;
+    if (n >= N) return;
+    double s, c;
+    sincospi(-2.0 * (double)n / (double)N, &s, &c);
+    twd[n] = make_double2(c, s);
+}
+
+int launch_twiddles_f64(double2* twd, int N, cudaStream_t st) {
+    ProfScope ps(PROF_OTHER, st);
+    k_twiddles_f64<<<(N + 255) / 256, 256, 0, st>>>(twd, N);
+    ADMM_CUDA_CHECK(cudaGetLastError());
+    return 0;
+}
+
 // ------------------------------------------------------------------------------------------ tables
 // G[a][v] = sum_b kern[a][b] e^{-2 pi i v b / W},  v in [0, W/2]        (row DFT of the zero-padded PSF)
-__global__ void k_kern_rowdft(const float* __restrict__ kern, int ks, int W,
+template <typename T>
+__global__ void k_kern_rowdft(const T* __restrict__ kern, int ks, int W,
                               const double2* __restrict__ twWd, double2* __restrict__ G) {
     const int Wh = W / 2 + 1;
     int idx = blockIdx.x * blockDim.x + threadIdx.x;
@@ -49,103 +66,126 @@ __global__ void k_kern_rowdft(const float* __restrict__ kern, int ks, int W,
     G[idx] = make_double2(re, im);
 }
 
+template <typename T>
 __global__ void k_tables(int H, int W, int Wc, int ks, const double2* __restrict__ G,
                          const double2* __restrict__ twHd, const double2* __restrict__ twWd,
-                         const float* __restrict__ rho_p,
-                         float* __restrict__ Bm, float* __restrict__ Bq,
-                         float2* __restrict__ Mul, float2* __restrict__ Mq) {
+                         const T* __restrict__ rho_p,
+                         T* __restrict__ Bm, T* __restrict__ Bq,
+                         cplx_t<T>* __restrict__ Mul, cplx_t<T>* __restrict__ Mq) {
     int idx = blockIdx.x * blockDim.x + threadIdx.x;
     if (idx >= H * Wc) return;
     const int u = idx / Wc, c = idx - u * Wc;
     const double rho = (double)rho_p[0];
     TabEntry e = table_entry(u, c, H, W, ks, G, twHd, twWd, rho);
     if (c > 0) {
-        Bm[idx] = (float)e.bm;
-        Mul[idx] = make_float2((float)e.mul.x, (float)e.mul.y);
+        Bm[idx] = (T)e.bm;
+        Mul[idx] = make_cplx((T)e.mul.x, (T)e.mul.y);
     } else {
         // packed column 0 carries the DC and the Nyquist column: X = A0 + Bp Z + Bq conj(Z[-u])
         TabEntry n = e;
         if ((W & 1) == 0) n = table_entry(u, W / 2, H, W, ks, G, twHd, twWd, rho);
-        Bm[idx] = (float)(0.5 * (e.bm + n.bm));
-        Bq[u] = (float)(0.5 * (e.bm - n.bm));
-        Mul[idx] = make_float2((float)(0.5 * (e.mul.x + n.mul.x)), (float)(0.5 * (e.mul.y + n.mul.y)));
-        Mq[u] = make_float2((float)(0.5 * (e.mul.x - n.mul.x)), (float)(0.5 * (e.mul.y - n.mul.y)));
+        Bm[idx] = (T)(0.5 * (e.bm + n.bm));
+        Bq[u] = (T)(0.5 * (e.bm - n.bm));
+        Mul[idx] = make_cplx((T)(0.5 * (e.mul.x + n.mul.x)), (T)(0.5 * (e.mul.y + n.mul.y)));
+        Mq[u] = make_cplx((T)(0.5 * (e.mul.x - n.mul.x)), (T)(0.5 * (e.mul.y - n.mul.y)));
     }
 }
 
-int launch_tables(const Geometry& g, const Workspace& ws, const float* kern, int ksize,
-                  const float* rho, cudaStream_t st) {
+template <typename T>
+static int launch_tables_t(const Geometry& g, const double2* twWd, const double2* twHd, double2* kdft, T* Bm, T* Bq,
+                           cplx_t<T>* Mul, cplx_t<T>* Mq, const T* kern, int ksize, const T* rho, cudaStream_t st) {
     if (ksize > 0) {
         int n = ksize * (g.W / 2 + 1);
         ProfScope ps(PROF_OTHER, st);
-        k_kern_rowdft<<<(n + 127) / 128, 128, 0, st>>>(kern, ksize, g.W, ws.twWd, ws.kdft);
+        k_kern_rowdft<<<(n + 127) / 128, 128, 0, st>>>(kern, ksize, g.W, twWd, kdft);
         ADMM_CUDA_CHECK(cudaGetLastError());
     }
     int n = g.H * g.Wc;
     ProfScope ps(PROF_OTHER, st);
-    k_tables<<<(n + 127) / 128, 128, 0, st>>>(g.H, g.W, g.Wc, ksize, ws.kdft, ws.twHd, ws.twWd, rho,
-                                              ws.Bm, ws.Bq, ws.Mul, ws.Mq);
+    k_tables<<<(n + 127) / 128, 128, 0, st>>>(g.H, g.W, g.Wc, ksize, kdft, twHd, twWd, rho, Bm, Bq, Mul, Mq);
     ADMM_CUDA_CHECK(cudaGetLastError());
     return 0;
 }
 
+int launch_tables(const Geometry& g, const Workspace& ws, const float* kern, int ksize,
+                  const float* rho, cudaStream_t st) {
+    return launch_tables_t(g, ws.twWd, ws.twHd, ws.kdft, ws.Bm, ws.Bq, ws.Mul, ws.Mq, kern, ksize, rho, st);
+}
+
+int launch_tables_f64(const Geometry& g, const double2* twWd, const double2* twHd, double2* kdft, double* Bm, double* Bq,
+                      double2* Mul, double2* Mq, const double* kern, int ksize, const double* rho, cudaStream_t st) {
+    return launch_tables_t(g, twWd, twHd, kdft, Bm, Bq, Mul, Mq, kern, ksize, rho, st);
+}
+
 // ------------------------------------------------------------------------------------------ row pass
-__device__ __forceinline__ float clampf(float q, float tau) { return dual_any(q, tau); }      // u(q), any sign of tau (common.cuh)
+template <typename T> __device__ __forceinline__ T clampf(T q, T tau) { return dual_any(q, tau); }      // u(q), any sign of tau (common.cuh)
 // w = z - u with z = soft_thresh(q), u = q - z  ==>  w = q - 2 clamp(q)    (deconv.py:15-16, 104, 114-115)
-__device__ __forceinline__ float wfun(float q, float tau) { return fmaf(-2.0f, clampf(q, tau), q); }
+template <typename T> __device__ __forceinline__ T wfun(T q, T tau) { return xfma(T(-2), clampf(q, tau), q); }
+// the fused activation of the layer exists in float only (the float64 solve never sets one)
+__device__ __forceinline__ float act_out(float v, int act) { return act_apply(v, act); }
+__device__ __forceinline__ double act_out(double v, int) { return v; }
 
 // Two real rows <-> one complex FFT (z = row_a + i row_b).  Merge builds the full complex spectrum of z
 // from the two packed half spectra; split is the inverse.
-__device__ __forceinline__ void merge_pairs(const float2* __restrict__ S, int H, int W, int Wc, int BS,
-                                            int rfirst, int nrows, int NP, float2* __restrict__ buf) {
+template <typename V>
+__device__ __forceinline__ void merge_pairs(const V* __restrict__ S, int H, int W, int Wc, int BS,
+                                            int rfirst, int nrows, int NP, V* __restrict__ buf) {
+    using T = real_t<V>;
     const bool even = (W & 1) == 0;
     for (int w = threadIdx.x; w < NP * Wc; w += blockDim.x) {
         const int m = w / Wc, c = w - m * Wc;
         int ra = rfirst + 2 * m; ra %= H; if (ra < 0) ra += H;
-        float2 a = S[(size_t)ra * Wc + c];
-        float2 b = make_float2(0.f, 0.f);
+        V a = S[(size_t)ra * Wc + c];
+        V b = make_cplx(T(0), T(0));
         if (2 * m + 1 < nrows) {
             int rb = ra + 1; if (rb >= H) rb -= H;
             b = S[(size_t)rb * Wc + c];
         }
         if (c == 0) {
-            buf[m] = make_float2(a.x, b.x);
-            if (even) buf[(W / 2) * BS + m] = make_float2(a.y, b.y);
+            buf[m] = make_cplx(a.x, b.x);
+            if (even) buf[(W / 2) * BS + m] = make_cplx(a.y, b.y);
         } else {
-            buf[c * BS + m] = make_float2(a.x - b.y, a.y + b.x);
-            buf[(W - c) * BS + m] = make_float2(a.x + b.y, b.x - a.y);
+            buf[c * BS + m] = make_cplx(a.x - b.y, a.y + b.x);
+            buf[(W - c) * BS + m] = make_cplx(a.x + b.y, b.x - a.y);
         }
     }
 }
 
-__device__ __forceinline__ void split_pairs(const float2* __restrict__ res, int W, int Wc, int BS,
-                                            int r0, int Rb, int NP, float2* __restrict__ out) {
+template <typename V>
+__device__ __forceinline__ void split_pairs(const V* __restrict__ res, int W, int Wc, int BS,
+                                            int r0, int Rb, int NP, V* __restrict__ out) {
+    using T = real_t<V>;
     const bool even = (W & 1) == 0;
     for (int w = threadIdx.x; w < NP * Wc; w += blockDim.x) {
         const int m = w / Wc, c = w - m * Wc;
-        const float2 Z = res[c * BS + m];
-        float2 Xa, Xb;
+        const V Z = res[c * BS + m];
+        V Xa, Xb;
         if (c == 0) {
-            float2 Zn = even ? res[(W / 2) * BS + m] : make_float2(0.f, 0.f);
-            Xa = make_float2(Z.x, Zn.x);
-            Xb = make_float2(Z.y, Zn.y);
+            V Zn = even ? res[(W / 2) * BS + m] : make_cplx(T(0), T(0));
+            Xa = make_cplx(Z.x, Zn.x);
+            Xb = make_cplx(Z.y, Zn.y);
         } else {
-            const float2 Zm = res[(W - c) * BS + m];
-            Xa = make_float2(0.5f * (Z.x + Zm.x), 0.5f * (Z.y - Zm.y));
-            Xb = make_float2(0.5f * (Z.y + Zm.y), 0.5f * (Zm.x - Z.x));
+            const V Zm = res[(W - c) * BS + m];
+            Xa = make_cplx(T(0.5) * (Z.x + Zm.x), T(0.5) * (Z.y - Zm.y));
+            Xb = make_cplx(T(0.5) * (Z.y + Zm.y), T(0.5) * (Zm.x - Z.x));
         }
         out[(size_t)(r0 + 2 * m) * Wc + c] = Xa;
         if (2 * m + 1 < Rb) out[(size_t)(r0 + 2 * m + 1) * Wc + c] = Xb;
     }
 }
 
-template <int MODE>
-__global__ void __launch_bounds__(1024)
-k_rows(RowArgs a, FftPlan plan, int H, int W, int Wc, int R, int BS, int nbands) {
-    extern __shared__ float2 smem[];
-    float2* bufA = smem;
-    float2* bufB = bufA + (size_t)W * BS;
-    float2* tw = bufB + (size_t)W * BS;
+// Threads per CTA of the generic kernels: float as tuned; double at most 256 (a radix-16 butterfly holds 32 doubles:
+// with 512 or 1024 threads the 128 / 64 registers per thread spill, with 256 nothing does)
+template <typename T> constexpr int kGenericMaxThreads = sizeof(T) == 4 ? 1024 : 256;
+
+template <int MODE, typename T>
+__global__ void __launch_bounds__(kGenericMaxThreads<T>)
+k_rows(RowArgsT<T> a, FftPlan plan, int H, int W, int Wc, int R, int BS, int nbands) {
+    using V = cplx_t<T>;
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    V* bufA = reinterpret_cast<V*>(smem_raw);
+    V* bufB = bufA + (size_t)W * BS;
+    V* tw = bufB + (size_t)W * BS;
     const int band = blockIdx.x % nbands;
     const int p = blockIdx.x / nbands;
     const int r0 = band * R;
@@ -156,17 +196,17 @@ k_rows(RowArgs a, FftPlan plan, int H, int W, int Wc, int R, int BS, int nbands)
 
     if (MODE == ROWS_R2C) {
         const int NP = (Rb + 1) / 2;
-        const float* in = a.real_in + plane_real;
+        const T* in = a.real_in + plane_real;
         const unsigned char* in8 = a.real_in_u8 ? a.real_in_u8 + plane_real : nullptr;
         for (int w = threadIdx.x; w < NP * W; w += blockDim.x) {
             const int m = w / W, c = w - m * W;
             const int ra = r0 + 2 * m;
-            float xa = in8 ? ld_u8_div255(in8 + (size_t)ra * W + c) : in[(size_t)ra * W + c];
-            float xb = (2 * m + 1 < Rb) ? (in8 ? ld_u8_div255(in8 + (size_t)(ra + 1) * W + c) : in[(size_t)(ra + 1) * W + c]) : 0.f;
-            bufA[c * BS + m] = make_float2(xa, xb);
+            T xa = in8 ? (T)ld_u8_div255(in8 + (size_t)ra * W + c) : in[(size_t)ra * W + c];
+            T xb = (2 * m + 1 < Rb) ? (in8 ? (T)ld_u8_div255(in8 + (size_t)(ra + 1) * W + c) : in[(size_t)(ra + 1) * W + c]) : T(0);
+            bufA[c * BS + m] = make_cplx(xa, xb);
         }
         __syncthreads();
-        float2* res = fft_batched<-1>(bufA, bufB, plan, NP, BS, tw);
+        V* res = fft_batched<-1>(bufA, bufB, plan, NP, BS, tw);
         split_pairs(res, W, Wc, BS, r0, Rb, NP, a.spec_out + plane_spec);
         return;
     }
@@ -175,16 +215,16 @@ k_rows(RowArgs a, FftPlan plan, int H, int W, int Wc, int R, int BS, int nbands)
         const int NP = (Rb + 1) / 2;
         merge_pairs(a.spec_in + plane_spec, H, W, Wc, BS, r0, Rb, NP, bufA);
         __syncthreads();
-        float2* res = fft_batched<+1>(bufA, bufB, plan, NP, BS, tw);
-        float* out = a.real_out + out_plane_offset(a, p, H, W);
-        const float bias = a.bias ? a.bias[0] : 0.f;
+        V* res = fft_batched<+1>(bufA, bufB, plan, NP, BS, tw);
+        T* out = a.real_out + out_plane_offset(a, p, H, W);
+        const T bias = a.bias ? a.bias[0] : T(0);
         const int act = a.act;
         for (int w = threadIdx.x; w < NP * W; w += blockDim.x) {
             const int m = w / W, c = w - m * W;
             const int ra = r0 + 2 * m;
-            const float2 z = res[c * BS + m];
-            out[(size_t)ra * W + c] = act_apply(z.x + bias, act);
-            if (2 * m + 1 < Rb) out[(size_t)(ra + 1) * W + c] = act_apply(z.y + bias, act);
+            const V z = res[c * BS + m];
+            out[(size_t)ra * W + c] = act_out(z.x + bias, act);
+            if (2 * m + 1 < Rb) out[(size_t)(ra + 1) * W + c] = act_out(z.y + bias, act);
         }
         return;
     }
@@ -195,27 +235,27 @@ k_rows(RowArgs a, FftPlan plan, int H, int W, int Wc, int R, int BS, int nbands)
         const int NP = (nrows + 1) / 2;
         merge_pairs(a.spec_in + plane_spec, H, W, Wc, BS, r0 - 1, nrows, NP, bufA);
         __syncthreads();
-        float2* res = fft_batched<+1>(bufA, bufB, plan, NP, BS, tw);
-        float2* zb = (res == bufA) ? bufB : bufA;
-        const float tau = a.lmbd[0] / a.rho[0];                     // deconv.py:44
-        const float* qxi = a.qx_in ? a.qx_in + plane_real : nullptr;
-        const float* qyi = a.qy_in ? a.qy_in + plane_real : nullptr;
-        float* qxo = a.qx_out + plane_real;
-        float* qyo = a.qy_out + plane_real;
+        V* res = fft_batched<+1>(bufA, bufB, plan, NP, BS, tw);
+        V* zb = (res == bufA) ? bufB : bufA;
+        const T tau = a.lmbd[0] / a.rho[0];                         // deconv.py:44
+        const T* qxi = a.qx_in ? a.qx_in + plane_real : nullptr;
+        const T* qyi = a.qy_in ? a.qy_in + plane_real : nullptr;
+        T* qxo = a.qx_out + plane_real;
+        T* qyo = a.qy_out + plane_real;
         const int NPv = (Rb + 1) / 2;
         for (int w = threadIdx.x; w < NPv * W; w += blockDim.x) {
             const int m = w / W, c = w - m * W;
             const int cl = (c == 0) ? W - 1 : c - 1;
             const int cr = (c == W - 1) ? 0 : c + 1;
-            const float2 P0c = res[c * BS + m],  P1c = res[c * BS + m + 1];
-            const float2 P0l = res[cl * BS + m], P1l = res[cl * BS + m + 1];
-            const float2 P0r = res[cr * BS + m], P1r = res[cr * BS + m + 1];
+            const V P0c = res[c * BS + m],  P1c = res[c * BS + m + 1];
+            const V P0l = res[cl * BS + m], P1l = res[cl * BS + m + 1];
+            const V P0r = res[cr * BS + m], P1r = res[cr * BS + m + 1];
             const int ra = r0 + 2 * m;
             const bool hasb = (2 * m + 1 < Rb);
             int rb = ra + 1; if (rb >= H) rb -= H;
             int rc = rb + 1; if (rc >= H) rc -= H;
             // previous dual u = clamp(q_prev)   (q_prev == 0 on the first iteration)
-            float uxa = 0.f, uxar = 0.f, uya = 0.f, uyb = 0.f, uxb = 0.f, uxbr = 0.f, uyc = 0.f;
+            T uxa = 0, uxar = 0, uya = 0, uyb = 0, uxb = 0, uxbr = 0, uyc = 0;
             if (qxi) {
                 uxa  = clampf(qxi[(size_t)ra * W + c], tau);
                 uxar = clampf(qxi[(size_t)ra * W + cr], tau);
@@ -227,41 +267,41 @@ k_rows(RowArgs a, FftPlan plan, int H, int W, int Wc, int R, int BS, int nbands)
                     uyc  = clampf(qyi[(size_t)rc * W + c], tau);
                 }
             }
-            const float xu = P0c.x;                                  // row ra-1
-            const float xa_c = P0c.y, xa_l = P0l.y, xa_r = P0r.y;    // row ra
-            const float xb_c = P1c.x, xb_l = P1l.x, xb_r = P1r.x;    // row ra+1
-            const float xd = P1c.y;                                  // row ra+2
-            const float qx_a  = xa_c - xa_l + uxa;                   // deconv.py:108,111,114
-            const float qx_ar = xa_r - xa_c + uxar;
-            const float qy_a  = xa_c - xu + uya;                     // deconv.py:109,112,115
-            const float qy_b  = xb_c - xa_c + uyb;
-            const float va = wfun(qx_a, tau) - wfun(qx_ar, tau) + wfun(qy_a, tau) - wfun(qy_b, tau);   // deconv.py:104
+            const T xu = P0c.x;                                  // row ra-1
+            const T xa_c = P0c.y, xa_l = P0l.y, xa_r = P0r.y;    // row ra
+            const T xb_c = P1c.x, xb_l = P1l.x, xb_r = P1r.x;    // row ra+1
+            const T xd = P1c.y;                                  // row ra+2
+            const T qx_a  = xa_c - xa_l + uxa;                   // deconv.py:108,111,114
+            const T qx_ar = xa_r - xa_c + uxar;
+            const T qy_a  = xa_c - xu + uya;                     // deconv.py:109,112,115
+            const T qy_b  = xb_c - xa_c + uyb;
+            const T va = wfun(qx_a, tau) - wfun(qx_ar, tau) + wfun(qy_a, tau) - wfun(qy_b, tau);   // deconv.py:104
             qxo[(size_t)ra * W + c] = qx_a;
             qyo[(size_t)ra * W + c] = qy_a;
-            float vb = 0.f;
+            T vb = 0;
             if (hasb) {
-                const float qx_b  = xb_c - xb_l + uxb;
-                const float qx_br = xb_r - xb_c + uxbr;
-                const float qy_c  = xd - xb_c + uyc;
+                const T qx_b  = xb_c - xb_l + uxb;
+                const T qx_br = xb_r - xb_c + uxbr;
+                const T qy_c  = xd - xb_c + uyc;
                 vb = wfun(qx_b, tau) - wfun(qx_br, tau) + wfun(qy_b, tau) - wfun(qy_c, tau);
                 qxo[(size_t)rb * W + c] = qx_b;
                 qyo[(size_t)rb * W + c] = qy_b;
             }
-            zb[c * BS + m] = make_float2(va, vb);
+            zb[c * BS + m] = make_cplx(va, vb);
         }
         __syncthreads();
-        float2* res2 = fft_batched<-1>(zb, res, plan, NPv, BS, tw);
+        V* res2 = fft_batched<-1>(zb, res, plan, NPv, BS, tw);
         split_pairs(res2, W, Wc, BS, r0, Rb, NPv, a.spec_out + plane_spec);
         return;
     }
 }
 
-static size_t rows_smem(int W, int BS) { return ((size_t)2 * W * BS + W) * sizeof(float2); }
+template <typename T>
+static size_t rows_smem(int W, int BS) { return ((size_t)2 * W * BS + W) * sizeof(cplx_t<T>); }
 
-int launch_rows(RowMode mode, const Geometry& g, const RowArgs& a, cudaStream_t st) {
-    if (rows_pow2_supported(g)) return launch_rows_pow2(mode, g, a, st);
-    if ((mode == ROWS_FULL || mode == ROWS_FULL_U) && rows_big_supported(g)) return launch_rows_big(mode, g, a, st);
-    if ((mode == ROWS_R2C || mode == ROWS_C2R) && rows_big_supported(g)) return launch_rows_big_plain(mode, g, a, st);
+// the generic engine (any W); float and double
+template <typename T>
+static int launch_rows_generic(RowMode mode, const Geometry& g, const RowArgsT<T>& a, cudaStream_t st) {
     if (mode == ROWS_ADJ || mode == ROWS_FULL_U) return fail(4, "this row-pass mode exists for power-of-two widths only");
     FftPlan plan;
     if (!make_plan(g.W, plan)) return fail(4, "cannot plan row FFT length");
@@ -275,19 +315,19 @@ int launch_rows(RowMode mode, const Geometry& g, const RowArgs& a, cudaStream_t 
     for (;; R -= 2) {
         int NP = (R + halo + 1) / 2;
         BS = NP | 1;
-        if (rows_smem(g.W, BS) <= kMax) break;
-        if (rows_smem(g.W, NP) <= kMax) { BS = NP; break; }
+        if (rows_smem<T>(g.W, BS) <= kMax) break;
+        if (rows_smem<T>(g.W, NP) <= kMax) { BS = NP; break; }
         if (R <= 2) return fail(4, "row FFT does not fit in shared memory (W too large for the generic kernel)");
     }
     // prefer bands that leave >= 2 CTAs per SM when the image is wide
-    while (R > 4 && rows_smem(g.W, ((R + halo + 1) / 2) | 1) > 100 * 1024) {
+    while (R > 4 && rows_smem<T>(g.W, ((R + halo + 1) / 2) | 1) > 100 * 1024) {
         R -= 2; BS = ((R + halo + 1) / 2) | 1;
     }
     const int nbands = (g.H + R - 1) / R;
-    const size_t smem = rows_smem(g.W, BS);
+    const size_t smem = rows_smem<T>(g.W, BS);
     // one or two fat CTAs per SM need more warps each to keep the SM busy
-    const int threads = options().threads > 0 ? options().threads.load()
-                                              : (smem > 113 * 1024 ? 1024 : (smem > 75 * 1024 ? 512 : 256));
+    const int threads = std::min(kGenericMaxThreads<T>, options().threads > 0 ? options().threads.load()
+                                              : (smem > 113 * 1024 ? 1024 : (smem > 75 * 1024 ? 512 : 256)));
     dim3 grid((unsigned)((size_t)nbands * g.P));
     // the opt-in shared-memory limit is a per-device function attribute: raised once to the maximum (the call costs
     // several microseconds of host time, which dominated small problems when it was repeated for every launch)
@@ -297,10 +337,10 @@ int launch_rows(RowMode mode, const Geometry& g, const RowArgs& a, cudaStream_t 
     do {                                                                                                   \
         static std::atomic<bool> attr_set[64];                                                                     \
         if (dev_id >= 64 || !attr_set[dev_id]) {                                                           \
-            ADMM_CUDA_CHECK(cudaFuncSetAttribute(k_rows<M>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMax)); \
+            ADMM_CUDA_CHECK(cudaFuncSetAttribute(k_rows<M, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMax)); \
             if (dev_id < 64) attr_set[dev_id] = true;                                                      \
         }                                                                                                  \
-        k_rows<M><<<grid, threads, smem, st>>>(a, plan, g.H, g.W, g.Wc, R, BS, nbands);                     \
+        k_rows<M, T><<<grid, threads, smem, st>>>(a, plan, g.H, g.W, g.Wc, R, BS, nbands);                  \
     } while (0)
     ProfScope ps(mode == ROWS_FULL ? PROF_ROWS : PROF_OTHER, st);
     switch (mode) {
@@ -314,27 +354,41 @@ int launch_rows(RowMode mode, const Geometry& g, const RowArgs& a, cudaStream_t 
     return 0;
 }
 
+int launch_rows(RowMode mode, const Geometry& g, const RowArgs& a, cudaStream_t st) {
+    if (rows_pow2_supported(g)) return launch_rows_pow2(mode, g, a, st);
+    if ((mode == ROWS_FULL || mode == ROWS_FULL_U) && rows_big_supported(g)) return launch_rows_big(mode, g, a, st);
+    if ((mode == ROWS_R2C || mode == ROWS_C2R) && rows_big_supported(g)) return launch_rows_big_plain(mode, g, a, st);
+    return launch_rows_generic(mode, g, a, st);
+}
+
+// float64: the generic engine only (no specialised double kernels)
+int launch_rows(RowMode mode, const Geometry& g, const RowArgsT<double>& a, cudaStream_t st) {
+    return launch_rows_generic(mode, g, a, st);
+}
+
 // ------------------------------------------------------------------------------------------ column pass
-template <int MODE>
-__global__ void __launch_bounds__(1024)
-k_cols(ColArgs a, FftPlan plan, int H, int Wc, int T, int ntiles) {
-    extern __shared__ float2 smem[];
-    float2* bufA = smem;
-    float2* bufB = bufA + (size_t)H * T;
-    float2* tw = bufB + (size_t)H * T;
+// Real: float or double (T is the tile width here)
+template <int MODE, typename Real>
+__global__ void __launch_bounds__(kGenericMaxThreads<Real>)
+k_cols(ColArgsT<Real> a, FftPlan plan, int H, int Wc, int T, int ntiles) {
+    using V = cplx_t<Real>;
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    V* bufA = reinterpret_cast<V*>(smem_raw);
+    V* bufB = bufA + (size_t)H * T;
+    V* tw = bufB + (size_t)H * T;
     const int tile = blockIdx.x % ntiles;
     const int p = blockIdx.x / ntiles;
     const int c0 = tile * T;
     const int Tb = min(T, Wc - c0);
     const size_t plane = (size_t)p * H * Wc;
     for (int i = threadIdx.x; i < H; i += blockDim.x) tw[i] = a.tw[i];
-    const float2* in = a.spec_in + plane;
+    const V* in = a.spec_in + plane;
     for (int w = threadIdx.x; w < H * T; w += blockDim.x) {
         const int u = w / T, t = w - u * T;
-        bufA[w] = (t < Tb) ? in[(size_t)u * Wc + c0 + t] : make_float2(0.f, 0.f);
+        bufA[w] = (t < Tb) ? in[(size_t)u * Wc + c0 + t] : make_cplx(Real(0), Real(0));
     }
     __syncthreads();
-    float2* res;
+    V* res;
     if (MODE == COLS_FFT_INV) {
         res = fft_batched<+1>(bufA, bufB, plan, T, T, tw);
     } else if (MODE == COLS_BM_INV || MODE == COLS_CMUL_INV || MODE == COLS_INIT_SPEC) {
@@ -343,33 +397,33 @@ k_cols(ColArgs a, FftPlan plan, int H, int Wc, int T, int ntiles) {
         res = fft_batched<-1>(bufA, bufB, plan, T, T, tw);
     }
     if (MODE == COLS_INIT || MODE == COLS_ITER || MODE == COLS_BM_INV || MODE == COLS_CMUL_INV || MODE == COLS_INIT_SPEC) {
-        float2* other = (res == bufA) ? bufB : bufA;
-        float2* Ap = (MODE == COLS_INIT || MODE == COLS_ITER || MODE == COLS_INIT_SPEC) ? a.A + plane : nullptr;
+        V* other = (res == bufA) ? bufB : bufA;
+        V* Ap = (MODE == COLS_INIT || MODE == COLS_ITER || MODE == COLS_INIT_SPEC) ? a.A + plane : nullptr;
         for (int w = threadIdx.x; w < H * T; w += blockDim.x) {
             const int u = w / T, t = w - u * T;
-            float2 o = make_float2(0.f, 0.f);
+            V o = make_cplx(Real(0), Real(0));
             if (t < Tb) {
                 const int c = c0 + t;
-                const float2 Z = res[w];
+                const V Z = res[w];
                 if (MODE == COLS_ITER || MODE == COLS_BM_INV) {
                     // X = A + Bm F(v)      (deconv.py:104-106 with freq_c, rho folded into A and Bm)
                     // COLS_BM_INV: the same self-adjoint operator without A (backward: vbar = F^-1[Bm F(xbar)])
-                    const float2 Av = (MODE == COLS_ITER) ? Ap[(size_t)u * Wc + c] : make_float2(0.f, 0.f);
-                    const float bm = a.Bm[(size_t)u * Wc + c];
-                    o = make_float2(fmaf(bm, Z.x, Av.x), fmaf(bm, Z.y, Av.y));
+                    const V Av = (MODE == COLS_ITER) ? Ap[(size_t)u * Wc + c] : make_cplx(Real(0), Real(0));
+                    const Real bm = a.Bm[(size_t)u * Wc + c];
+                    o = make_cplx(xfma(bm, Z.x, Av.x), xfma(bm, Z.y, Av.y));
                     if (c == 0) {
                         const int um = (u == 0) ? 0 : H - u;
-                        const float2 Zm = res[um * T + t];
-                        const float bq = a.Bq[u];
-                        o.x = fmaf(bq, Zm.x, o.x);
-                        o.y = fmaf(-bq, Zm.y, o.y);
+                        const V Zm = res[um * T + t];
+                        const Real bq = a.Bq[u];
+                        o.x = xfma(bq, Zm.x, o.x);
+                        o.y = xfma(-bq, Zm.y, o.y);
                     }
                 } else if (MODE == COLS_CMUL_INV) {
                     // adjoint of A = Mul F(y):  ybar = F^-1[conj(Mul) sum_k F(xbar_k)]
                     o = cmul(cconj(a.Mul[(size_t)u * Wc + c]), Z);
                     if (c == 0) {
                         const int um = (u == 0) ? 0 : H - u;
-                        const float2 Zm = res[um * T + t];
+                        const V Zm = res[um * T + t];
                         o = cadd(o, cmul(cconj(a.Mq[u]), cconj(Zm)));
                     }
                 } else {
@@ -377,7 +431,7 @@ k_cols(ColArgs a, FftPlan plan, int H, int Wc, int T, int ntiles) {
                     o = cmul(a.Mul[(size_t)u * Wc + c], Z);
                     if (c == 0) {
                         const int um = (u == 0) ? 0 : H - u;
-                        const float2 Zm = res[um * T + t];
+                        const V Zm = res[um * T + t];
                         o = cadd(o, cmul(a.Mq[u], cconj(Zm)));
                     }
                     Ap[(size_t)u * Wc + c] = o;
@@ -388,33 +442,33 @@ k_cols(ColArgs a, FftPlan plan, int H, int Wc, int T, int ntiles) {
         __syncthreads();
         res = fft_batched<+1>(other, res, plan, T, T, tw);
     }
-    float2* out = a.spec_out + plane;
+    V* out = a.spec_out + plane;
     for (int w = threadIdx.x; w < H * T; w += blockDim.x) {
         const int u = w / T, t = w - u * T;
         if (t < Tb) out[(size_t)u * Wc + c0 + t] = res[w];
     }
 }
 
-static size_t cols_smem(int H, int T) { return ((size_t)2 * H * T + H) * sizeof(float2); }
+template <typename Real>
+static size_t cols_smem(int H, int T) { return ((size_t)2 * H * T + H) * sizeof(cplx_t<Real>); }
 
-int launch_cols(ColMode mode, const Geometry& g, const ColArgs& a, cudaStream_t st) {
-    if (cols_pow2_mode_supported(mode) && cols_pow2_supported(g)) return launch_cols_pow2(mode, g, a, st);
-    if ((mode == COLS_ITER || mode == COLS_INIT) && cols_big_supported(g)) return launch_cols_big(mode, g, a, st);
+template <typename Real>
+static int launch_cols_generic(ColMode mode, const Geometry& g, const ColArgsT<Real>& a, cudaStream_t st) {
     FftPlan plan;
     if (!make_plan(g.H, plan)) return fail(4, "cannot plan column FFT length");
     const size_t kMax = 227 * 1024;
     int T = options().cols_per_tile;
     if (T <= 0) {
         T = 16;
-        while (T > 4 && cols_smem(g.H, T) > 80 * 1024) T >>= 1;       // keep >= 32-byte global runs
+        while (T > 4 && cols_smem<Real>(g.H, T) > 80 * 1024) T >>= 1;       // keep >= 32-byte global runs
     }
-    while (T > 1 && cols_smem(g.H, T) > kMax) T >>= 1;
-    if (cols_smem(g.H, T) > kMax) return fail(4, "column FFT does not fit in shared memory (H too large for the generic kernel)");
+    while (T > 1 && cols_smem<Real>(g.H, T) > kMax) T >>= 1;
+    if (cols_smem<Real>(g.H, T) > kMax) return fail(4, "column FFT does not fit in shared memory (H too large for the generic kernel)");
     T = std::min(T, std::max(1, g.Wc));
     const int ntiles = (g.Wc + T - 1) / T;
-    const size_t smem = cols_smem(g.H, T);
-    const int threads = options().threads > 0 ? options().threads.load()
-                                              : (smem > 113 * 1024 ? 1024 : (smem > 75 * 1024 ? 512 : 256));
+    const size_t smem = cols_smem<Real>(g.H, T);
+    const int threads = std::min(kGenericMaxThreads<Real>, options().threads > 0 ? options().threads.load()
+                                              : (smem > 113 * 1024 ? 1024 : (smem > 75 * 1024 ? 512 : 256)));
     dim3 grid((unsigned)((size_t)ntiles * g.P));
     int dev_id = 0;
     ADMM_CUDA_CHECK(cudaGetDevice(&dev_id));
@@ -422,10 +476,10 @@ int launch_cols(ColMode mode, const Geometry& g, const ColArgs& a, cudaStream_t 
     do {                                                                                                   \
         static std::atomic<bool> attr_set[64];                                                                     \
         if (dev_id >= 64 || !attr_set[dev_id]) {                                                           \
-            ADMM_CUDA_CHECK(cudaFuncSetAttribute(k_cols<M>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMax)); \
+            ADMM_CUDA_CHECK(cudaFuncSetAttribute(k_cols<M, Real>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMax)); \
             if (dev_id < 64) attr_set[dev_id] = true;                                                      \
         }                                                                                                  \
-        k_cols<M><<<grid, threads, smem, st>>>(a, plan, g.H, g.Wc, T, ntiles);                              \
+        k_cols<M, Real><<<grid, threads, smem, st>>>(a, plan, g.H, g.Wc, T, ntiles);                        \
     } while (0)
     ProfScope ps(mode == COLS_ITER ? PROF_COLS : PROF_OTHER, st);
     switch (mode) {
@@ -439,6 +493,36 @@ int launch_cols(ColMode mode, const Geometry& g, const ColArgs& a, cudaStream_t 
     }
 #undef ADMM_LAUNCH_COLS
     ADMM_CUDA_CHECK(cudaGetLastError());
+    return 0;
+}
+
+int launch_cols(ColMode mode, const Geometry& g, const ColArgs& a, cudaStream_t st) {
+    if (cols_pow2_mode_supported(mode) && cols_pow2_supported(g)) return launch_cols_pow2(mode, g, a, st);
+    if ((mode == COLS_ITER || mode == COLS_INIT) && cols_big_supported(g)) return launch_cols_big(mode, g, a, st);
+    return launch_cols_generic(mode, g, a, st);
+}
+
+int launch_cols(ColMode mode, const Geometry& g, const ColArgsT<double>& a, cudaStream_t st) {
+    return launch_cols_generic(mode, g, a, st);
+}
+
+// float64: whether the generic passes of a solve fit in shared memory (the smallest band / tile the launchers above would
+// pick), so that an unsupported size fails before anything is launched
+int check_generic_f64(const Geometry& g, bool full_rows) {
+    const size_t kMax = 227 * 1024;
+    FftPlan plan;
+    if (!make_plan(g.W, plan)) return fail(4, "cannot plan row FFT length");
+    if (!make_plan(g.H, plan)) return fail(4, "cannot plan column FFT length");
+    const int halo = full_rows ? 2 : 0;
+    const size_t rows = rows_smem<double>(g.W, (2 + halo + 1) / 2);
+    if (rows > kMax)
+        return fail(4, "float64 row FFT does not fit in shared memory: W = " + std::to_string(g.W) + " needs " +
+                       std::to_string(rows) + " bytes, the limit is " + std::to_string(kMax) +
+                       (full_rows ? " (iso = 0 keeps two halo rows: W <= 2905)" : " (W <= 4842)"));
+    const size_t cols = cols_smem<double>(g.H, 1);
+    if (cols > kMax)
+        return fail(4, "float64 column FFT does not fit in shared memory: H = " + std::to_string(g.H) + " needs " +
+                       std::to_string(cols) + " bytes, the limit is " + std::to_string(kMax) + " (H <= 4842)");
     return 0;
 }
 

@@ -79,17 +79,20 @@ static size_t carve_backward(const Geometry& g, int ksize, int ckpt, char* base,
 size_t backward_extra_bytes(const Geometry& g, int ksize, int ckpt) { return carve_backward(g, ksize, ckpt, nullptr, nullptr); }
 
 // ------------------------------------------------------------------------------------------ spatial kernels
-__device__ __forceinline__ float qbar_of(float wb, float ub, float q, float tau) {
-    return (fabsf(q) < tau) ? (ub - wb) : wb;          // wbar + m (ubar - 2 wbar)
+// Templated on the real type: float for the solver, double for the float64 solve (f64.cu).
+template <typename T>
+__device__ __forceinline__ T qbar_of(T wb, T ub, T q, T tau) {
+    return (xabs(q) < tau) ? (ub - wb) : wb;          // wbar + m (ubar - 2 wbar)
 }
 
 // adjoint of prox / dual update / gradient for the state produced by iteration k+1
-__global__ void k_bwd_spatial(const float* __restrict__ vb, const float* __restrict__ ubx_in, const float* __restrict__ uby_in,
-                              const float* __restrict__ qx, const float* __restrict__ qy,
-                              float* __restrict__ ubx_out, float* __restrict__ uby_out, float* __restrict__ xb,
-                              const float* __restrict__ lmbd, const float* __restrict__ rho,
+template <typename T>
+__global__ void k_bwd_spatial(const T* __restrict__ vb, const T* __restrict__ ubx_in, const T* __restrict__ uby_in,
+                              const T* __restrict__ qx, const T* __restrict__ qy,
+                              T* __restrict__ ubx_out, T* __restrict__ uby_out, T* __restrict__ xb,
+                              const T* __restrict__ lmbd, const T* __restrict__ rho,
                               double* __restrict__ taubar, int H, int W, size_t total) {
-    const float tau = lmbd[0] / rho[0];
+    const T tau = lmbd[0] / rho[0];
     double tsum = 0.0;
     for (size_t idx = blockIdx.x * (size_t)blockDim.x + threadIdx.x; idx < total; idx += (size_t)gridDim.x * blockDim.x) {
         const int c = (int)(idx % W);
@@ -98,22 +101,22 @@ __global__ void k_bwd_spatial(const float* __restrict__ vb, const float* __restr
         const size_t pl = (rowi / H) * (size_t)H * W;
         const int cl = c == 0 ? W - 1 : c - 1, cr = c == W - 1 ? 0 : c + 1;
         const int ru = r == 0 ? H - 1 : r - 1, rd = r == H - 1 ? 0 : r + 1;
-        const float* V = vb + pl;
-        const float v00 = V[(size_t)r * W + c];
-        const float wbx = v00 - V[(size_t)r * W + cl];                       // (Dx vbar)[r][c]
-        const float wby = v00 - V[(size_t)ru * W + c];                       // (Dy vbar)[r][c]
-        const float wbx_r = V[(size_t)r * W + cr] - v00;                     // (Dx vbar)[r][c+1]
-        const float wby_d = V[(size_t)rd * W + c] - v00;                     // (Dy vbar)[r+1][c]
+        const T* V = vb + pl;
+        const T v00 = V[(size_t)r * W + c];
+        const T wbx = v00 - V[(size_t)r * W + cl];                       // (Dx vbar)[r][c]
+        const T wby = v00 - V[(size_t)ru * W + c];                       // (Dy vbar)[r][c]
+        const T wbx_r = V[(size_t)r * W + cr] - v00;                     // (Dx vbar)[r][c+1]
+        const T wby_d = V[(size_t)rd * W + c] - v00;                     // (Dy vbar)[r+1][c]
         const size_t i00 = pl + (size_t)r * W + c, i0r = pl + (size_t)r * W + cr, id0 = pl + (size_t)rd * W + c;
-        const float ubx = ubx_in ? ubx_in[i00] : 0.f, uby = uby_in ? uby_in[i00] : 0.f;
-        const float ubx_r = ubx_in ? ubx_in[i0r] : 0.f, uby_d = uby_in ? uby_in[id0] : 0.f;
-        const float qx0 = qx[i00], qy0 = qy[i00];
-        const float qbx = qbar_of(wbx, ubx, qx0, tau), qby = qbar_of(wby, uby, qy0, tau);
-        const float qbx_r = qbar_of(wbx_r, ubx_r, qx[i0r], tau), qby_d = qbar_of(wby_d, uby_d, qy[id0], tau);
+        const T ubx = ubx_in ? ubx_in[i00] : T(0), uby = uby_in ? uby_in[i00] : T(0);
+        const T ubx_r = ubx_in ? ubx_in[i0r] : T(0), uby_d = uby_in ? uby_in[id0] : T(0);
+        const T qx0 = qx[i00], qy0 = qy[i00];
+        const T qbx = qbar_of(wbx, ubx, qx0, tau), qby = qbar_of(wby, uby, qy0, tau);
+        const T qbx_r = qbar_of(wbx_r, ubx_r, qx[i0r], tau), qby_d = qbar_of(wby_d, uby_d, qy[id0], tau);
         ubx_out[i00] = qbx; uby_out[i00] = qby;
         xb[i00] = (qbx - qbx_r) + (qby - qby_d);                             // Dx^T qbar_x + Dy^T qbar_y
-        if (fabsf(qx0) >= tau) tsum += (double)((ubx - 2.f * wbx) * (qx0 > 0.f ? 1.f : (qx0 < 0.f ? -1.f : 0.f)));
-        if (fabsf(qy0) >= tau) tsum += (double)((uby - 2.f * wby) * (qy0 > 0.f ? 1.f : (qy0 < 0.f ? -1.f : 0.f)));
+        if (xabs(qx0) >= tau) tsum += (double)((ubx - T(2) * wbx) * (qx0 > T(0) ? T(1) : (qx0 < T(0) ? T(-1) : T(0))));
+        if (xabs(qy0) >= tau) tsum += (double)((uby - T(2) * wby) * (qy0 > T(0) ? T(1) : (qy0 < T(0) ? T(-1) : T(0))));
     }
     // block reduction -> this block's slot (single writer; the launches of a sweep are stream-ordered)
     __shared__ double red[32];
@@ -128,9 +131,10 @@ __global__ void k_bwd_spatial(const float* __restrict__ vb, const float* __restr
 }
 
 // v = Dx^T w_x + Dy^T w_y with w = q - 2 clamp(q)   (recomputed from the saved pre-clamp state; deconv.py:104)
-__global__ void k_bwd_recompute_v(const float* __restrict__ qx, const float* __restrict__ qy, float* __restrict__ v,
-                                  const float* __restrict__ lmbd, const float* __restrict__ rho, int H, int W, size_t total) {
-    const float tau = lmbd[0] / rho[0];
+template <typename T>
+__global__ void k_bwd_recompute_v(const T* __restrict__ qx, const T* __restrict__ qy, T* __restrict__ v,
+                                  const T* __restrict__ lmbd, const T* __restrict__ rho, int H, int W, size_t total) {
+    const T tau = lmbd[0] / rho[0];
     for (size_t idx = blockIdx.x * (size_t)blockDim.x + threadIdx.x; idx < total; idx += (size_t)gridDim.x * blockDim.x) {
         const int c = (int)(idx % W);
         const size_t rowi = idx / W;
@@ -139,7 +143,7 @@ __global__ void k_bwd_recompute_v(const float* __restrict__ qx, const float* __r
         const int cr = c == W - 1 ? 0 : c + 1, rd = r == H - 1 ? 0 : r + 1;
         // same operations in the same order as the forward's fused spatial step (rows_pow2.cu, admm_kernels.cu), so a
         // checkpointed backward that restarts the forward from a saved state reproduces its fields bit for bit
-        auto wf = [tau](float q) { return fmaf(-2.0f, dual_any(q, tau), q); };
+        auto wf = [tau](T q) { return xfma(T(-2), dual_any(q, tau), q); };
         const size_t i00 = pl + (size_t)r * W + c;
         v[i00] = wf(qx[i00]) - wf(qx[pl + (size_t)r * W + cr]) + wf(qy[i00]) - wf(qy[pl + (size_t)rd * W + c]);
     }
@@ -147,16 +151,19 @@ __global__ void k_bwd_recompute_v(const float* __restrict__ qx, const float* __r
 
 // ------------------------------------------------------------------------------------------ spectral accumulation
 // Full-spectrum entry (u, v), v in [0, W/2], from a packed column-transformed spectrum (column 0 = DC + i Nyquist).
-__device__ __forceinline__ float2 unpack_spec(const float2* __restrict__ Z, int u, int v, int H, int Wc) {
+template <typename V>
+__device__ __forceinline__ V unpack_spec(const V* __restrict__ Z, int u, int v, int H, int Wc) {
+    using T = real_t<V>;
     if (v >= 1 && v < Wc) return Z[(size_t)u * Wc + v];
-    const float2 z0 = Z[(size_t)u * Wc];
-    const float2 zm = Z[(size_t)((H - u) % H) * Wc];          // conj applied below
-    if (v == 0) return make_float2(0.5f * (z0.x + zm.x), 0.5f * (z0.y - zm.y));
-    return make_float2(0.5f * (z0.y + zm.y), -0.5f * (z0.x - zm.x));   // Nyquist column: (z0 - conj(zm)) / (2i)
+    const V z0 = Z[(size_t)u * Wc];
+    const V zm = Z[(size_t)((H - u) % H) * Wc];               // conj applied below
+    if (v == 0) return make_cplx(T(0.5) * (z0.x + zm.x), T(0.5) * (z0.y - zm.y));
+    return make_cplx(T(0.5) * (z0.y + zm.y), T(-0.5) * (z0.x - zm.x));   // Nyquist column: (z0 - conj(zm)) / (2i)
 }
 
-__global__ void k_bwd_accumulate(const float2* __restrict__ ZG, const float2* __restrict__ ZV, const float2* __restrict__ ZY,
-                                 float2* __restrict__ Gs, double2* __restrict__ C1, double2* __restrict__ GV,
+template <typename V>
+__global__ void k_bwd_accumulate(const V* __restrict__ ZG, const V* __restrict__ ZV, const V* __restrict__ ZY,
+                                 V* __restrict__ Gs, double2* __restrict__ C1, double2* __restrict__ GV,
                                  int P, int H, int W, int Wc, int update_gs) {
     // blockIdx.y splits the planes into gridDim.y groups; group y owns slice y of C1 / GV (single writer per entry,
     // accumulated over the stream-ordered launches of a sweep); k_bwd_finalize adds the slices in a fixed order
@@ -170,20 +177,20 @@ __global__ void k_bwd_accumulate(const float2* __restrict__ ZG, const float2* __
         const size_t pl = (size_t)p * H * Wc;
         if (update_gs && v < Wc) {
             const size_t e = pl + (size_t)u * Wc + v;
-            const float2 g = ZG[e];
-            float2 s = Gs[e];
+            const V g = ZG[e];
+            V s = Gs[e];
             s.x += g.x; s.y += g.y;
             Gs[e] = s;
         }
         if (ZY || ZV) {
-            const float2 g = unpack_spec(ZG + pl, u, v, H, Wc);
+            const V g = unpack_spec(ZG + pl, u, v, H, Wc);
             if (ZY) {
-                const float2 y = unpack_spec(ZY + pl, u, v, H, Wc);
+                const V y = unpack_spec(ZY + pl, u, v, H, Wc);
                 c1x += (double)g.x * y.x + (double)g.y * y.y;             // conj(g) * y
                 c1y += (double)g.x * y.y - (double)g.y * y.x;
             }
             if (ZV) {
-                const float2 w = unpack_spec(ZV + pl, u, v, H, Wc);
+                const V w = unpack_spec(ZV + pl, u, v, H, Wc);
                 gvx += (double)g.x * w.x + (double)g.y * w.y;
                 gvy += (double)g.x * w.y - (double)g.y * w.x;
             }
@@ -211,10 +218,11 @@ __global__ void k_bwd_reduce_gv(const float2* __restrict__ GVp, const float2* __
 }
 
 // rho gradient (spectral part) and the kernel-gradient spectrum S(u, v)
+template <typename T>
 __global__ void k_bwd_finalize(const double2* __restrict__ C1, const double2* __restrict__ GV, int nsplit, double2* __restrict__ S,
                                double* __restrict__ rho_part, int H, int W, int ks, const double2* __restrict__ G,
                                const double2* __restrict__ twHd, const double2* __restrict__ twWd,
-                               const float* __restrict__ rho_p) {
+                               const T* __restrict__ rho_p) {
     const int Wh = W / 2 + 1;
     const int idx = blockIdx.x * blockDim.x + threadIdx.x;
     double term = 0.0;
@@ -272,7 +280,8 @@ __global__ void k_bwd_kgrad_rows(const double2* __restrict__ S, double2* __restr
 }
 
 // gk[a][b] = sum_u Re(Tk[u][b] e^{+2 pi i u a / H})
-__global__ void k_bwd_kgrad_cols(const double2* __restrict__ Tk, float* __restrict__ gk, int H, int ks,
+template <typename T>
+__global__ void k_bwd_kgrad_cols(const double2* __restrict__ Tk, T* __restrict__ gk, int H, int ks,
                                  const double2* __restrict__ twHd) {
     const int idx = blockIdx.x * blockDim.x + threadIdx.x;
     if (idx >= ks * ks) return;
@@ -283,7 +292,7 @@ __global__ void k_bwd_kgrad_cols(const double2* __restrict__ Tk, float* __restri
         const double2 w = twHd[(int)(((long long)u * a) % H)];
         acc += t.x * w.x + t.y * w.y;                                   // Re(t * conj(w))
     }
-    gk[idx] = (float)acc;
+    gk[idx] = (T)acc;
 }
 
 // fixed-order sum of n doubles by one block of 256 threads (strided partials, then a tree)
@@ -301,21 +310,78 @@ __device__ double block_sum_256(const double* __restrict__ v, size_t n, double* 
     return r;
 }
 
+template <typename T>
 __global__ void __launch_bounds__(256)
 k_bwd_scalars(const double* __restrict__ tau_part, size_t n_tau, const double* __restrict__ rho_part, size_t n_rho,
-              const float* __restrict__ lmbd, const float* __restrict__ rho, float* __restrict__ grad_lmbd,
-              float* __restrict__ grad_rho) {
+              const T* __restrict__ lmbd, const T* __restrict__ rho, T* __restrict__ grad_lmbd,
+              T* __restrict__ grad_rho) {
     __shared__ double red[256];
     const double taubar = block_sum_256(tau_part, n_tau, red);
     const double rhospec = block_sum_256(rho_part, n_rho, red);
     if (threadIdx.x == 0) {
         const double lam = lmbd[0], r = rho[0];
-        if (grad_lmbd) grad_lmbd[0] = (float)(taubar / r);
-        if (grad_rho) grad_rho[0] = (float)(rhospec - taubar * lam / (r * r));
+        if (grad_lmbd) grad_lmbd[0] = (T)(taubar / r);
+        if (grad_rho) grad_rho[0] = (T)(rhospec - taubar * lam / (r * r));
     }
 }
 
 static int ew_grid(size_t total) { return (int)std::min<size_t>((total + 255) / 256, 148 * 16); }
+
+// ---- the same kernels in double, for the float64 backward (f64.cu); launch shapes as in run_backward below
+int launch_bwd_spatial(const Geometry& g, const double* vb, const double* ubx_in, const double* uby_in, const double* qx,
+                       const double* qy, double* ubx_out, double* uby_out, double* xb, const double* lmbd, const double* rho,
+                       double* taubar, cudaStream_t st) {
+    ProfScope ps(PROF_OTHER, st);
+    const size_t fe = (size_t)g.P * g.H * g.W;
+    k_bwd_spatial<<<ew_grid(fe), 256, 0, st>>>(vb, ubx_in, uby_in, qx, qy, ubx_out, uby_out, xb, lmbd, rho, taubar, g.H, g.W, fe);
+    ADMM_CUDA_CHECK(cudaGetLastError());
+    return 0;
+}
+
+int launch_bwd_recompute_v(const Geometry& g, const double* qx, const double* qy, double* v, const double* lmbd,
+                           const double* rho, cudaStream_t st) {
+    ProfScope ps(PROF_OTHER, st);
+    const size_t fe = (size_t)g.P * g.H * g.W;
+    k_bwd_recompute_v<<<ew_grid(fe), 256, 0, st>>>(qx, qy, v, lmbd, rho, g.H, g.W, fe);
+    ADMM_CUDA_CHECK(cudaGetLastError());
+    return 0;
+}
+
+int launch_bwd_accumulate(const Geometry& g, int nsplit, const double2* ZG, const double2* ZV, const double2* ZY, double2* Gs,
+                          double2* C1, double2* GV, int update_gs, cudaStream_t st) {
+    ProfScope ps(PROF_OTHER, st);
+    const int HWh = g.H * (g.W / 2 + 1);
+    k_bwd_accumulate<<<dim3((HWh + 127) / 128, nsplit), 128, 0, st>>>(ZG, ZV, ZY, Gs, C1, GV, g.P, g.H, g.W, g.Wc, update_gs);
+    ADMM_CUDA_CHECK(cudaGetLastError());
+    return 0;
+}
+
+int launch_bwd_finalize(const Geometry& g, const double2* C1, const double2* GV, int nsplit, double2* S, double* rho_part,
+                        int ks, const double2* G, const double2* twHd, const double2* twWd, const double* rho, cudaStream_t st) {
+    ProfScope ps(PROF_OTHER, st);
+    const int HWh = g.H * (g.W / 2 + 1);
+    k_bwd_finalize<<<(HWh + 127) / 128, 128, 0, st>>>(C1, GV, nsplit, S, rho_part, g.H, g.W, ks, G, twHd, twWd, rho);
+    ADMM_CUDA_CHECK(cudaGetLastError());
+    return 0;
+}
+
+int launch_bwd_kgrad(const Geometry& g, const double2* S, double2* Tk, int ks, const double2* twWd, const double2* twHd,
+                     double* grad_kern, cudaStream_t st) {
+    ProfScope ps(PROF_OTHER, st);
+    k_bwd_kgrad_rows<<<(g.H * ks + 127) / 128, 128, 0, st>>>(S, Tk, g.H, g.W, ks, twWd);
+    ADMM_CUDA_CHECK(cudaGetLastError());
+    k_bwd_kgrad_cols<<<(ks * ks + 63) / 64, 64, 0, st>>>(Tk, grad_kern, g.H, ks, twHd);
+    ADMM_CUDA_CHECK(cudaGetLastError());
+    return 0;
+}
+
+int launch_bwd_scalars(const double* tau_part, size_t n_tau, const double* rho_part, size_t n_rho, const double* lmbd,
+                       const double* rho, double* grad_lmbd, double* grad_rho, cudaStream_t st) {
+    ProfScope ps(PROF_OTHER, st);
+    k_bwd_scalars<<<1, 256, 0, st>>>(tau_part, n_tau, rho_part, n_rho, lmbd, rho, grad_lmbd, grad_rho);
+    ADMM_CUDA_CHECK(cudaGetLastError());
+    return 0;
+}
 
 int run_backward(const Geometry& g, const Workspace& ws, const BwdWorkspace& bw, const float* y, const float* grad_out,
                  const float* kern, int ksize, const float* lmbd, const float* rho, int maxit, const float* saved,
@@ -500,7 +566,7 @@ int run_backward(const Geometry& g, const Workspace& ws, const BwdWorkspace& bw,
                 ProfScope ps(PROF_OTHER, st);
                 const dim3 grid((HWh + 127) / 128, bw.nsplit);
                 // C1 = sum_planes conj(sum_k G_k) F(y) is formed once after the sweep from Gs; only GV needs every iteration
-                k_bwd_accumulate<<<grid, 128, 0, st>>>(bw.ZG, ZV, nullptr, bw.Gs, bw.C1, bw.GV, g.P, g.H, g.W, g.Wc, 1);
+                k_bwd_accumulate<float2><<<grid, 128, 0, st>>>(bw.ZG, ZV, nullptr, bw.Gs, bw.C1, bw.GV, g.P, g.H, g.W, g.Wc, 1);
                 ADMM_CUDA_CHECK(cudaGetLastError());
             }
             if (k > 0) {                                        // vbar = F^-1[Bm G]
@@ -522,7 +588,7 @@ int run_backward(const Geometry& g, const Workspace& ws, const BwdWorkspace& bw,
     if (need_spec) {                                            // C1 = sum_planes conj(Gs) F(y) / (HW)
         ProfScope ps(PROF_OTHER, st);
         const dim3 grid((HWh + 127) / 128, bw.nsplit);
-        k_bwd_accumulate<<<grid, 128, 0, st>>>(bw.Gs, nullptr, ZY, bw.Gs, bw.C1, bw.GV, g.P, g.H, g.W, g.Wc, 0);
+        k_bwd_accumulate<float2><<<grid, 128, 0, st>>>(bw.Gs, nullptr, ZY, bw.Gs, bw.C1, bw.GV, g.P, g.H, g.W, g.Wc, 0);
         ADMM_CUDA_CHECK(cudaGetLastError());
     }
     if (grad_y) {                                               // ybar = F^-1[conj(sigma ph / den) Gs]

@@ -102,6 +102,12 @@ __device__ __forceinline__ float dual_of(float q, float tau) {
     return fminf(fmaxf(q, -tau), tau);
 }
 __device__ __forceinline__ float dual_any(float q, float tau) { return tau < 0.f ? dual_of<true>(q, tau) : dual_of<false>(q, tau); }
+template <bool NEG>
+__device__ __forceinline__ double dual_of(double q, double tau) {
+    if (NEG) return q > 0.0 ? tau : (q < 0.0 ? -tau : 0.0);
+    return fmin(fmax(q, -tau), tau);
+}
+__device__ __forceinline__ double dual_any(double q, double tau) { return tau < 0.0 ? dual_of<true>(q, tau) : dual_of<false>(q, tau); }
 struct TauPos { static constexpr bool neg = false; };
 struct TauNeg { static constexpr bool neg = true; };
 
@@ -140,35 +146,41 @@ enum RowMode { ROWS_R2C = 0, ROWS_C2R = 1, ROWS_FULL = 2, ROWS_ADJ = 3, ROWS_FUL
 // COLS_INIT_SPEC: like COLS_INIT but the input already is the column-transformed spectrum of y (shared by several solvers)
 enum ColMode { COLS_FFT_FWD = 0, COLS_FFT_INV = 1, COLS_INIT = 2, COLS_ITER = 3, COLS_BM_INV = 4, COLS_CMUL_INV = 5, COLS_INIT_SPEC = 6 };
 
-struct RowArgs {
-    const float*  real_in;    // ROWS_R2C: input rows
-    float*        real_out;   // ROWS_C2R: output rows
-    const float2* spec_in;    // ROWS_C2R / ROWS_FULL
-    float2*       spec_out;   // ROWS_R2C / ROWS_FULL
-    const float*  qx_in; const float* qy_in;     // ROWS_FULL: previous pre-clamp state (NULL = zeros)
-    float*        qx_out; float* qy_out;         // ROWS_FULL
-    const float*  lmbd; const float* rho;        // ROWS_FULL: tau = lmbd/rho
-    const float*  bias;                          // ROWS_C2R: optional scalar added to the output
+// Arguments of the row and column passes, templated on the real type: T = float for the solver, T = double for the
+// float64 solve (f64.cu, generic kernels only).  V = cplx_t<T>.
+template <typename T>
+struct RowArgsT {
+    using V = cplx_t<T>;
+    const T*      real_in;    // ROWS_R2C: input rows
+    T*            real_out;   // ROWS_C2R: output rows
+    const V*      spec_in;    // ROWS_C2R / ROWS_FULL
+    V*            spec_out;   // ROWS_R2C / ROWS_FULL
+    const T*      qx_in; const T* qy_in;         // ROWS_FULL: previous pre-clamp state (NULL = zeros)
+    T*            qx_out; T* qy_out;             // ROWS_FULL
+    const T*      lmbd; const T* rho;            // ROWS_FULL: tau = lmbd/rho
+    const T*      bias;                          // ROWS_C2R: optional scalar added to the output
     // fused prologue / epilogue of the layer (admm_ext, include/admm_b200.h):
     const unsigned char* real_in_u8;             // ROWS_R2C: uint8 input; the transform sees (float)v / 255 (etransforms.py:29-31)
     int           act;                           // ROWS_C2R: activation on (x + bias) (admmdeconv.py:64): 0 none, 1 relu, 2 sigmoid, 3 tanh
+                                                 // (float only: the float64 solve ignores it)
     int           out_C;                         // ROWS_C2R with out_bstride != 0: plane p goes to
     long long     out_bstride;                   //   real_out + (p / out_C) * out_bstride + (p % out_C) * H * W   (channel slice of a wider tensor)
     int           out_p0;                        // ROWS_C2R: index of this launch's first plane in the whole batch (plane chunks)
-    const float*  cmap;                          // ROWS_R2C with r2c_div (power-of-two sizes): coefficient maps 2s-1 (2 x H x W),
+    const T*      cmap;                          // ROWS_R2C with r2c_div (power-of-two sizes): coefficient maps 2s-1 (2 x H x W),
                                                  // NULL = all ones
     int           r2c_div;                       // ROWS_R2C: the input is v = D^T(cmap * q) built from qx_in / qy_in on the fly
     // ROWS_ADJ (backward sweep, one fused row pass): spec_in = row spectrum of vbar, qx_in/qy_in = saved q_{k+1},
     // ub*_in = ubar (NULL = zeros), ub*_out = new ubar (= qbar), spec_out = row spectrum of xbar = D^T qbar,
     // taubar accumulates d/dtau; optional second output: qv* = saved q_k -> spec_out2 = row spectrum of v_k
-    const float*  ubx_in; const float* uby_in;
-    float*        ubx_out; float* uby_out;
+    const T*      ubx_in; const T* uby_in;
+    T*            ubx_out; T* uby_out;
     double*       taubar;
-    const float*  qvx; const float* qvy;
-    float2*       spec_out2;
-    const float2* tw;
+    const T*      qvx; const T* qvy;
+    V*            spec_out2;
+    const V*      tw;
     int tiled;                // large kernels: spec_in / spec_out are tile-major (see kSpecTile)
 };
+using RowArgs = RowArgsT<float>;
 
 // Tile-major packed spectrum shared by the two large-frame kernels (rows_big.cu <-> cols_big.cu): per plane
 // [tile = col / 8][row pair][col % 8][row in pair] float2.  One row pair of one tile is a 128-byte run for the row kernel
@@ -177,17 +189,20 @@ struct RowArgs {
 // (2k, 2k+1); the spectrum of x (columns -> rows) pairs rows (2k-1, 2k), the pairs the row kernel transforms together.
 constexpr int kSpecTile = 8;
 
-struct ColArgs {
-    const float2* spec_in;
-    float2*       spec_out;
-    float2*       A;          // COLS_INIT: written; COLS_ITER: read.  Private to a kernel family: the power-of-two kernels keep
+template <typename T>
+struct ColArgsT {
+    using V = cplx_t<T>;
+    const V*      spec_in;
+    V*            spec_out;
+    V*            A;          // COLS_INIT: written; COLS_ITER: read.  Private to a kernel family: the power-of-two kernels keep
                               // P0[A] (A after their first inverse pass, cols_pow2_body.cuh), cols_big.cu a tile-major A
-    const float*  Bm; const float* Bq;
-    const float*  Bmt;        // large column kernel: Bm as [tile][u][4] (A is kept in the same layout there)
-    const float2* Mul; const float2* Mq;
-    const float2* tw;
+    const T*      Bm; const T* Bq;
+    const T*      Bmt;        // large column kernel: Bm as [tile][u][4] (A is kept in the same layout there)
+    const V*      Mul; const V* Mq;
+    const V*      tw;
     int in_tiled, out_tiled;  // large column kernel: layout of spec_in / spec_out
 };
+using ColArgs = ColArgsT<float>;
 
 int launch_twiddles(float2* tw, double2* twd, int N, cudaStream_t st);
 int launch_tables(const Geometry& g, const Workspace& ws, const float* kern, int ksize,
@@ -210,6 +225,37 @@ int launch_iso_div(const Geometry& g, const float* qx, const float* qy, const fl
 int launch_iso_bwd(const Geometry& g, const float* vb, const float* ubx_in, const float* uby_in, const float* qx,
                    const float* qy, const float* nmap, float* sbmap, float* ubx_out, float* uby_out, float* xb,
                    const float* lmbd, const float* rho, double* taubar, cudaStream_t st);
+
+// ------------------------------------------------------------------ float64 solve (f64.cu): the generic kernels in double
+int launch_twiddles_f64(double2* twd, int N, cudaStream_t st);
+int launch_tables_f64(const Geometry& g, const double2* twWd, const double2* twHd, double2* kdft, double* Bm, double* Bq,
+                      double2* Mul, double2* Mq, const double* kern, int ksize, const double* rho, cudaStream_t st);
+int launch_rows(RowMode mode, const Geometry& g, const RowArgsT<double>& a, cudaStream_t st);   // R2C, C2R, FULL
+int launch_cols(ColMode mode, const Geometry& g, const ColArgsT<double>& a, cudaStream_t st);
+int check_generic_f64(const Geometry& g, bool full_rows);       // 0, or ADMM_ERR_UNSUPPORTED with a message
+int launch_iso_prox(const Geometry& g, const double* x, const double* qx_prev, const double* qy_prev, const double* n_prev,
+                    double* qx_new, double* qy_new, double* n_new, double* c_new, const double* lmbd, const double* rho,
+                    cudaStream_t st);
+int launch_iso_cmap(const Geometry& g, const double* nmap, double* cmap, const double* lmbd, const double* rho, cudaStream_t st);
+int launch_iso_div(const Geometry& g, const double* qx, const double* qy, const double* nmap, const double* cmap, double* v,
+                   const double* lmbd, const double* rho, cudaStream_t st);
+int launch_iso_bwd(const Geometry& g, const double* vb, const double* ubx_in, const double* uby_in, const double* qx,
+                   const double* qy, const double* nmap, double* sbmap, double* ubx_out, double* uby_out, double* xb,
+                   const double* lmbd, const double* rho, double* taubar, cudaStream_t st);
+// backward.cu: the generic backward kernels in double (the float solver launches them itself)
+int launch_bwd_spatial(const Geometry& g, const double* vb, const double* ubx_in, const double* uby_in, const double* qx,
+                       const double* qy, double* ubx_out, double* uby_out, double* xb, const double* lmbd, const double* rho,
+                       double* taubar, cudaStream_t st);
+int launch_bwd_recompute_v(const Geometry& g, const double* qx, const double* qy, double* v, const double* lmbd,
+                           const double* rho, cudaStream_t st);
+int launch_bwd_accumulate(const Geometry& g, int nsplit, const double2* ZG, const double2* ZV, const double2* ZY, double2* Gs,
+                          double2* C1, double2* GV, int update_gs, cudaStream_t st);
+int launch_bwd_finalize(const Geometry& g, const double2* C1, const double2* GV, int nsplit, double2* S, double* rho_part,
+                        int ks, const double2* G, const double2* twHd, const double2* twWd, const double* rho, cudaStream_t st);
+int launch_bwd_kgrad(const Geometry& g, const double2* S, double2* Tk, int ks, const double2* twWd, const double2* twHd,
+                     double* grad_kern, cudaStream_t st);
+int launch_bwd_scalars(const double* tau_part, size_t n_tau, const double* rho_part, size_t n_rho, const double* lmbd,
+                       const double* rho, double* grad_lmbd, double* grad_rho, cudaStream_t st);
 
 // specialised power-of-two kernels (rows_pow2.cu, cols_pow2.cu)
 bool rows_pow2_supported(const Geometry& g);

@@ -38,6 +38,7 @@ def convert_admm_layer(ref: torch.nn.Module) -> ADMMDeconv:
     new.iso = ref.iso
     new.activation = ref.activation
     new.ckpt_interval = 0
+    new.precision = "float32"
     new.train(ref.training)
     return new
 

@@ -11,7 +11,7 @@ from typing import Callable, Tuple
 
 import torch
 
-from ..eops.deconv import admm_solve, identity
+from ..eops.deconv import admm_solve, fft_admm_tv_f64, identity
 
 __all__ = ["ADMMDeconv"]
 
@@ -45,6 +45,9 @@ class ADMMDeconv(torch.nn.Module):
         # not a constructor argument of the reference: set `layer.ckpt_interval = K` (or -1 for sqrt(max_iters)) to train
         # with checkpointed state (see admm_solve); 0 keeps the state of every iteration
         self.ckpt_interval = 0
+        # not a constructor argument either: "float64" solves in double (fft_admm_tv_f64) for a model converted with
+        # `.double()`, like the reference does for float64 inputs; "float32" (default) is the fused float32 path
+        self.precision = "float32"
 
     def _scalar(self, name: str, value):
         """Falsy (None or 0) -> learnable U(0,1) Parameter of shape (1,); else a fixed fp32 buffer."""
@@ -56,6 +59,14 @@ class ADMMDeconv(torch.nn.Module):
             self.register_buffer(name, torch.tensor([value], dtype=torch.float32))
 
     def forward(self, x: torch.Tensor, out: torch.Tensor = None, yhat: torch.Tensor = None) -> torch.Tensor:
+        precision = getattr(self, "precision", "float32")
+        if precision == "float64":
+            # admmdeconv.py:63-64 in double: the bias and the activation run in torch (the float64 solve fuses neither)
+            if out is not None or yhat is not None:
+                raise ValueError("out / yhat are float32-path options; not available with precision = 'float64'")
+            return self.activation(fft_admm_tv_f64(x, self.lmbda, self.rho, self.w, self.iso, self.max_iters) + self.b)
+        if precision != "float32":
+            raise ValueError("ADMMDeconv.precision must be 'float32' or 'float64', got %r" % (precision,))
         # activation(fft_admm_tv(x, lmbda, rho, w, iso, max_iters) + b)   (admmdeconv.py:63-64): the scalar bias and an
         # identity / relu / sigmoid / tanh activation are applied by the last kernel of the solve; any other callable
         # runs afterwards.  A uint8 image batch is read as x / 255 by the first kernel (etransforms.py:29-31).

@@ -18,7 +18,7 @@ import torch.nn.functional as F
 from .. import _lib
 
 __all__ = ["fft_admm_tv", "soft_thresh", "block_thresh", "pixelnorm", "hard_thresh", "torch_abs2", "identity",
-           "conv_circular", "admm_solve", "activation_code", "shared_spectrum", "fft_admm_tv_cast"]
+           "conv_circular", "admm_solve", "activation_code", "shared_spectrum", "fft_admm_tv_cast", "fft_admm_tv_f64"]
 
 
 # ------------------------------------------------------------------------------------------------
@@ -346,7 +346,7 @@ def fft_admm_tv_cast(xin: torch.Tensor, lmbd, rho, kern, iso: bool = False, maxi
     deconv.py:50-67): the sm_100a kernels compute in float32, so the input is cast to float32, solved, and the result
     cast back to `xin.dtype`; gradients flow through the casts.  The result then carries float32 accuracy (~1e-6
     relative to a float64 run of the reference), which is why this is an explicit opt-in and `fft_admm_tv` itself
-    raises TypeError for other dtypes (INTEGRATION.md, "dtypes")."""
+    raises TypeError for other dtypes (INTEGRATION.md, "dtypes").  `fft_admm_tv_f64` solves float64 in double."""
     dt = xin.dtype
     f = lambda t: t.to(torch.float32) if torch.is_tensor(t) and t.is_floating_point() else t
     return fft_admm_tv(f(xin), f(lmbd), f(rho), f(kern), iso, maxit).to(dt)
@@ -370,3 +370,106 @@ def fft_admm_tv(xin: torch.Tensor,
     rho and kern through a hand-written backward (no autograd graph over the iterations is kept).
     """
     return admm_solve(xin, lmbd, rho, kern, iso, maxit, None)
+
+
+# ------------------------------------------------------------------------------------------------
+# float64 solve (admm_*_f64 of include/admm_b200.h: the generic kernels instantiated for double)
+# ------------------------------------------------------------------------------------------------
+class _AdmmTV64(torch.autograd.Function):
+    """float64 `fft_admm_tv`; every tensor argument is a float64 tensor on xin's device (fft_admm_tv_f64 casts)."""
+
+    @staticmethod
+    def forward(ctx, xin, lmbd, rho, kern, iso, maxit, need_grad):
+        lib = _lib.load()
+        B, C, H, W = xin.shape
+        dev = xin.device
+        ksize = int(kern.shape[2]) if kern.numel() else 0
+        x = xin.contiguous()
+        lam_d = lmbd.detach().reshape(1).contiguous()
+        rho_d = rho.detach().reshape(1).contiguous()
+        kern_d = kern.detach().reshape(ksize, ksize).contiguous() if ksize else None
+        out = torch.empty((B, C, H, W), dtype=torch.float64, device=dev)
+        with torch.cuda.device(dev):
+            ws_bytes = lib.admm_query_workspace_f64(B * C, H, W, ksize, int(iso), maxit)
+            if ws_bytes == 0:
+                _lib.check(1, "admm_query_workspace_f64")
+            ws = _workspace(ws_bytes, dev)
+            saved = None
+            saved_bytes = 0
+            if need_grad:
+                saved_bytes = lib.admm_query_saved_f64(B * C, H, W, ksize, int(iso), maxit)
+                saved = _workspace(saved_bytes, dev)
+            stream = torch.cuda.current_stream(dev).cuda_stream
+            st = lib.admm_tv_forward_f64(_ptr(x), _ptr(out), _ptr(kern_d), ksize, _ptr(lam_d), _ptr(rho_d),
+                                         B, C, H, W, int(iso), maxit, _ptr(ws), ws.numel(), _ptr(saved), saved_bytes,
+                                         ctypes.c_void_p(stream))
+            _lib.check(st, "admm_tv_forward_f64")
+        if need_grad:
+            ctx.save_for_backward(x, lam_d, rho_d, kern_d if kern_d is not None else x.new_empty(0), saved)
+            ctx.cfg = (ksize, bool(iso), int(maxit), tuple(kern.shape), tuple(lmbd.shape), tuple(rho.shape))
+        return out
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, grad_out):
+        lib = _lib.load()
+        x, lam_d, rho_d, kern_d, saved = ctx.saved_tensors
+        ksize, iso, maxit, kshape, lshape, rshape = ctx.cfg
+        B, C, H, W = x.shape
+        dev = x.device
+        g = grad_out.to(torch.float64).contiguous()
+        need_x, need_l, need_r, need_k = ctx.needs_input_grad[:4]
+        gx = torch.empty_like(x) if need_x else None
+        gl = torch.zeros(1, dtype=torch.float64, device=dev) if need_l else None
+        gr = torch.zeros(1, dtype=torch.float64, device=dev) if need_r else None
+        gk = torch.zeros(ksize, ksize, dtype=torch.float64, device=dev) if (need_k and ksize) else None
+        with torch.cuda.device(dev):
+            ws = _workspace(lib.admm_query_workspace_backward_f64(B * C, H, W, ksize, int(iso), maxit), dev)
+            stream = torch.cuda.current_stream(dev).cuda_stream
+            st = lib.admm_tv_backward_f64(_ptr(x), _ptr(g), _ptr(kern_d if ksize else None), ksize, _ptr(lam_d), _ptr(rho_d),
+                                          B, C, H, W, int(iso), maxit, _ptr(saved), saved.numel(), _ptr(ws), ws.numel(),
+                                          _ptr(gx), _ptr(gk), _ptr(gl), _ptr(gr), ctypes.c_void_p(stream))
+            _lib.check(st, "admm_tv_backward_f64")
+        return (gx,
+                gl.reshape(lshape) if gl is not None else None,
+                gr.reshape(rshape) if gr is not None else None,
+                gk.reshape(kshape) if gk is not None else None,
+                None, None, None)
+
+
+def _f64_scalar(v, device, name):
+    if not torch.is_tensor(v):
+        return torch.tensor([float(v)], dtype=torch.float64, device=device)
+    if v.numel() != 1:
+        raise ValueError("%s must hold exactly one element, got shape %s" % (name, tuple(v.shape)))
+    return v.to(device=device, dtype=torch.float64)
+
+
+def fft_admm_tv_f64(xin: torch.Tensor, lmbd, rho, kern, iso: bool = False, maxit: int = 100) -> torch.Tensor:
+    """`fft_admm_tv` in float64: the reference's semantics for a float64 `xin` (it computes in xin.dtype,
+    deconv.py:50-67), solved in double by the generic sm_100a kernels instantiated for double.
+
+    xin   (B, C, H, W) float64 CUDA tensor (anything else raises TypeError)
+    lmbd, rho, kern   as for `fft_admm_tv`, any floating dtype: they are cast to float64 here, so autograd returns their
+          gradients in their own dtype
+    Differentiable w.r.t. xin, lmbd, rho and kern (hand-written adjoint in double).  Work is enqueued on the current
+    stream without a host sync.  Size limits (shared memory of the generic kernels): H <= 4842, and W <= 2905 for
+    iso=False (W <= 4842 for iso=True); larger frames raise RuntimeError.  No fused bias / activation / uint8 input."""
+    if not torch.is_tensor(xin) or xin.dtype != torch.float64:
+        raise TypeError("fft_admm_tv_f64 takes a float64 tensor (got %s); fft_admm_tv is the float32 entry point"
+                        % (xin.dtype if torch.is_tensor(xin) else type(xin).__name__))
+    if not xin.is_cuda:
+        raise TypeError("fft_admm_tv_f64 takes a CUDA tensor: there is no CPU fallback")
+    if xin.dim() != 4:
+        raise ValueError("xin must be 4-D (B, C, H, W), got %d-D" % xin.dim())
+    dev = xin.device
+    maxit = int(maxit)
+    lmbd = _f64_scalar(lmbd, dev, "lmbd")
+    rho = _f64_scalar(rho, dev, "rho")
+    if kern is None or kern.numel() == 0:
+        kern = xin.new_empty(0)
+    else:
+        _prep_kernel(kern)                             # shape checks: (1, 1, k, k), square
+        kern = kern.to(device=dev, dtype=torch.float64)
+    need_grad = torch.is_grad_enabled() and any(t.requires_grad for t in (xin, lmbd, rho, kern))
+    return _AdmmTV64.apply(xin, lmbd, rho, kern, bool(iso), maxit, need_grad)
