@@ -82,7 +82,8 @@ typedef struct admm_ext {
     int       activation;        /* ADMM_ACT_*: out = act(x + bias), applied by the last row pass (admmdeconv.py:64) */
     int       ckpt_interval;     /* training only: K >= 2 keeps the per-iteration state of every K-th iteration instead of all of
                                     them (memory / recompute trade: the backward re-runs each block of K iterations from its
-                                    checkpoint).  0 or 1 = keep every iteration.  iso = 0 only.  Sizes: admm_query_saved_ex,
+                                    checkpoint).  0 or 1 = keep every iteration.  iso = 0 only (every frame size, the large
+                                    frames of the tile-major kernels included).  Sizes: admm_query_saved_ex,
                                     admm_query_workspace_backward_ex; pass the same K to admm_tv_backward_ex. */
     long long out_batch_stride;  /* floats between consecutive images of `out`; 0 = dense (C*H*W).  With a larger stride the
                                     C planes of image b land at out + b*stride: the channel slice of a concatenated tensor

@@ -127,8 +127,9 @@ static int check_kernel(int ksize, int H, int W) {
 }
 
 int make_geometry_pub(int planes, int H, int W, Geometry* g) { return make_geometry(planes, H, W, g); }
-// checkpointed training re-runs blocks of the forward inside the backward; kept to the row-major spectrum layouts
-bool ckpt_supported(const Geometry& g) { return !g.iso && !(rows_big_supported(g) && cols_big_supported(g)); }
+// checkpointed training re-runs blocks of the forward inside the backward (backward.cu, regen_block), on every kernel
+// route of iso = 0; the iso = 1 state (pixel-norm maps of every iteration) has no restart
+bool ckpt_supported(const Geometry& g) { return !g.iso; }
 int check_kernel_pub(int ksize, int H, int W) { return check_kernel(ksize, H, W); }
 
 }  // namespace admm
@@ -410,7 +411,7 @@ int admm_tv_forward_ex(const void* y_any, float* out, const float* kern, int ksi
     const size_t map_floats = (size_t)2 * H * W;
     const int ckpt = (saved && ext.ckpt_interval >= 2) ? ext.ckpt_interval : 0;
     if (ckpt && !ckpt_supported(g))
-        return fail(ADMM_ERR_UNSUPPORTED, "checkpointed training (admm_ext.ckpt_interval) is not available for iso = 1 or the large-frame kernels");
+        return fail(ADMM_ERR_UNSUPPORTED, "checkpointed training (admm_ext.ckpt_interval) is not available for iso = 1");
     if (saved) {
         const size_t kept = ckpt ? (size_t)(slots / ckpt) : (size_t)slots;
         const size_t need_saved = kept * 2 * g.field_bytes + (iso ? (size_t)slots * map_floats * sizeof(float) : 0);

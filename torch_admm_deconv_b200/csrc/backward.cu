@@ -401,6 +401,11 @@ int run_backward(const Geometry& g, const Workspace& ws, const BwdWorkspace& bw,
         if (is_ckpt(i)) return saved + (size_t)((i + 1) / ckpt - 1) * 2 * fe;
         return bw.ck_slots + (size_t)(i % ckpt) * 2 * fe;
     };
+    // The re-run uses the forward's kernels and layouts (abi.cu, solve_planes).  Large-frame row kernel: v is formed inside
+    // its R2C from the checkpoint (r2c_div = 2) with the march's operation order; with both large-frame kernels the
+    // spectra between them are tile-major and A is item-major (the layout COLS_INIT of cols_big.cu writes and COLS_ITER reads).
+    const bool big_rows = rows_big_supported(g);
+    const int tiled = (big_rows && cols_big_supported(g)) ? 1 : 0;
     auto regen_block = [&](int b) -> int {
         RowArgs rr; std::memset(&rr, 0, sizeof(rr));
         ColArgs cc; std::memset(&cc, 0, sizeof(cc));
@@ -412,29 +417,36 @@ int run_backward(const Geometry& g, const Workspace& ws, const BwdWorkspace& bw,
         if (b == 0 || !ck_A_valid) {                                     // A = Mul F(y)   (and x_1 for b = 0)
             rr.real_in = y; rr.spec_out = bw.ck_S1;
             if (int e = launch_rows(ROWS_R2C, g, rr, st)) return e;
-            cc.spec_in = bw.ck_S1; cc.spec_out = bw.ck_S0;
+            cc.spec_in = bw.ck_S1; cc.spec_out = bw.ck_S0; cc.in_tiled = 0; cc.out_tiled = tiled;
             if (int e = launch_cols(COLS_INIT, g, cc, st)) return e;
             ck_A_valid = true;
         }
         if (b > 0) {                                                     // x_{m0+1} from the checkpoint q_{m0}
             qprev = slot_ptr(m0 - 1);
-            {
-                ProfScope ps(PROF_OTHER, st);
-                k_bwd_recompute_v<<<ew_grid(fe), 256, 0, st>>>(qprev, qprev + fe, bw.ck_v, lmbd, rho, g.H, g.W, fe);
-                ADMM_CUDA_CHECK(cudaGetLastError());
+            if (big_rows) {
+                RowArgs rv = rr;
+                rv.r2c_div = 2; rv.qx_in = qprev; rv.qy_in = qprev + fe; rv.spec_out = bw.ck_S1; rv.tiled = tiled;
+                if (int e = launch_rows(ROWS_R2C, g, rv, st)) return e;
+            } else {
+                {
+                    ProfScope ps(PROF_OTHER, st);
+                    k_bwd_recompute_v<<<ew_grid(fe), 256, 0, st>>>(qprev, qprev + fe, bw.ck_v, lmbd, rho, g.H, g.W, fe);
+                    ADMM_CUDA_CHECK(cudaGetLastError());
+                }
+                rr.real_in = bw.ck_v; rr.spec_out = bw.ck_S1;
+                if (int e = launch_rows(ROWS_R2C, g, rr, st)) return e;
             }
-            rr.real_in = bw.ck_v; rr.spec_out = bw.ck_S1;
-            if (int e = launch_rows(ROWS_R2C, g, rr, st)) return e;
-            cc.spec_in = bw.ck_S1; cc.spec_out = bw.ck_S0;
+            cc.spec_in = bw.ck_S1; cc.spec_out = bw.ck_S0; cc.in_tiled = tiled; cc.out_tiled = tiled;
             if (int e = launch_cols(COLS_ITER, g, cc, st)) return e;
         }
+        rr.tiled = tiled;
         for (int i = m0; i < end; ++i) {
             float* qn = bw.ck_slots + (size_t)(i - m0) * 2 * fe;
             rr.spec_in = bw.ck_S0; rr.spec_out = bw.ck_S1;
             rr.qx_in = qprev; rr.qy_in = qprev ? qprev + fe : nullptr; rr.qx_out = qn; rr.qy_out = qn + fe;
             if (int e = launch_rows(ROWS_FULL, g, rr, st)) return e;
-            if (i + 1 < end) {
-                cc.spec_in = bw.ck_S1; cc.spec_out = bw.ck_S0;
+            if (i + 1 < end) {                                           // another row pass follows: tile-major output
+                cc.spec_in = bw.ck_S1; cc.spec_out = bw.ck_S0; cc.in_tiled = tiled; cc.out_tiled = tiled;
                 if (int e = launch_cols(COLS_ITER, g, cc, st)) return e;
             }
             qprev = qn;

@@ -168,7 +168,8 @@ struct RowArgsT {
     int           out_p0;                        // ROWS_C2R: index of this launch's first plane in the whole batch (plane chunks)
     const T*      cmap;                          // ROWS_R2C with r2c_div (power-of-two sizes): coefficient maps 2s-1 (2 x H x W),
                                                  // NULL = all ones
-    int           r2c_div;                       // ROWS_R2C: the input is v = D^T(cmap * q) built from qx_in / qy_in on the fly
+    int           r2c_div;                       // ROWS_R2C: the input is v = D^T(cmap * q) built from qx_in / qy_in on the fly;
+                                                 // 2 (large-frame kernel only): v = D^T(q - 2 dual(q, lmbd/rho)), the anisotropic step
     // ROWS_ADJ (backward sweep, one fused row pass): spec_in = row spectrum of vbar, qx_in/qy_in = saved q_{k+1},
     // ub*_in = ubar (NULL = zeros), ub*_out = new ubar (= qbar), spec_out = row spectrum of xbar = D^T qbar,
     // taubar accumulates d/dtau; optional second output: qv* = saved q_k -> spec_out2 = row spectrum of v_k

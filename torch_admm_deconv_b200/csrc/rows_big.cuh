@@ -315,8 +315,9 @@ k_rows_big(RowArgs a, int H, int nbands) {
 
 // ------------------------------------------------------------------------------------------ plain row passes
 // ROWS_C2R: packed spectrum -> real rows (unnormalised, + optional bias);  ROWS_R2C: real rows -> packed spectrum, the
-// input either a real field or, with r2c_div, the divergence v = D^T(cmap * q) formed while loading (iso=True forward:
-// cmap = 2s-1, deconv.py:19-24,104; NULL = unit coefficients).  Same passes and tables as the march kernel, one row
+// input either a real field or, with r2c_div = 1, the divergence v = D^T(cmap * q) formed while loading (iso=True forward:
+// cmap = 2s-1, deconv.py:19-24,104; NULL = unit coefficients), or with r2c_div = 2 the anisotropic v = D^T(q - 2 dual(q))
+// of k_rows_big's spatial step (restart of a checkpointed block, backward.cu).  Same passes and tables as the march kernel, one row
 // pair at a time per CTA, no halo.  C2R pairs rows (2k-1, 2k), R2C pairs rows (2k, 2k+1): the pairings of the two
 // tile-major spectra (common.cuh, kSpecTile), so both layouts work for either mode.
 template <int W, int MODE, bool TILED>
@@ -422,21 +423,46 @@ k_rows_big_plain(RowArgs a, int H, int nbands) {
         const int ra = 2 * k, rb = ra + 1;                                   // rows (2k, 2k+1)
         int rc = rb + 1; if (rc >= H) rc -= H;
         const size_t oa = (size_t)ra * W, ob = (size_t)rb * W, oc = (size_t)rc * W;
+        // r2c_div = 2 (checkpointed backward, restart of a block): v = Dx^T w_x + Dy^T w_y with w = q - 2 dual(q) from the
+        // saved pre-clamp state, with the expressions and the association of k_rows_big's spatial step, so the packed
+        // spectrum equals the one the march wrote in the forward bit for bit.  One uniform branch on the sign of tau.
+        auto aniso_div = [&](auto tsign, float tau) {
+            constexpr bool NEG = decltype(tsign)::neg;
+            auto wf = [](float q_, float tau_) { return fmaf(-2.0f, dual_of<NEG>(q_, tau_), q_); };
 #pragma unroll
-        for (int r = 0; r < R0; ++r) {
-            const int c = j + r * NT;
-            if (!div) {
-                v[r] = in8 ? make_float2(ld_u8_div255(in8 + oa + c), ld_u8_div255(in8 + ob + c))
-                           : make_float2(__ldg(in + oa + c), __ldg(in + ob + c));
-            } else {
-                const int cr = (c == W - 1) ? 0 : c + 1;
-                float xa = __ldg(qx + oa + c), xar = __ldg(qx + oa + cr), xb = __ldg(qx + ob + c), xbr = __ldg(qx + ob + cr);
-                float ya = __ldg(qy + oa + c), yb = __ldg(qy + ob + c), yc = __ldg(qy + oc + c);
-                if (!unit) {
-                    xa *= __ldg(kx + oa + c); xar *= __ldg(kx + oa + cr); xb *= __ldg(kx + ob + c); xbr *= __ldg(kx + ob + cr);
-                    ya *= __ldg(ky + oa + c); yb *= __ldg(ky + ob + c); yc *= __ldg(ky + oc + c);
+            for (int r = 0; r < R0; ++r) {
+                const int c = j + r * NT;
+                const float wxa = wf(__ldg(qx + oa + c), tau), wxb = wf(__ldg(qx + ob + c), tau);
+                const float wya = wf(__ldg(qy + oa + c), tau), wyb = wf(__ldg(qy + ob + c), tau), wyc = wf(__ldg(qy + oc + c), tau);
+                // w_x of column c+1 from the next lane; a warp's last lane loads it (fewer loads in flight: no spills)
+                float wxar = __shfl_down_sync(0xffffffffu, wxa, 1), wxbr = __shfl_down_sync(0xffffffffu, wxb, 1);
+                if ((j & 31) == 31) {
+                    const int cr = (c == W - 1) ? 0 : c + 1;
+                    wxar = wf(__ldg(qx + oa + cr), tau); wxbr = wf(__ldg(qx + ob + cr), tau);
                 }
-                v[r] = make_float2(xa - xar + ya - yb, xb - xbr + yb - yc);      // D^T: w_x[c] - w_x[c+1] + w_y[r] - w_y[r+1]
+                v[r] = make_float2(wxa + wya - wyb - wxar, wxb + wyb - wyc - wxbr);   // ((w_x + w_y) - w_y below) - w_x right
+            }
+        };
+        if (a.r2c_div == 2) {
+            const float tau = a.lmbd[0] / a.rho[0];                          // as in k_rows_big
+            if (tau < 0.f) aniso_div(TauNeg{}, tau); else aniso_div(TauPos{}, tau);
+        } else {
+#pragma unroll
+            for (int r = 0; r < R0; ++r) {
+                const int c = j + r * NT;
+                if (!div) {
+                    v[r] = in8 ? make_float2(ld_u8_div255(in8 + oa + c), ld_u8_div255(in8 + ob + c))
+                               : make_float2(__ldg(in + oa + c), __ldg(in + ob + c));
+                } else {
+                    const int cr = (c == W - 1) ? 0 : c + 1;
+                    float xa = __ldg(qx + oa + c), xar = __ldg(qx + oa + cr), xb = __ldg(qx + ob + c), xbr = __ldg(qx + ob + cr);
+                    float ya = __ldg(qy + oa + c), yb = __ldg(qy + ob + c), yc = __ldg(qy + oc + c);
+                    if (!unit) {
+                        xa *= __ldg(kx + oa + c); xar *= __ldg(kx + oa + cr); xb *= __ldg(kx + ob + c); xbr *= __ldg(kx + ob + cr);
+                        ya *= __ldg(ky + oa + c); yb *= __ldg(ky + ob + c); yc *= __ldg(ky + oc + c);
+                    }
+                    v[r] = make_float2(xa - xar + ya - yb, xb - xbr + yb - yc);      // D^T: w_x[c] - w_x[c+1] + w_y[r] - w_y[r+1]
+                }
             }
         }
         passes();

@@ -169,7 +169,7 @@ class _AdmmTV(torch.autograd.Function):
             if need_grad:
                 if ckpt >= 2:                          # memory-saving training: keep every ckpt-th iteration's state only
                     saved_bytes = lib.admm_query_saved_ex(B * C, H, W, ksize, int(iso), maxit, ckpt)
-                    if saved_bytes == 0:               # not available for this problem (iso=True, large-frame kernels)
+                    if saved_bytes == 0:               # not available for this problem (iso=True)
                         ckpt = 0
                 if ckpt < 2:
                     ckpt = 0
