@@ -38,7 +38,7 @@ except Exception:  # pragma: no cover
 __all__ = [
     "soft_thresh", "block_thresh", "pixelnorm", "hard_thresh", "abs2",
     "admm_tv_stencil_form", "admm_tv_spectral_form", "admm_deconv_layer",
-    "admm_tv_backward", "rel_err", "make_psf", "make_blurred",
+    "admm_tv_backward", "admm_tv_replay", "rel_err", "pair_err", "make_psf", "make_blurred",
 ]
 
 
@@ -261,6 +261,75 @@ def admm_tv_spectral_form(xin, lmbd, rho, kern, iso=False, maxit=100, workers=1,
     return x
 
 
+def _dual(q_x, q_y, iso, tau, nmap=None):
+    """u = q - prox(q) of one state, in float64.  iso: s = max(1 - tau / (n + eps), 0) with n the pixel norm of q, or
+    `nmap` = (n_x, n_y) when given, so the threshold is decided on those numbers."""
+    if iso:
+        eps = 1e-15
+        if nmap is None:
+            nmap = (np.sqrt(np.sum(q_x ** 2, (0, 1)) + eps), np.sqrt(np.sum(q_y ** 2, (0, 1)) + eps))
+        n_x, n_y = (np.asarray(n, dtype=np.float64) for n in nmap)
+        s_x = np.maximum(1 - tau / (n_x + eps), 0); s_y = np.maximum(1 - tau / (n_y + eps), 0)
+        return (1 - s_x) * q_x, (1 - s_y) * q_y
+    return q_x - soft_thresh(q_x, tau), q_y - soft_thresh(q_y, tau)
+
+
+def admm_tv_replay(xin, lmbd, rho, kern, states, iso=False, tau=None, nmaps=None, workers=1):
+    """One iteration of the reduced-state form, in float64, from each saved state of an implementation under test.
+
+    `states` is the list of pre-threshold (q_x, q_y) after iterations 1 .. N-1 of an N-iteration solve (what a training
+    forward saves).  Iteration k+1 is a deterministic function of q_k and y:
+        u = q_k - prox(q_k),  v = Dx^T(q_x - 2u_x) + Dy^T(q_y - 2u_y),  x = F^-1[A + Bm F(v)],  q_{k+1} = D x + u.
+    Replaying it from the saved q_k takes every threshold decision on the implementation's own numbers, so what remains
+    is one iteration's rounding, whatever the sign of tau or the number of iterations (a whole fp32 trajectory with
+    tau < 0 can separate from the fp64 one: u jumps by 2|tau| where q changes sign).
+
+    `tau`: the threshold the implementation used (float32(lmbd) / float32(rho) for the float32 solver); default
+    lmbd / rho.  `nmaps` (iso): the (n_x, n_y) pixel-norm maps saved with each state; when given, the block threshold
+    of state k is decided from them rather than from a recomputed norm.
+
+    Returns (preds, norms, x_out): preds[i] is the prediction of states[i] (q_1 from the zero state, q_{k+1} from
+    states[k-1]); norms[i] is the fp64 pixel-norm pair of states[i] (iso; None otherwise); x_out is the output x_N
+    predicted from the last state (from the zero state when `states` is empty, N = 1)."""
+    x = np.asarray(xin, dtype=np.float64)
+    B, C, H, W = x.shape
+    lam = float(np.asarray(lmbd).reshape(-1)[0]); rh = float(np.asarray(rho).reshape(-1)[0])
+    tau = lam / rh if tau is None else float(tau)
+    k2d = _kernel_2d(kern)
+    sigma, ph, L, den = _spectral_tables(H, W, None if k2d is None else np.asarray(k2d, dtype=np.float64), rh, np.float64)
+    A = sigma * ph * _rfft2(x, workers) / den
+    Bm = rh / den
+    states = [tuple(np.asarray(t, dtype=np.float64) for t in s) for s in states]
+
+    def step(k):       # x and q after the iteration that consumes states[k - 1] (k = 0: the zero state)
+        if k == 0:
+            xn = _irfft2(A, (H, W), workers)
+            return xn, (_dx(xn), _dy(xn))
+        q_x, q_y = states[k - 1]
+        u_x, u_y = _dual(q_x, q_y, iso, tau, None if nmaps is None else nmaps[k - 1])
+        v = _dxt(q_x - 2 * u_x) + _dyt(q_y - 2 * u_y)
+        xn = _irfft2(A + Bm * _rfft2(v, workers), (H, W), workers)
+        return xn, (_dx(xn) + u_x, _dy(xn) + u_y)
+
+    preds = [step(k)[1] for k in range(len(states))]
+    norms = None
+    if iso:
+        norms = [(pixelnorm(q_x), pixelnorm(q_y)) for q_x, q_y in states]
+    return preds, norms, step(len(states))[0]
+
+
+def pair_err(got, want, floor=0.0):
+    """`rel_err` over a list of field pairs (states or norm maps): max|a-b| over every field / max|b| over every field;
+    0 for empty lists.  `floor`: a lower bound of the denominator.  The replay gate passes max|x_N|: q = D x + u is
+    formed from x, so its rounding scales with |x|, and a solve that saved only q_1 = D x_1 (max|q_1| ~ 0.4 max|x_1| on
+    the test images) would otherwise grade the rounding of x against a smaller scale."""
+    if not want:
+        return 0.0
+    num = max(float(np.max(np.abs(np.asarray(a, np.float64) - b))) for ga, wa in zip(got, want) for a, b in zip(ga, wa))
+    den = max([float(floor)] + [float(np.max(np.abs(b))) for wa in want for b in wa])
+    return num / (den if den > 0 else 1.0)
+
+
 def admm_deconv_layer(x, w, lmbda, rho, b, iso=True, max_iters=100, activation=None,
                       form="spectral"):
     """`ADMMDeconv.forward`: activation(fft_admm_tv(x, lmbda, rho, w, iso, max_iters) + b)
@@ -273,7 +342,8 @@ def admm_deconv_layer(x, w, lmbda, rho, b, iso=True, max_iters=100, activation=N
 # ----------------------------------------------------------------------------------------
 # hand-derived adjoint  (SURVEY.md appendix B; replaces stock autograd over deconv.py:103-115)
 # ----------------------------------------------------------------------------------------
-def admm_tv_backward(xin, lmbd, rho, kern, grad_out, iso=False, maxit=100, qs_override=None, tau_override=None):
+def admm_tv_backward(xin, lmbd, rho, kern, grad_out, iso=False, maxit=100, qs_override=None, tau_override=None,
+                     nmaps_override=None, workers=1):
     """Returns (grad_xin, grad_lmbd, grad_rho, grad_kern) in float64.
 
     Reverse sweep over the reduced-state iteration of `admm_tv_spectral_form`.  The forward
@@ -285,7 +355,11 @@ def admm_tv_backward(xin, lmbd, rho, kern, grad_out, iso=False, maxit=100, qs_ov
     forward decides a handful of borderline masks differently from an fp64 one and each such element changes the
     gradient by O(1) locally -- for ANY fp32 implementation, the reference's included.  With the state given, the
     masks (and the recomputed v_k) are taken from it, which makes the comparison of the adjoint itself sharp;
-    `tau_override` is the threshold those masks were decided with (float32(lmbd) / float32(rho))."""
+    `tau_override` is the threshold those masks were decided with (float32(lmbd) / float32(rho)).
+
+    `nmaps_override` (iso): optional list of the (n_x, n_y) pixel-norm maps saved with each state of `qs_override`.
+    The block threshold s = max(1 - tau / (n + eps), 0) and its active set s > 0 are then decided from those maps, as
+    the aniso masks are decided from the given q.  `workers`: scipy FFT threads, for large frames."""
     xin = np.asarray(xin, dtype=np.float64)
     g = np.asarray(grad_out, dtype=np.float64)
     B, C, H, W = xin.shape
@@ -295,20 +369,21 @@ def admm_tv_backward(xin, lmbd, rho, kern, grad_out, iso=False, maxit=100, qs_ov
     k2d64 = None if k2d is None else np.asarray(k2d, dtype=np.float64)
     sigma, ph, L, den = _spectral_tables(H, W, k2d64, rh, np.float64)
     Bm = rh / den
-    Fy = np.fft.rfft2(xin)
+    Fy = _rfft2(xin, workers)
     A = sigma * ph * Fy / den
     N = int(maxit)
     if N == 0:
         gk = None if k2d is None else np.zeros((1, 1) + k2d.shape)
         return np.zeros_like(xin), 0.0, 0.0, gk
-    # forward, keeping q_k and v_k
+    # forward, keeping q_k and v_k (all but v_0 = 0 are replaced below when the whole state is given)
     w_x = np.zeros_like(xin); w_y = np.zeros_like(xin)
     u_x = np.zeros_like(xin); u_y = np.zeros_like(xin)
     qs = []; vs = []
     eps = 1e-15
-    for _ in range(N):
+    full_override = qs_override is not None and len(qs_override) >= N - 1
+    for _ in range(1 if full_override else N):
         v = _dxt(w_x) + _dyt(w_y)
-        x = np.fft.irfft2(A + Bm * np.fft.rfft2(v), s=(H, W))
+        x = _irfft2(A + Bm * _rfft2(v, workers), (H, W), workers)
         q_x = _dx(x) + u_x; q_y = _dy(x) + u_y
         if iso:
             n_x = np.sqrt(np.sum(q_x ** 2, (0, 1)) + eps); n_y = np.sqrt(np.sum(q_y ** 2, (0, 1)) + eps)
@@ -320,13 +395,19 @@ def admm_tv_backward(xin, lmbd, rho, kern, grad_out, iso=False, maxit=100, qs_ov
         qs.append((q_x, q_y)); vs.append(v)
     if tau_override is not None:
         tau = float(tau_override)
+    nm = [None] * N                                             # per state: (n_x, n_y) to decide the block threshold with
     if qs_override is not None:
+        if full_override:
+            qs = qs[:1] + [None] * (N - 1); vs = vs[:1] + [None] * (N - 1)
         for k, (oq_x, oq_y) in enumerate(qs_override):
             qs[k] = (np.asarray(oq_x, dtype=np.float64), np.asarray(oq_y, dtype=np.float64))
+        if iso and nmaps_override is not None:
+            for k, (n_x, n_y) in enumerate(nmaps_override):
+                nm[k] = (np.asarray(n_x, dtype=np.float64), np.asarray(n_y, dtype=np.float64))
         for k in range(1, N):                                   # v_k = D^T w(q_k) from the given state
             q_x, q_y = qs[k - 1]
             if iso:
-                n_x = np.sqrt(np.sum(q_x ** 2, (0, 1)) + eps); n_y = np.sqrt(np.sum(q_y ** 2, (0, 1)) + eps)
+                n_x, n_y = nm[k - 1] or (np.sqrt(np.sum(q_x ** 2, (0, 1)) + eps), np.sqrt(np.sum(q_y ** 2, (0, 1)) + eps))
                 s_x = np.maximum(1 - tau / (n_x + eps), 0); s_y = np.maximum(1 - tau / (n_y + eps), 0)
                 w_x = (2 * s_x - 1) * q_x; w_y = (2 * s_y - 1) * q_y
             else:
@@ -351,7 +432,7 @@ def admm_tv_backward(xin, lmbd, rho, kern, grad_out, iso=False, maxit=100, qs_ov
                 q = qs[k][f]
                 ut = ub[f] - 2 * wb[f]
                 if iso:
-                    n = np.sqrt(np.sum(q ** 2, (0, 1)) + eps)
+                    n = nm[k][f] if nm[k] is not None else np.sqrt(np.sum(q ** 2, (0, 1)) + eps)
                     s = np.maximum(1 - tau / (n + eps), 0)
                     act = (s > 0).astype(np.float64)
                     sb = np.sum((2 * wb[f] - ub[f]) * q, (0, 1))
@@ -364,15 +445,17 @@ def admm_tv_backward(xin, lmbd, rho, kern, grad_out, iso=False, maxit=100, qs_ov
                 qb.append(qb_f)
             xb = xb + _dxt(qb[0]) + _dyt(qb[1])
             ub = qb
-        G = np.fft.rfft2(xb) / (H * W)          # adjoint of irfft2 w.r.t. its half-spectrum input (weights cw applied below)
+        Fxb = _rfft2(xb, workers)
+        G = Fxb / (H * W)                        # adjoint of irfft2 w.r.t. its half-spectrum input (weights cw applied below)
         Gsum += G
-        GVsum += np.conj(G) * np.fft.rfft2(vs[k])
-        vb = np.fft.irfft2(Bm * np.fft.rfft2(xb), s=(H, W))
+        if k > 0:                                # v_0 = 0
+            GVsum += np.conj(G) * _rfft2(vs[k], workers)
+        vb = _irfft2(Bm * Fxb, (H, W), workers)
         wb = [_dx(vb), _dy(vb)]
         xb = np.zeros_like(xin)
     # G above is F(xbar)/(HW); with Parseval weights cw the pairing <X, G> = sum cw Re(conj(G) X)
     wgt = cw[None, None, None, :]
-    gy = np.fft.irfft2(np.conj(sigma * ph / den) * Gsum * (H * W), s=(H, W))
+    gy = _irfft2(np.conj(sigma * ph / den) * Gsum * (H * W), (H, W), workers)
     dA_drho = -A * L / den
     dBm_drho = np.abs(sigma) ** 2 / den ** 2
     rho_bar = float(np.sum(wgt * np.real(np.conj(Gsum) * dA_drho + GVsum * dBm_drho))) - tau_bar * lam / rh ** 2
