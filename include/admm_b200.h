@@ -58,7 +58,10 @@ size_t admm_query_saved(int planes, int H, int W, int ksize, int iso, int maxit)
 /* Replaces fft_admm_tv (deconv.py:35-117): out = last x iterate, zeros when maxit == 0 (deconv.py:61,117).
  *   y, out : (B, C, H, W) fp32     bias: optional device pointer to one float added to out
  *                                  (ADMMDeconv.forward's `+ self.b`, admmdeconv.py:64), or NULL
- *   saved  : NULL for inference; otherwise receives the per-iteration state the backward needs. */
+ *   saved  : NULL for inference; otherwise receives the per-iteration state the backward needs.
+ * Sizes without a specialised kernel run on the generic kernels, which hold a row or column in shared memory: the column
+ * pass needs H <= 9685, the row pass W <= 5811 for iso = 0 with maxit >= 2 (two halo rows) and W <= 9685 otherwise.  A
+ * larger frame returns ADMM_ERR_UNSUPPORTED before anything is launched (the backward checks the same limits). */
 int admm_tv_forward(const float* y, float* out,
                     const float* kern, int ksize,
                     const float* lmbd, const float* rho, const float* bias,

@@ -403,6 +403,7 @@ int admm_tv_forward_ex(const void* y_any, float* out, const float* kern, int ksi
         }
         return 0;
     }
+    if (int e = check_generic_f32(g, !iso && maxit > 1)) return e;
     if (!workspace || ((uintptr_t)workspace & 255)) return fail(ADMM_ERR_WORKSPACE, "workspace is NULL or not 256-byte aligned");
     Workspace ws;
     const size_t need = carve_workspace(g, ksize, maxit, (char*)workspace, &ws);

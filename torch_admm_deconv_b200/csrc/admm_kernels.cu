@@ -506,24 +506,40 @@ int launch_cols(ColMode mode, const Geometry& g, const ColArgsT<double>& a, cuda
     return launch_cols_generic(mode, g, a, st);
 }
 
-// float64: whether the generic passes of a solve fit in shared memory (the smallest band / tile the launchers above would
-// pick), so that an unsupported size fails before anything is launched
-int check_generic_f64(const Geometry& g, bool full_rows) {
+// Whether the generic passes of a solve fit in shared memory (the smallest band / tile the launchers above would pick), so
+// that an unsupported size fails before anything is launched.  `rows`: the solve runs the generic row kernel; full_rows:
+// that includes ROWS_FULL, whose band keeps two halo rows.  Limits (227 KB): float W <= 5811 with the halo, W <= 9685
+// without, H <= 9685; double W <= 2905, W <= 4842, H <= 4842.
+template <typename T>
+static int check_generic(const Geometry& g, bool rows, bool full_rows) {
+    const std::string prec = sizeof(T) == 4 ? "float32" : "float64";
     const size_t kMax = 227 * 1024;
     FftPlan plan;
-    if (!make_plan(g.W, plan)) return fail(4, "cannot plan row FFT length");
+    if (rows) {
+        if (!make_plan(g.W, plan)) return fail(4, "cannot plan row FFT length");
+        const int np = full_rows ? 2 : 1;                        // row pairs of a two-row band, halo included
+        const size_t need = rows_smem<T>(g.W, np);
+        if (need > kMax)
+            return fail(4, prec + " row FFT does not fit in shared memory: W = " + std::to_string(g.W) + " needs " +
+                           std::to_string(need) + " bytes, the limit is " + std::to_string(kMax) +
+                           (full_rows ? " (iso = 0 keeps two halo rows: W <= " : " (W <= ") +
+                           std::to_string(kMax / rows_smem<T>(1, np)) + ")");
+    }
     if (!make_plan(g.H, plan)) return fail(4, "cannot plan column FFT length");
-    const int halo = full_rows ? 2 : 0;
-    const size_t rows = rows_smem<double>(g.W, (2 + halo + 1) / 2);
-    if (rows > kMax)
-        return fail(4, "float64 row FFT does not fit in shared memory: W = " + std::to_string(g.W) + " needs " +
-                       std::to_string(rows) + " bytes, the limit is " + std::to_string(kMax) +
-                       (full_rows ? " (iso = 0 keeps two halo rows: W <= 2905)" : " (W <= 4842)"));
-    const size_t cols = cols_smem<double>(g.H, 1);
-    if (cols > kMax)
-        return fail(4, "float64 column FFT does not fit in shared memory: H = " + std::to_string(g.H) + " needs " +
-                       std::to_string(cols) + " bytes, the limit is " + std::to_string(kMax) + " (H <= 4842)");
+    const size_t need = cols_smem<T>(g.H, 1);
+    if (need > kMax)
+        return fail(4, prec + " column FFT does not fit in shared memory: H = " + std::to_string(g.H) + " needs " +
+                       std::to_string(need) + " bytes, the limit is " + std::to_string(kMax) + " (H <= " +
+                       std::to_string(kMax / cols_smem<T>(1, 1)) + ")");
     return 0;
+}
+
+int check_generic_f64(const Geometry& g, bool full_rows) { return check_generic<double>(g, true, full_rows); }
+
+// float32: the row check mirrors launch_rows (the specialised kernels take their widths in every mode); the columns are
+// always checked, since every height runs some generic column mode (the plain FFT passes of the backward)
+int check_generic_f32(const Geometry& g, bool full_rows) {
+    return check_generic<float>(g, !rows_pow2_supported(g) && !rows_big_supported(g), full_rows);
 }
 
 }  // namespace admm

@@ -682,6 +682,7 @@ int admm_tv_backward_ex(const float* y, const float* grad_out, const float* kern
         if (grad_rho) ADMM_CUDA_CHECK(cudaMemsetAsync(grad_rho, 0, sizeof(float), st));
         return 0;
     }
+    if (int e = check_generic_f32(g, ckpt != 0)) return e;   // the halo row pass runs only to re-run checkpointed blocks
     if (!workspace || ((uintptr_t)workspace & 255)) return fail(ADMM_ERR_WORKSPACE, "workspace is NULL or not 256-byte aligned");
     Workspace ws; BwdWorkspace bw;
     if (ckpt && !ckpt_supported(g)) return fail(ADMM_ERR_UNSUPPORTED, "checkpointed training is not available for this problem");

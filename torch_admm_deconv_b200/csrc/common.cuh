@@ -234,6 +234,7 @@ int launch_tables_f64(const Geometry& g, const double2* twWd, const double2* twH
 int launch_rows(RowMode mode, const Geometry& g, const RowArgsT<double>& a, cudaStream_t st);   // R2C, C2R, FULL
 int launch_cols(ColMode mode, const Geometry& g, const ColArgsT<double>& a, cudaStream_t st);
 int check_generic_f64(const Geometry& g, bool full_rows);       // 0, or ADMM_ERR_UNSUPPORTED with a message
+int check_generic_f32(const Geometry& g, bool full_rows);       // the same for the float32 solver's generic passes
 int launch_iso_prox(const Geometry& g, const double* x, const double* qx_prev, const double* qy_prev, const double* n_prev,
                     double* qx_new, double* qy_new, double* n_new, double* c_new, const double* lmbd, const double* rho,
                     cudaStream_t st);
