@@ -16,7 +16,8 @@
  *   - lmbd / rho are device pointers to ONE float each (learnable parameters: never read on host);
  *   - kern is (ksize x ksize) fp32 row-major, or NULL with ksize == 0 for the TV-denoise branch
  *     (deconv.py:46-47, 86-87);
- *   - all work is enqueued on `stream` (a cudaStream_t passed as void*); nothing synchronises;
+ *   - all work is enqueued on `stream` (a cudaStream_t passed as void*); nothing synchronises, with one exception: a
+ *     solve with a tolerance (admm_ext.rtol / atol) waits on its own event at each residual check;
  *   - the library allocates nothing: the caller owns `workspace` (size from admm_query_workspace)
  *     and the optional `saved` state; both must be 256-byte aligned;
  *   - return value 0 = ok; non-zero = error, text available from admm_last_error() (thread-local).
@@ -94,7 +95,25 @@ typedef struct admm_ext {
     const float* yhat_in;        /* optional: column-transformed packed spectrum of y, as written through yhat_out by an
                                     earlier call on the same y (solvers that share the input skip their R2C + column FFT) */
     float*    yhat_out;          /* optional: receives that spectrum (admm_query_yhat bytes) */
+    /* Convergence residuals of the splitting Dx - z = 0 (Boyd et al. 2011, 3.3), per plane (DESIGN section 10).  With
+     * resid_every = M >= 1 the solve writes, after iterations k = M, 2M, ... <= maxit - 1, the primal residual
+     * r = ||u_k - u_{k-1}||, the dual residual s = rho ||D^T(z_k - z_{k-1})|| and the tolerances
+     * eps_pri = sqrt(2HW) atol + rtol max(||Dx_k||, ||z_k||), eps_dual = sqrt(HW) atol + rtol rho ||D^T u_k||.  The cluster
+     * solver, the cooperative kernel and plane chunks (which run iterations out of the host's sight) are not used then.
+     * With rtol > 0 or atol > 0 (inference only: saved == NULL) the solve stops at the first check k at which every
+     * plane has r <= eps_pri and s <= eps_dual, and returns x_k: exactly what maxit = k returns.  It then waits for each
+     * check's result on the host (not capturable in a CUDA graph). */
+    float*    resid;             /* device, admm_query_resid bytes, 256-byte aligned: [check][plane][4] =
+                                    (r, s, eps_pri, eps_dual) fp32, then scratch */
+    int       resid_every;       /* M >= 1: residuals after iterations M, 2M, ... (0 = off) */
+    float     rtol, atol;        /* either > 0: stop at the first check where every plane has converged (saved == NULL only) */
+    int*      host_flag;         /* pinned host int the check copies into; required when stopping early */
+    int*      iters_out;         /* optional host int: x-updates performed (maxit unless stopped early) */
 } admm_ext;
+
+/* Bytes of admm_ext.resid for this problem: the history of (maxit - 1) / resid_every checks (none for maxit <= 1), scratch,
+ * and with early_stop != 0 a spare spectrum.  0 when resid_every <= 0 or the shape is invalid. */
+size_t admm_query_resid(int planes, int H, int W, int maxit, int resid_every, int early_stop);
 
 size_t admm_query_yhat(int planes, int H, int W);      /* bytes of the shared spectrum buffer (0 on error) */
 

@@ -37,13 +37,16 @@ SIGNATURES = {
 class AdmmExt(ctypes.Structure):
     """`admm_ext` of include/admm_b200.h (fused layer prologue / epilogue, output placement, shared spectrum)."""
     _fields_ = [("struct_size", _i), ("in_dtype", _i), ("activation", _i), ("ckpt_interval", _i),
-                ("out_batch_stride", ctypes.c_longlong), ("yhat_in", _vp), ("yhat_out", _vp)]
+                ("out_batch_stride", ctypes.c_longlong), ("yhat_in", _vp), ("yhat_out", _vp),
+                ("resid", _vp), ("resid_every", _i), ("rtol", ctypes.c_float), ("atol", ctypes.c_float),
+                ("host_flag", _vp), ("iters_out", _vp)]
 
 
 IN_F32, IN_U8_DIV255 = 0, 1
 ACT_NONE, ACT_RELU, ACT_SIGMOID, ACT_TANH = 0, 1, 2, 3
 
 SIGNATURES["admm_query_yhat"] = (_sz, [_i] * 3)
+SIGNATURES["admm_query_resid"] = (_sz, [_i] * 6)
 SIGNATURES["admm_query_saved_ex"] = (_sz, [_i] * 7)
 SIGNATURES["admm_query_workspace_backward_ex"] = (_sz, [_i] * 7)
 SIGNATURES["admm_tv_backward_ex"] = (_i, SIGNATURES["admm_tv_backward"][1] + [_i])

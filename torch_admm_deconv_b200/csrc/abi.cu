@@ -139,11 +139,34 @@ using namespace admm;
 // Default L2 working-set budget of a plane chunk (MB); see admm_tv_forward_ex.  B200: 126 MB L2.
 static constexpr int kDefaultChunkMB = 0;
 
+// Residual checks of one solve (admm_ext.resid_every > 0; resid.cu).  With `stop` the loop waits on `ev` after each check
+// and ends when the device flag, copied to *host_flag, reports every plane converged.
+struct ResidRun {
+    ResidBufs b;
+    int every;
+    bool stop;
+    float rtol, atol;
+    int* host_flag;
+    cudaEvent_t ev;
+    int iters;                 // out: x-updates performed
+};
+
+// one event per (host thread, device): the wait of a check must not see another thread's record
+static int resid_event(cudaEvent_t* ev) {
+    static thread_local cudaEvent_t evs[kMaxProfDevices] = {};
+    int dev = 0;
+    ADMM_CUDA_CHECK(cudaGetDevice(&dev));
+    if (dev < 0 || dev >= kMaxProfDevices) return fail(ADMM_ERR_INVALID, "residuals: device index out of range");
+    if (!evs[dev]) ADMM_CUDA_CHECK(cudaEventCreateWithFlags(&evs[dev], cudaEventDisableTiming));
+    *ev = evs[dev];
+    return 0;
+}
+
 // All iterations for the planes of one chunk (gc.P planes starting at plane p0 of the batch described by gall).
 static int solve_planes(const Geometry& g, const Geometry& gall, const Workspace& ws, const float* y, const unsigned char* y8,
                         float* out, int p0, int C, const float* kern, int ksize, const float* lmbd, const float* rho,
                         const float* bias, int maxit, float* saved, size_t fe_all, int slots, size_t map_floats,
-                        const admm_ext& ext, size_t off_spec, cudaStream_t st) {
+                        const admm_ext& ext, size_t off_spec, ResidRun* rr, cudaStream_t st) {
     const int H = g.H, W = g.W;
     const bool iso = g.iso != 0;
     (void)kern; (void)ksize; (void)gall;
@@ -179,12 +202,18 @@ static int solve_planes(const Geometry& g, const Geometry& gall, const Workspace
 
     const float* qx_prev = nullptr; const float* qy_prev = nullptr;
     // small, latency-bound batches (inference): iterations 1 .. maxit-1 in ONE cooperative launch (coop_small.cu)
-    const bool coop = !saved && maxit > 1 && !tiled && coop_solver_supported(g) && coop_solver_preferred(g);
+    const bool coop = !saved && !rr && maxit > 1 && !tiled && coop_solver_supported(g) && coop_solver_preferred(g);
     if (coop) {
         if (int e = launch_coop_iterations(g, ws, lmbd, rho, maxit, st)) return e;
     }
+    // S0 holds the spectrum of the current x.  Early stop: column pass k writes the spare buffer, so after the check at k
+    // S0 still holds X_k (tile-major on the large-frame route) and the buffers swap when the solve goes on
+    float2* S0 = ws.S0;
+    float2* spare = rr ? rr->b.spare : nullptr;
+    bool stopped = false;
     for (int it = 1; it < maxit && !coop; ++it) {
         float* qx_new; float* qy_new;
+        const float* n_prev = nullptr; const float* n_new = nullptr;
         const int K = ext.ckpt_interval;
         if (saved && K >= 2 && (it % K) != 0) {        // checkpointed training: this iteration's state is not kept
             qx_new = ws.q[it & 1][0]; qy_new = ws.q[it & 1][1];
@@ -198,35 +227,59 @@ static int solve_planes(const Geometry& g, const Geometry& gall, const Workspace
         if (iso) {
             // block threshold couples all planes of a pixel (pixelnorm over dims (0,1), deconv.py:19-24): the row
             // pass is split into C2R, a per-pixel prox over the planes, the divergence, and R2C   (never chunked)
-            const float* n_prev = (it == 1) ? nullptr
-                                : (saved ? saved + (size_t)slots * 2 * fe_all + (size_t)(it - 2) * map_floats : ws.nmap[(it - 1) & 1]);
-            float* n_new = saved ? saved + (size_t)slots * 2 * fe_all + (size_t)(it - 1) * map_floats : ws.nmap[it & 1];
-            ra.spec_in = ws.S0; ra.real_out = ws.xreal; ra.bias = nullptr; ra.tiled = tiled ? 1 : 0;
+            n_prev = (it == 1) ? nullptr
+                   : (saved ? saved + (size_t)slots * 2 * fe_all + (size_t)(it - 2) * map_floats : ws.nmap[(it - 1) & 1]);
+            float* nm = saved ? saved + (size_t)slots * 2 * fe_all + (size_t)(it - 1) * map_floats : ws.nmap[it & 1];
+            n_new = nm;
+            ra.spec_in = S0; ra.real_out = ws.xreal; ra.bias = nullptr; ra.tiled = tiled ? 1 : 0;
             if (int e = launch_rows(ROWS_C2R, g, ra, st)) return e;
-            if (int e = launch_iso_prox(g, ws.xreal, qx_prev, qy_prev, n_prev, qx_new, qy_new, n_new, ws.sbmap, lmbd, rho, st)) return e;
+            if (int e = launch_iso_prox(g, ws.xreal, qx_prev, qy_prev, n_prev, qx_new, qy_new, nm, ws.sbmap, lmbd, rho, st)) return e;
             if (rows_pow2_supported(g) || rows_big_supported(g)) {   // divergence fused into the R2C row pass
                 RowArgs rb = ra;
                 rb.r2c_div = 1; rb.cmap = ws.sbmap; rb.qx_in = qx_new; rb.qy_in = qy_new; rb.spec_out = ws.S1;
                 if (int e = launch_rows(ROWS_R2C, g, rb, st)) return e;
             } else {
-                if (int e = launch_iso_div(g, qx_new, qy_new, n_new, ws.sbmap, ws.vreal, lmbd, rho, st)) return e;
+                if (int e = launch_iso_div(g, qx_new, qy_new, nm, ws.sbmap, ws.vreal, lmbd, rho, st)) return e;
                 ra.real_in = ws.vreal; ra.spec_out = ws.S1;
                 if (int e = launch_rows(ROWS_R2C, g, ra, st)) return e;
             }
         } else {
-            ra.spec_in = ws.S0; ra.spec_out = ws.S1;
+            ra.spec_in = S0; ra.spec_out = ws.S1;
             ra.qx_in = qx_prev; ra.qy_in = qy_prev; ra.qx_out = qx_new; ra.qy_out = qy_new;
             ra.tiled = tiled ? 1 : 0;
-            // inference on the specialised kernels keeps the clamped dual as state (no clamp on reload)
-            const RowMode fm = (!saved && (rows_pow2_supported(g) || rows_big_supported(g))) ? ROWS_FULL_U : ROWS_FULL;
+            // inference on the specialised kernels keeps the clamped dual as state (no clamp on reload); the residuals
+            // need q itself (same results: DESIGN section 5)
+            const RowMode fm = (!saved && !rr && (rows_pow2_supported(g) || rows_big_supported(g))) ? ROWS_FULL_U : ROWS_FULL;
             if (int e = launch_rows(fm, g, ra, st)) return e;
         }
-        ca.spec_in = ws.S1; ca.spec_out = ws.S0;
+        const bool check = rr && it % rr->every == 0;
+        if (check) {
+            float* hist = rr->b.hist + (size_t)(it / rr->every - 1) * g.P * 4;
+            if (int e = launch_resid(g, qx_prev, qy_prev, qx_new, qy_new, n_prev, n_new, lmbd, rho, rr->b, hist, rr->rtol,
+                                     rr->atol, st)) return e;
+            if (rr->stop) {
+                ADMM_CUDA_CHECK(cudaMemcpyAsync(rr->host_flag, rr->b.dflag, sizeof(int), cudaMemcpyDeviceToHost, st));
+                ADMM_CUDA_CHECK(cudaEventRecord(rr->ev, st));
+            }
+        }
+        const bool wait = check && rr->stop;
+        ca.spec_in = ws.S1; ca.spec_out = wait ? spare : S0;
         ca.in_tiled = tiled ? 1 : 0; ca.out_tiled = (tiled && it + 1 < maxit) ? 1 : 0;
         if (int e = launch_cols(COLS_ITER, g, ca, st)) return e;
         qx_prev = qx_new; qy_prev = qy_new;
+        if (wait) {                                    // the column pass runs while the host waits for the check
+            ADMM_CUDA_CHECK(cudaEventSynchronize(rr->ev));
+            if (*rr->host_flag) {
+                rr->iters = it;
+                stopped = true;
+                break;
+            }
+            std::swap(S0, spare);
+        }
     }
-    ra.spec_in = ws.S0; ra.real_out = out; ra.bias = bias; ra.tiled = 0;
+    // S0 was written by column pass `iters` - 1 (or the init pass): row-major after the last iteration, tile-major when the
+    // solve stopped early on the large-frame route
+    ra.spec_in = S0; ra.real_out = out; ra.bias = bias; ra.tiled = (stopped && tiled) ? 1 : 0;
     ra.act = ext.activation; ra.out_C = C; ra.out_p0 = p0;
     ra.out_bstride = (ext.out_batch_stride == (long long)C * H * W) ? 0 : ext.out_batch_stride;
     if (int e = launch_rows(ROWS_C2R, g, ra, st)) return e;
@@ -322,6 +375,12 @@ size_t admm_query_workspace(int planes, int H, int W, int ksize, int iso, int ma
     return carve_workspace(g, ksize, maxit, nullptr, nullptr);
 }
 
+size_t admm_query_resid(int planes, int H, int W, int maxit, int resid_every, int early_stop) {
+    Geometry g;
+    if (resid_every <= 0 || maxit < 0 || make_geometry(planes, H, W, &g)) return 0;
+    return carve_resid(g, maxit, resid_every, early_stop ? 1 : 0, nullptr, nullptr);
+}
+
 size_t admm_query_saved(int planes, int H, int W, int ksize, int iso, int maxit) {
     return admm_query_saved_ex(planes, H, W, ksize, iso, maxit, 0);
 }
@@ -378,6 +437,21 @@ int admm_tv_forward_ex(const void* y_any, float* out, const float* kern, int ksi
     if (ext.activation < ADMM_ACT_NONE || ext.activation > ADMM_ACT_TANH) return fail(ADMM_ERR_INVALID, "unknown admm_ext.activation");
     if (ext.out_batch_stride != 0 && ext.out_batch_stride < (long long)C * H * W)
         return fail(ADMM_ERR_INVALID, "admm_ext.out_batch_stride is smaller than one image (C*H*W floats)");
+    const bool tol = ext.rtol > 0.f || ext.atol > 0.f;
+    if (ext.resid_every < 0) return fail(ADMM_ERR_INVALID, "admm_ext.resid_every must be >= 0");
+    if (!(ext.rtol >= 0.f) || !(ext.atol >= 0.f)) return fail(ADMM_ERR_INVALID, "admm_ext.rtol and atol must be >= 0");
+    if (tol && saved) return fail(ADMM_ERR_INVALID, "a tolerance (admm_ext.rtol / atol) stops inference only: saved must be NULL");
+    if (tol && !ext.host_flag) return fail(ADMM_ERR_INVALID, "a tolerance (admm_ext.rtol / atol) needs admm_ext.host_flag");
+    if (tol && ext.resid_every == 0) return fail(ADMM_ERR_INVALID, "a tolerance (admm_ext.rtol / atol) needs admm_ext.resid_every >= 1");
+    if (ext.resid_every > 0 && (!ext.resid || ((uintptr_t)ext.resid & 255)))
+        return fail(ADMM_ERR_INVALID, "admm_ext.resid is NULL or not 256-byte aligned");
+    if (tol) {
+        cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+        ADMM_CUDA_CHECK(cudaStreamIsCapturing(st, &cap));
+        if (cap != cudaStreamCaptureStatusNone)
+            return fail(ADMM_ERR_INVALID, "a tolerance (admm_ext.rtol / atol) waits on the host: not available in CUDA-graph capture");
+    }
+    if (ext.iters_out) *ext.iters_out = maxit;
     const float* y = (ext.in_dtype == ADMM_IN_F32) ? (const float*)y_any : nullptr;
     const unsigned char* y8 = (ext.in_dtype == ADMM_IN_U8_DIV255) ? (const unsigned char*)y_any : nullptr;
     if (!y_any || !out || !lmbd || !rho) return fail(ADMM_ERR_INVALID, "NULL tensor pointer");
@@ -428,8 +502,19 @@ int admm_tv_forward_ex(const void* y_any, float* out, const float* kern, int ksi
     if ((ext.yhat_in || ext.yhat_out) && cols_big_supported(g))
         return fail(ADMM_ERR_UNSUPPORTED, "shared spectrum (admm_ext.yhat_*) is not available for this frame size (admm_query_yhat returns 0)");
 
+    ResidRun run;
+    ResidRun* rr = nullptr;
+    if (ext.resid_every > 0) {
+        carve_resid(g, maxit, ext.resid_every, tol ? 1 : 0, (char*)ext.resid, &run.b);
+        run.every = ext.resid_every; run.stop = tol; run.rtol = ext.rtol; run.atol = ext.atol;
+        run.host_flag = ext.host_flag; run.ev = nullptr; run.iters = maxit;
+        if (tol)
+            if (int e = resid_event(&run.ev)) return e;
+        rr = &run;
+    }
+
     // ---- one or a few small planes: the cluster-resident solver runs the whole solve in one launch (cluster_pow2.cu)
-    if (!saved && !ext.yhat_in && !ext.yhat_out && cluster_solver_supported(g, iso, false) && cluster_solver_preferred(g)) {
+    if (!saved && !rr && !ext.yhat_in && !ext.yhat_out && cluster_solver_supported(g, iso, false) && cluster_solver_preferred(g)) {
         ClusterArgs ka; std::memset(&ka, 0, sizeof(ka));
         ka.y = y; ka.y8 = y8; ka.out = out; ka.twW = ws.twW; ka.twH = ws.twH; ka.Bm = ws.Bm; ka.Bq = ws.Bq; ka.Mul = ws.Mul; ka.Mq = ws.Mq;
         ka.lmbd = lmbd; ka.rho = rho; ka.bias = bias; ka.act = ext.activation; ka.out_C = C; ka.out_p0 = 0;
@@ -449,7 +534,7 @@ int admm_tv_forward_ex(const void* y_any, float* out, const float* kern, int ksi
         int mb = options().chunk_mb;
         if (mb < 0) mb = kDefaultChunkMB;
         const size_t per_plane = (size_t)H * W * sizeof(float) * 7;
-        if (mb > 0 && !iso && maxit > 2) {
+        if (mb > 0 && !iso && !rr && maxit > 2) {
             const size_t fit = ((size_t)mb << 20) / per_plane;
             if (fit >= 1 && (int)fit < g.P) {
                 // balanced chunks, each at least a wave's worth of work when possible
@@ -466,8 +551,9 @@ int admm_tv_forward_ex(const void* y_any, float* out, const float* kern, int ksi
         const size_t off_real = (size_t)p0 * H * W, off_spec = (size_t)p0 * H * g.Wc;
         if (int e = solve_planes(gc, g, ws, y ? y + off_real : nullptr, y8 ? y8 + off_real : nullptr, out, p0, C, kern, ksize,
                                  lmbd, rho, bias, maxit, saved ? (float*)saved + off_real : nullptr, fe_all, slots, map_floats,
-                                 ext, off_spec, st)) return e;
+                                 ext, off_spec, rr, st)) return e;
     }
+    if (rr && ext.iters_out) *ext.iters_out = rr->iters;
     return 0;
 }
 

@@ -108,6 +108,10 @@ __device__ __forceinline__ double dual_of(double q, double tau) {
     return fmin(fmax(q, -tau), tau);
 }
 __device__ __forceinline__ double dual_any(double q, double tau) { return tau < 0.0 ? dual_of<true>(q, tau) : dual_of<false>(q, tau); }
+// ---- block threshold scale s = max(1 - tau / (n + 1e-15), 0) of a pixel norm n (deconv.py:19-20; iso.cu, resid.cu), float
+// and double (the float64 solve, f64.cu); the epsilon is a constant of the element type
+template <typename T> __device__ __forceinline__ T iso_eps() { return ADMM_RC(T, 1e-15); }
+template <typename T> __device__ __forceinline__ T iso_scale(T n, T tau) { return xmax(T(1) - tau / (n + iso_eps<T>()), T(0)); }
 struct TauPos { static constexpr bool neg = false; };
 struct TauNeg { static constexpr bool neg = true; };
 
@@ -286,6 +290,21 @@ int  launch_cluster_solve(const Geometry& g, const ClusterArgs& a, cudaStream_t 
 bool coop_solver_supported(const Geometry& g);
 bool coop_solver_preferred(const Geometry& g);
 int  launch_coop_iterations(const Geometry& g, const Workspace& ws, const float* lmbd, const float* rho, int maxit, cudaStream_t st);
+
+// convergence residuals (resid.cu).  Buffer admm_ext.resid: history [check][plane][4], per-CTA partial sums, the device
+// flag and, when the solve may stop early, a spare spectrum (carve_resid; admm_query_resid)
+struct ResidBufs {
+    float*  hist;                      // (r, s, eps_pri, eps_dual) per check and plane
+    double* part;                      // [plane][block][5] partial sums of k_resid
+    int*    dflag;                     // 1 = every plane converged at the last check
+    float2* spare;                     // early stop: column pass k writes here, so S0 keeps X_k
+    int     nblk;                      // k_resid CTAs per plane
+};
+int    resid_checks(int maxit, int every);            // residual checks after iterations every, 2 every, ... <= maxit - 1
+size_t carve_resid(const Geometry& g, int maxit, int every, int early_stop, char* base, ResidBufs* rb);
+int    launch_resid(const Geometry& g, const float* qxp, const float* qyp, const float* qxk, const float* qyk, const float* np,
+                    const float* nk, const float* lmbd, const float* rho, const ResidBufs& rb, float* out, float rtol,
+                    float atol, cudaStream_t st);
 
 // large mixed-radix sizes (rows_big.cu, cols_big.cu): the 2160x3840 single-frame configuration
 bool rows_big_supported(const Geometry& g);

@@ -9,10 +9,6 @@
 
 namespace admm {
 
-// float and double (the float64 solve, f64.cu); the epsilon is a constant of the element type
-template <typename T> __device__ __forceinline__ T iso_eps() { return ADMM_RC(T, 1e-15); }
-template <typename T> __device__ __forceinline__ T iso_scale(T n, T tau) { return xmax(T(1) - tau / (n + iso_eps<T>()), T(0)); }
-
 template <typename T>
 __global__ void k_iso_prox(const T* __restrict__ x, const T* __restrict__ qxp, const T* __restrict__ qyp,
                            const T* __restrict__ n_prev, T* __restrict__ qxn, T* __restrict__ qyn,

@@ -11,7 +11,7 @@ from typing import Callable, Tuple
 
 import torch
 
-from ..eops.deconv import admm_solve, fft_admm_tv_f64, identity
+from ..eops.deconv import admm_solve, admm_solve_tol, fft_admm_tv_f64, identity
 
 __all__ = ["ADMMDeconv"]
 
@@ -45,6 +45,11 @@ class ADMMDeconv(torch.nn.Module):
         # not a constructor argument of the reference: set `layer.ckpt_interval = K` (or -1 for sqrt(max_iters)) to train
         # with checkpointed state (see admm_solve); 0 keeps the state of every iteration
         self.ckpt_interval = 0
+        # not a constructor argument either: `layer.tol = (rtol, atol, check_every)` makes a forward that needs no gradient
+        # stop at the first residual check where every plane has converged (admm_solve_tol); the solve's SolveInfo
+        # (iterations, residual history) is then kept in `last_solve_info`.  None (default): fixed max_iters
+        self.tol = None
+        self.last_solve_info = None
         # not a constructor argument either: "float64" solves in double (fft_admm_tv_f64) for a model converted with
         # `.double()`, like the reference does for float64 inputs; "float32" (default) is the fused float32 path
         self.precision = "float32"
@@ -70,6 +75,14 @@ class ADMMDeconv(torch.nn.Module):
         # activation(fft_admm_tv(x, lmbda, rho, w, iso, max_iters) + b)   (admmdeconv.py:63-64): the scalar bias and an
         # identity / relu / sigmoid / tanh activation are applied by the last kernel of the solve; any other callable
         # runs afterwards.  A uint8 image batch is read as x / 255 by the first kernel (etransforms.py:29-31).
+        tol = getattr(self, "tol", None)
+        if tol is not None and out is None and yhat is None and not (torch.is_grad_enabled() and any(
+                t.requires_grad for t in (x, self.lmbda, self.rho, self.w, self.b))):
+            rtol, atol, check_every = tol
+            res, self.last_solve_info = admm_solve_tol(x, self.lmbda, self.rho, self.w, self.iso, self.max_iters, rtol=rtol,
+                                                       atol=atol, check_every=check_every, bias=self.b,
+                                                       activation=self.activation)
+            return res
         return admm_solve(x, self.lmbda, self.rho, self.w, self.iso, self.max_iters, bias=self.b,
                           activation=self.activation, out=out, yhat=yhat, ckpt_interval=getattr(self, "ckpt_interval", 0))
 

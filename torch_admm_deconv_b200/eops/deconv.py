@@ -18,7 +18,8 @@ import torch.nn.functional as F
 from .. import _lib
 
 __all__ = ["fft_admm_tv", "soft_thresh", "block_thresh", "pixelnorm", "hard_thresh", "torch_abs2", "identity",
-           "conv_circular", "admm_solve", "activation_code", "shared_spectrum", "fft_admm_tv_cast", "fft_admm_tv_f64"]
+           "conv_circular", "admm_solve", "admm_solve_tol", "SolveInfo", "activation_code", "shared_spectrum",
+           "fft_admm_tv_cast", "fft_admm_tv_f64"]
 
 
 # ------------------------------------------------------------------------------------------------
@@ -139,7 +140,7 @@ def _act_grad(act: int, out: torch.Tensor, g: torch.Tensor) -> torch.Tensor:
 
 class _AdmmTV(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, xin, lmbd, rho, kern, bias, iso, maxit, need_grad, act, out_view, yhat=None, ckpt=0):
+    def forward(ctx, xin, lmbd, rho, kern, bias, iso, maxit, need_grad, act, out_view, yhat=None, ckpt=0, resid=None):
         lib = _lib.load()
         B, C, H, W = xin.shape
         dev = xin.device
@@ -176,6 +177,15 @@ class _AdmmTV(torch.autograd.Function):
                     saved_bytes = lib.admm_query_saved(B * C, H, W, ksize, int(iso), maxit)
                 saved = _workspace(saved_bytes, dev)
                 ext.ckpt_interval = ckpt
+            if resid is not None:                      # residual history / tolerance (admm_solve_tol)
+                stop = resid.rtol > 0 or resid.atol > 0
+                resid.buf = _workspace(lib.admm_query_resid(B * C, H, W, maxit, resid.every, int(stop)), dev)
+                ext.resid = resid.buf.data_ptr()
+                ext.resid_every = resid.every
+                ext.rtol, ext.atol = resid.rtol, resid.atol
+                if stop:
+                    ext.host_flag = _host_flag(dev).data_ptr()
+                ext.iters_out = ctypes.addressof(resid.iters)
             stream = torch.cuda.current_stream(dev).cuda_stream
             st = lib.admm_tv_forward_ex(_ptr(x), _ptr(out), _ptr(kern_d), ksize, _ptr(lam_d), _ptr(rho_d), _ptr(bias_d),
                                         B, C, H, W, int(iso), maxit, _ptr(ws), ws.numel(),
@@ -222,7 +232,7 @@ class _AdmmTV(torch.autograd.Function):
                 gl.reshape(lshape) if gl is not None else None,
                 gr.reshape(rshape) if gr is not None else None,
                 gk.reshape(kshape) if gk is not None else None,
-                gb, None, None, None, None, None, None, None)
+                gb, None, None, None, None, None, None, None, None)
 
 
 def shared_spectrum(xin: torch.Tensor) -> Optional[torch.Tensor]:
@@ -339,6 +349,103 @@ def admm_solve(xin: torch.Tensor, lmbd, rho, kern, iso: bool = False, maxit: int
         return out
     res = _AdmmTV.apply(xin, lmbd, rho, kern, bias, bool(iso), maxit, need_grad, code, out, yhat, ckpt_interval)
     return res if act is not None else activation(res)
+
+
+class SolveInfo:
+    """What `admm_solve_tol` reports about a solve.
+
+    iters      x-updates performed: maxit, or the iteration k at which every plane met the tolerance
+    residuals  float32 CUDA tensor (checks, B, C, 4): per check (after iterations M, 2M, ... with M = check_every) and
+               plane, (r, s, eps_pri, eps_dual) -- primal residual ||u_k - u_{k-1}||, dual residual
+               rho ||D^T(z_k - z_{k-1})|| and the two tolerances they are compared with (DESIGN.md section 10)"""
+
+    __slots__ = ("iters", "residuals")
+
+    def __init__(self, iters, residuals):
+        self.iters = iters
+        self.residuals = residuals
+
+    def __repr__(self):
+        return "SolveInfo(iters=%d, residuals=%s)" % (self.iters, tuple(self.residuals.shape))
+
+
+class _ResidRequest:
+    """Residual settings of one call and what the call hands back (filled by _AdmmTV.forward)."""
+
+    def __init__(self, every, rtol, atol):
+        self.every, self.rtol, self.atol = every, rtol, atol
+        self.buf = None
+        self.iters = ctypes.c_int(0)
+
+
+_HOST_FLAGS = {}
+
+
+def _host_flag(dev: torch.device) -> torch.Tensor:
+    """Pinned host int a tolerance check copies its "every plane converged" flag into; one per device."""
+    key = dev.index if dev.index is not None else torch.cuda.current_device()
+    t = _HOST_FLAGS.get(key)
+    if t is None:
+        t = _HOST_FLAGS[key] = torch.zeros(1, dtype=torch.int32, pin_memory=True)
+    return t
+
+
+def admm_solve_tol(xin: torch.Tensor, lmbd, rho, kern, iso: bool = False, maxit: int = 100, rtol: float = 1e-3,
+                   atol: float = 0.0, check_every: int = 10, bias: Optional[torch.Tensor] = None, activation=None,
+                   ckpt_interval: int = 0):
+    """`admm_solve` with convergence residuals and, optionally, a tolerance-based stop.  Returns (out, SolveInfo).
+
+    After iterations k = M, 2M, ... <= maxit - 1 (M = check_every) the primal and dual residuals of the splitting
+    Dx - z = 0 are computed per plane (Boyd et al. 2011, section 3.3; DESIGN.md section 10):
+        r_k = ||u_k - u_{k-1}||,  s_k = rho ||D^T(z_k - z_{k-1})||,
+        eps_pri = sqrt(2HW) atol + rtol max(||Dx_k||, ||z_k||),  eps_dual = sqrt(HW) atol + rtol rho ||D^T u_k||.
+    With rtol > 0 or atol > 0 the solve stops at the first check k at which every plane of the batch has
+    r_k <= eps_pri and s_k <= eps_dual, and returns x_k: bit for bit what `admm_solve(..., maxit=k)` returns on the
+    same kernel route.  Each check then waits for its result on the host, so the call synchronises with the GPU and
+    cannot be captured in a CUDA graph.  Stopping early is for inference: with gradients required a tolerance raises
+    ValueError.  rtol = atol = 0 records the history only: the solve runs maxit iterations, does not synchronise and
+    stays differentiable (same backward and saved state as `admm_solve`).
+    `bias`, `activation` and `ckpt_interval` as for `admm_solve`."""
+    if torch.cuda.is_available() and torch.cuda.is_current_stream_capturing():
+        raise RuntimeError("admm_solve_tol returns host-side results (iters, early stop): not available during CUDA-graph "
+                           "capture; use admm_solve")
+    rtol, atol, check_every, maxit = float(rtol), float(atol), int(check_every), int(maxit)
+    if not (rtol >= 0 and atol >= 0):
+        raise ValueError("rtol and atol must be >= 0 (got %r, %r)" % (rtol, atol))
+    if check_every < 1:
+        raise ValueError("check_every must be >= 1 (got %d)" % check_every)
+    ckpt_interval = int(ckpt_interval)
+    if ckpt_interval < 0:
+        ckpt_interval = int(math.ceil(math.sqrt(max(maxit - 1, 1))))
+    if not torch.is_tensor(xin):
+        raise TypeError("xin must be a torch.Tensor")
+    if xin.dim() != 4:
+        raise ValueError("xin must be 4-D (B, C, H, W), got %d-D" % xin.dim())
+    if not xin.is_cuda:
+        raise RuntimeError("torch_admm_deconv_b200 runs on CUDA (sm_100a) tensors only; there is no CPU fallback")
+    if xin.dtype not in (torch.float32, torch.uint8):
+        raise TypeError("float32 inputs (or uint8 images, read as x / 255) are supported by the sm_100a kernels (got %s)"
+                        % xin.dtype)
+    lmbd = _scalar_param(lmbd, xin.device, "lmbd")
+    rho = _scalar_param(rho, xin.device, "rho")
+    if kern is None:
+        kern = xin.new_empty(0, dtype=torch.float32)
+    act = activation_code(activation)
+    need_grad = torch.is_grad_enabled() and any(
+        torch.is_tensor(t) and t.requires_grad for t in (xin, lmbd, rho, kern, bias))
+    if need_grad and (rtol > 0 or atol > 0):
+        raise ValueError("a tolerance (rtol / atol > 0) stops inference early and has no backward; run under "
+                         "torch.no_grad(), or pass rtol = atol = 0 for a differentiable solve with residual history")
+    req = _ResidRequest(check_every, rtol, atol)
+    res = _AdmmTV.apply(xin, lmbd, rho, kern, bias, bool(iso), maxit, need_grad, act if act is not None else _lib.ACT_NONE,
+                        None, None, ckpt_interval, req)
+    B, C = xin.shape[:2]
+    iters = int(req.iters.value)
+    checks = min(iters, maxit - 1) // check_every if maxit > 1 else 0
+    hist = (req.buf[:checks * B * C * 16].view(torch.float32).reshape(checks, B, C, 4).clone() if req.buf is not None
+            else torch.empty((0, B, C, 4), dtype=torch.float32, device=xin.device))
+    out = res if act is not None else activation(res)
+    return out, SolveInfo(iters, hist)
 
 
 def fft_admm_tv_cast(xin: torch.Tensor, lmbd, rho, kern, iso: bool = False, maxit: int = 100) -> torch.Tensor:
