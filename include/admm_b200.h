@@ -109,6 +109,15 @@ typedef struct admm_ext {
     float     rtol, atol;        /* either > 0: stop at the first check where every plane has converged (saved == NULL only) */
     int*      host_flag;         /* pinned host int the check copies into; required when stopping early */
     int*      iters_out;         /* optional host int: x-updates performed (maxit unless stopped early) */
+    /* Spatially varying regularisation (DESIGN section 11).  tau_map != NULL: the threshold of element (b, c, h, w) is
+     * tau_map[(tau_map_planes > 1 ? b*C + c : 0) * H*W + h*W + w] instead of lmbd / rho, and `lmbd` is not read (may be
+     * NULL).  The caller forms tau = lambda / rho (the reference's deconv.py:44 applied element by element).  fp32, device,
+     * 16-byte aligned; tau_map_planes = 1 (one H x W map shared by every plane) or B*C.  iso = 1 takes a shared map only.
+     * Entries may be negative or zero, with the meaning of a scalar tau of that sign.  Not combined with resid_every or a
+     * tolerance.  The iterations run on the generic row kernel (any width); the column kernels are those of the scalar
+     * solve.  Training: pass the same map to admm_tv_backward_map. */
+    const float* tau_map;
+    int       tau_map_planes;
 } admm_ext;
 
 /* Bytes of admm_ext.resid for this problem: the history of (maxit - 1) / resid_every checks (none for maxit <= 1), scratch,
@@ -156,6 +165,23 @@ int admm_tv_backward_ex(const float* y, const float* grad_out,
                         void* workspace, size_t workspace_bytes,
                         float* grad_y, float* grad_kern, float* grad_lmbd, float* grad_rho,
                         void* stream, int ckpt_interval);
+
+/* Backward of a forward that ran with admm_ext.tau_map (and ckpt_interval K, 0 = every iteration kept).  Same as
+ * admm_tv_backward_ex with the map in place of lmbd:
+ *   grad_tau : tau_map_planes x H x W, the map's layout (overwritten).  A shared map's gradient is summed over the planes
+ *              in plane order, without atomics: the backward stays bit-reproducible.
+ *   grad_rho : one float, the gradient at FIXED tau (the spectral part).  A caller that forms tau = lambda / rho adds the
+ *              path through tau itself (autograd of that division does).
+ * Workspace: admm_query_workspace_backward_map (0 on an invalid request). */
+size_t admm_query_workspace_backward_map(int planes, int H, int W, int ksize, int iso, int maxit, int ckpt_interval,
+                                         int tau_map_planes);
+int admm_tv_backward_map(const float* y, const float* grad_out, const float* kern, int ksize,
+                         const float* tau_map, int tau_map_planes, const float* rho,
+                         int B, int C, int H, int W, int iso, int maxit,
+                         const void* saved, size_t saved_bytes,
+                         void* workspace, size_t workspace_bytes,
+                         float* grad_y, float* grad_kern, float* grad_tau, float* grad_rho,
+                         void* stream, int ckpt_interval);
 
 /* ---- float64 solve.  The reference computes in xin.dtype (deconv.py:50-67); these calls are the float32 ones above with
  * double in place of float for every tensor (y, out, kern, lmbd, rho, saved state, gradients), same conventions, error

@@ -39,7 +39,7 @@ class AdmmExt(ctypes.Structure):
     _fields_ = [("struct_size", _i), ("in_dtype", _i), ("activation", _i), ("ckpt_interval", _i),
                 ("out_batch_stride", ctypes.c_longlong), ("yhat_in", _vp), ("yhat_out", _vp),
                 ("resid", _vp), ("resid_every", _i), ("rtol", ctypes.c_float), ("atol", ctypes.c_float),
-                ("host_flag", _vp), ("iters_out", _vp)]
+                ("host_flag", _vp), ("iters_out", _vp), ("tau_map", _vp), ("tau_map_planes", _i)]
 
 
 IN_F32, IN_U8_DIV255 = 0, 1
@@ -52,6 +52,10 @@ SIGNATURES["admm_query_workspace_backward_ex"] = (_sz, [_i] * 7)
 SIGNATURES["admm_tv_backward_ex"] = (_i, SIGNATURES["admm_tv_backward"][1] + [_i])
 SIGNATURES["admm_spectrum_forward"] = (_i, [_vp, _i, _vp, _i, _i, _i, _vp, _sz, _vp])
 SIGNATURES["admm_tv_forward_ex"] = (_i, SIGNATURES["admm_tv_forward"][1] + [ctypes.POINTER(AdmmExt)])
+# threshold maps (admm_ext.tau_map): the backward takes the map in place of lmbd and returns grad_tau in its layout
+SIGNATURES["admm_query_workspace_backward_map"] = (_sz, [_i] * 8)
+SIGNATURES["admm_tv_backward_map"] = (_i, [_vp, _vp, _vp, _i, _vp, _i, _vp, _i, _i, _i, _i, _i, _i, _vp, _sz, _vp, _sz,
+                                           _vp, _vp, _vp, _vp, _vp, _i])
 # float64 solve: the float32 calls with double tensors (admm_tv_forward_f64 has no bias argument)
 SIGNATURES["admm_query_workspace_f64"] = (_sz, [_i] * 6)
 SIGNATURES["admm_query_workspace_backward_f64"] = (_sz, [_i] * 6)

@@ -132,6 +132,18 @@ int make_geometry_pub(int planes, int H, int W, Geometry* g) { return make_geome
 bool ckpt_supported(const Geometry& g) { return !g.iso; }
 int check_kernel_pub(int ksize, int H, int W) { return check_kernel(ksize, H, W); }
 
+// threshold maps (admm_ext.tau_map, admm_tv_backward_map): checked before anything is launched
+int check_tau_map(const float* tau_map, int tau_map_planes, int planes, int iso) {
+    if (!tau_map) return fail(ADMM_ERR_INVALID, "tau_map is NULL");
+    if ((uintptr_t)tau_map & 15) return fail(ADMM_ERR_INVALID, "tau_map is not 16-byte aligned");
+    if (tau_map_planes != 1 && tau_map_planes != planes)
+        return fail(ADMM_ERR_INVALID, "tau_map_planes must be 1 (one H x W map for every plane) or B*C");
+    if (iso && tau_map_planes != 1)
+        return fail(ADMM_ERR_INVALID, "iso = 1 takes one H x W map (tau_map_planes = 1): the block threshold scales every "
+                                      "plane of a pixel by one factor");
+    return 0;
+}
+
 }  // namespace admm
 
 using namespace admm;
@@ -173,11 +185,14 @@ static int solve_planes(const Geometry& g, const Geometry& gall, const Workspace
     RowArgs ra; std::memset(&ra, 0, sizeof(ra));
     ColArgs ca; std::memset(&ca, 0, sizeof(ca));
     ra.tw = ws.twW; ra.lmbd = lmbd; ra.rho = rho;
+    const bool map = ext.tau_map != nullptr;         // threshold map (DESIGN section 11): generic rows, no fused variants
     ca.tw = ws.twH; ca.A = ws.A; ca.Bm = ws.Bm; ca.Bq = ws.Bq; ca.Bmt = ws.Bmt; ca.Mul = ws.Mul; ca.Mq = ws.Mq;
 
     // 2160x3840 frames: between the two large kernels the packed spectra travel tile-major (common.cuh, kSpecTile);
     // the generic R2C before the loop and C2R after it keep the row-major layout
-    const bool tiled = rows_big_supported(g) && cols_big_supported(g);
+    // a map with iso = 0 runs its iterations on the generic row kernel, which reads row-major spectra; iso = 1 reads tau in
+    // its prox kernel only and keeps the large-frame layout
+    const bool tiled = rows_big_supported(g) && cols_big_supported(g) && !(map && !iso);
     if (!ext.yhat_in) {
         ra.real_in = y; ra.real_in_u8 = y8; ra.spec_out = ws.S1;
         if (int e = launch_rows(ROWS_R2C, g, ra, st)) return e;
@@ -202,7 +217,7 @@ static int solve_planes(const Geometry& g, const Geometry& gall, const Workspace
 
     const float* qx_prev = nullptr; const float* qy_prev = nullptr;
     // small, latency-bound batches (inference): iterations 1 .. maxit-1 in ONE cooperative launch (coop_small.cu)
-    const bool coop = !saved && !rr && maxit > 1 && !tiled && coop_solver_supported(g) && coop_solver_preferred(g);
+    const bool coop = !saved && !rr && !map && maxit > 1 && !tiled && coop_solver_supported(g) && coop_solver_preferred(g);
     if (coop) {
         if (int e = launch_coop_iterations(g, ws, lmbd, rho, maxit, st)) return e;
     }
@@ -233,7 +248,12 @@ static int solve_planes(const Geometry& g, const Geometry& gall, const Workspace
             n_new = nm;
             ra.spec_in = S0; ra.real_out = ws.xreal; ra.bias = nullptr; ra.tiled = tiled ? 1 : 0;
             if (int e = launch_rows(ROWS_C2R, g, ra, st)) return e;
-            if (int e = launch_iso_prox(g, ws.xreal, qx_prev, qy_prev, n_prev, qx_new, qy_new, nm, ws.sbmap, lmbd, rho, st)) return e;
+            if (map) {
+                if (int e = launch_iso_prox_map(g, ws.xreal, qx_prev, qy_prev, n_prev, qx_new, qy_new, nm, ws.sbmap, ext.tau_map, st))
+                    return e;
+            } else if (int e = launch_iso_prox(g, ws.xreal, qx_prev, qy_prev, n_prev, qx_new, qy_new, nm, ws.sbmap, lmbd, rho, st)) {
+                return e;
+            }
             if (rows_pow2_supported(g) || rows_big_supported(g)) {   // divergence fused into the R2C row pass
                 RowArgs rb = ra;
                 rb.r2c_div = 1; rb.cmap = ws.sbmap; rb.qx_in = qx_new; rb.qy_in = qy_new; rb.spec_out = ws.S1;
@@ -249,8 +269,11 @@ static int solve_planes(const Geometry& g, const Geometry& gall, const Workspace
             ra.tiled = tiled ? 1 : 0;
             // inference on the specialised kernels keeps the clamped dual as state (no clamp on reload); the residuals
             // need q itself (same results: DESIGN section 5)
-            const RowMode fm = (!saved && !rr && (rows_pow2_supported(g) || rows_big_supported(g))) ? ROWS_FULL_U : ROWS_FULL;
-            if (int e = launch_rows(fm, g, ra, st)) return e;
+            const RowMode fm = map ? ROWS_FULL_MAP
+                             : (!saved && !rr && (rows_pow2_supported(g) || rows_big_supported(g))) ? ROWS_FULL_U : ROWS_FULL;
+            RowArgs rf = ra;
+            if (map) { rf.cmap = ext.tau_map; rf.tau_map_planes = ext.tau_map_planes; }
+            if (int e = launch_rows(fm, g, rf, st)) return e;
         }
         const bool check = rr && it % rr->every == 0;
         if (check) {
@@ -451,10 +474,16 @@ int admm_tv_forward_ex(const void* y_any, float* out, const float* kern, int ksi
         if (cap != cudaStreamCaptureStatusNone)
             return fail(ADMM_ERR_INVALID, "a tolerance (admm_ext.rtol / atol) waits on the host: not available in CUDA-graph capture");
     }
+    const bool map = ext.tau_map != nullptr;
+    if (map) {
+        if (int e = check_tau_map(ext.tau_map, ext.tau_map_planes, B * C, iso)) return e;
+        if (ext.resid_every > 0 || tol)
+            return fail(ADMM_ERR_INVALID, "a threshold map (admm_ext.tau_map) does not combine with residuals or a tolerance");
+    }
     if (ext.iters_out) *ext.iters_out = maxit;
     const float* y = (ext.in_dtype == ADMM_IN_F32) ? (const float*)y_any : nullptr;
     const unsigned char* y8 = (ext.in_dtype == ADMM_IN_U8_DIV255) ? (const unsigned char*)y_any : nullptr;
-    if (!y_any || !out || !lmbd || !rho) return fail(ADMM_ERR_INVALID, "NULL tensor pointer");
+    if (!y_any || !out || (!lmbd && !map) || !rho) return fail(ADMM_ERR_INVALID, "NULL tensor pointer");
     if (B < 1 || C < 1) return fail(ADMM_ERR_INVALID, "B and C must be >= 1");
     if (maxit < 0) return fail(ADMM_ERR_INVALID, "maxit must be >= 0");
     if (ksize > 0 && !kern) return fail(ADMM_ERR_INVALID, "kern is NULL but ksize > 0");
@@ -477,7 +506,7 @@ int admm_tv_forward_ex(const void* y_any, float* out, const float* kern, int ksi
         }
         return 0;
     }
-    if (int e = check_generic_f32(g, !iso && maxit > 1)) return e;
+    if (int e = (map && !iso) ? check_generic_f32_map(g, maxit > 1) : check_generic_f32(g, !iso && maxit > 1)) return e;
     if (!workspace || ((uintptr_t)workspace & 255)) return fail(ADMM_ERR_WORKSPACE, "workspace is NULL or not 256-byte aligned");
     Workspace ws;
     const size_t need = carve_workspace(g, ksize, maxit, (char*)workspace, &ws);
@@ -514,7 +543,7 @@ int admm_tv_forward_ex(const void* y_any, float* out, const float* kern, int ksi
     }
 
     // ---- one or a few small planes: the cluster-resident solver runs the whole solve in one launch (cluster_pow2.cu)
-    if (!saved && !rr && !ext.yhat_in && !ext.yhat_out && cluster_solver_supported(g, iso, false) && cluster_solver_preferred(g)) {
+    if (!saved && !rr && !map && !ext.yhat_in && !ext.yhat_out && cluster_solver_supported(g, iso, false) && cluster_solver_preferred(g)) {
         ClusterArgs ka; std::memset(&ka, 0, sizeof(ka));
         ka.y = y; ka.y8 = y8; ka.out = out; ka.twW = ws.twW; ka.twH = ws.twH; ka.Bm = ws.Bm; ka.Bq = ws.Bq; ka.Mul = ws.Mul; ka.Mq = ws.Mq;
         ka.lmbd = lmbd; ka.rho = rho; ka.bias = bias; ka.act = ext.activation; ka.out_C = C; ka.out_p0 = 0;
@@ -534,7 +563,7 @@ int admm_tv_forward_ex(const void* y_any, float* out, const float* kern, int ksi
         int mb = options().chunk_mb;
         if (mb < 0) mb = kDefaultChunkMB;
         const size_t per_plane = (size_t)H * W * sizeof(float) * 7;
-        if (mb > 0 && !iso && !rr && maxit > 2) {
+        if (mb > 0 && !iso && !rr && !map && maxit > 2) {
             const size_t fit = ((size_t)mb << 20) / per_plane;
             if (fit >= 1 && (int)fit < g.P) {
                 // balanced chunks, each at least a wave's worth of work when possible

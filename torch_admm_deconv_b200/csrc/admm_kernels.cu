@@ -177,9 +177,11 @@ __device__ __forceinline__ void split_pairs(const V* __restrict__ res, int W, in
 // Threads per CTA of the generic kernels: float as tuned; double at most 256 (a radix-16 butterfly holds 32 doubles:
 // with 512 or 1024 threads the 128 / 64 registers per thread spill, with 256 nothing does)
 template <typename T> constexpr int kGenericMaxThreads = sizeof(T) == 4 ? 1024 : 256;
+// per mode: the threshold-map iteration holds five more values per element and is built for 512 threads (128 registers)
+template <int MODE, typename T> constexpr int kRowsMaxThreads = MODE == ROWS_FULL_MAP ? 512 : kGenericMaxThreads<T>;
 
 template <int MODE, typename T>
-__global__ void __launch_bounds__(kGenericMaxThreads<T>)
+__global__ void __launch_bounds__(kRowsMaxThreads<MODE, T>)
 k_rows(RowArgsT<T> a, FftPlan plan, int H, int W, int Wc, int R, int BS, int nbands) {
     using V = cplx_t<T>;
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -294,6 +296,76 @@ k_rows(RowArgsT<T> a, FftPlan plan, int H, int W, int Wc, int R, int BS, int nba
         split_pairs(res2, W, Wc, BS, r0, Rb, NPv, a.spec_out + plane_spec);
         return;
     }
+
+    if (MODE == ROWS_FULL_MAP) {
+        // ROWS_FULL with tau read per pixel from the map: every dual and every w = q - 2u of pixel (r, c) uses
+        // tau[r][c], so a q_x and the q_y of one pixel share a threshold (both are thresholded element by element,
+        // deconv.py:111-112 with a broadcast tensor lmbd).  The sign of tau varies inside a map: dual_any per element.
+        const int nrows = Rb + 2;
+        const int NP = (nrows + 1) / 2;
+        merge_pairs(a.spec_in + plane_spec, H, W, Wc, BS, r0 - 1, nrows, NP, bufA);
+        __syncthreads();
+        V* res = fft_batched<+1>(bufA, bufB, plan, NP, BS, tw);
+        V* zb = (res == bufA) ? bufB : bufA;
+        const T* tm = a.cmap + (a.tau_map_planes > 1 ? plane_real : 0);
+        const T* qxi = a.qx_in ? a.qx_in + plane_real : nullptr;
+        const T* qyi = a.qy_in ? a.qy_in + plane_real : nullptr;
+        T* qxo = a.qx_out + plane_real;
+        T* qyo = a.qy_out + plane_real;
+        const int NPv = (Rb + 1) / 2;
+        for (int w = threadIdx.x; w < NPv * W; w += blockDim.x) {
+            const int m = w / W, c = w - m * W;
+            const int cl = (c == 0) ? W - 1 : c - 1;
+            const int cr = (c == W - 1) ? 0 : c + 1;
+            const V P0c = res[c * BS + m],  P1c = res[c * BS + m + 1];
+            const V P0l = res[cl * BS + m], P1l = res[cl * BS + m + 1];
+            const V P0r = res[cr * BS + m], P1r = res[cr * BS + m + 1];
+            const int ra = r0 + 2 * m;
+            const bool hasb = (2 * m + 1 < Rb);
+            int rb = ra + 1; if (rb >= H) rb -= H;
+            int rc = rb + 1; if (rc >= H) rc -= H;
+            const T t_ac = tm[(size_t)ra * W + c], t_ar = tm[(size_t)ra * W + cr], t_bc = tm[(size_t)rb * W + c];
+            T t_br = T(0), t_cc = T(0);
+            if (hasb) { t_br = tm[(size_t)rb * W + cr]; t_cc = tm[(size_t)rc * W + c]; }
+            T uxa = 0, uxar = 0, uya = 0, uyb = 0, uxb = 0, uxbr = 0, uyc = 0;
+            if (qxi) {
+                uxa  = clampf(qxi[(size_t)ra * W + c], t_ac);
+                uxar = clampf(qxi[(size_t)ra * W + cr], t_ar);
+                uya  = clampf(qyi[(size_t)ra * W + c], t_ac);
+                uyb  = clampf(qyi[(size_t)rb * W + c], t_bc);
+                if (hasb) {
+                    uxb  = clampf(qxi[(size_t)rb * W + c], t_bc);
+                    uxbr = clampf(qxi[(size_t)rb * W + cr], t_br);
+                    uyc  = clampf(qyi[(size_t)rc * W + c], t_cc);
+                }
+            }
+            const T xu = P0c.x;
+            const T xa_c = P0c.y, xa_l = P0l.y, xa_r = P0r.y;
+            const T xb_c = P1c.x, xb_l = P1l.x, xb_r = P1r.x;
+            const T xd = P1c.y;
+            const T qx_a  = xa_c - xa_l + uxa;
+            const T qx_ar = xa_r - xa_c + uxar;
+            const T qy_a  = xa_c - xu + uya;
+            const T qy_b  = xb_c - xa_c + uyb;
+            const T va = wfun(qx_a, t_ac) - wfun(qx_ar, t_ar) + wfun(qy_a, t_ac) - wfun(qy_b, t_bc);
+            qxo[(size_t)ra * W + c] = qx_a;
+            qyo[(size_t)ra * W + c] = qy_a;
+            T vb = 0;
+            if (hasb) {
+                const T qx_b  = xb_c - xb_l + uxb;
+                const T qx_br = xb_r - xb_c + uxbr;
+                const T qy_c  = xd - xb_c + uyc;
+                vb = wfun(qx_b, t_bc) - wfun(qx_br, t_br) + wfun(qy_b, t_bc) - wfun(qy_c, t_cc);
+                qxo[(size_t)rb * W + c] = qx_b;
+                qyo[(size_t)rb * W + c] = qy_b;
+            }
+            zb[c * BS + m] = make_cplx(va, vb);
+        }
+        __syncthreads();
+        V* res2 = fft_batched<-1>(zb, res, plan, NPv, BS, tw);
+        split_pairs(res2, W, Wc, BS, r0, Rb, NPv, a.spec_out + plane_spec);
+        return;
+    }
 }
 
 template <typename T>
@@ -302,11 +374,13 @@ static size_t rows_smem(int W, int BS) { return ((size_t)2 * W * BS + W) * sizeo
 // the generic engine (any W); float and double
 template <typename T>
 static int launch_rows_generic(RowMode mode, const Geometry& g, const RowArgsT<T>& a, cudaStream_t st) {
-    if (mode == ROWS_ADJ || mode == ROWS_FULL_U) return fail(4, "this row-pass mode exists for power-of-two widths only");
+    if (mode == ROWS_ADJ || mode == ROWS_FULL_U || mode == ROWS_ADJ_MAP)
+        return fail(4, "this row-pass mode exists for power-of-two widths only");
+    if (mode == ROWS_FULL_MAP && sizeof(T) != 4) return fail(4, "threshold maps exist in the float32 solve only");
     FftPlan plan;
     if (!make_plan(g.W, plan)) return fail(4, "cannot plan row FFT length");
     const size_t kMax = 227 * 1024;
-    const int halo = (mode == ROWS_FULL) ? 2 : 0;
+    const int halo = (mode == ROWS_FULL || mode == ROWS_FULL_MAP) ? 2 : 0;
     int R = options().rows_per_band;
     if (R <= 0) R = 16;
     R = std::max(2, std::min(R, g.H + (g.H & 1)));
@@ -326,8 +400,9 @@ static int launch_rows_generic(RowMode mode, const Geometry& g, const RowArgsT<T
     const int nbands = (g.H + R - 1) / R;
     const size_t smem = rows_smem<T>(g.W, BS);
     // one or two fat CTAs per SM need more warps each to keep the SM busy
-    const int threads = std::min(kGenericMaxThreads<T>, options().threads > 0 ? options().threads.load()
-                                              : (smem > 113 * 1024 ? 1024 : (smem > 75 * 1024 ? 512 : 256)));
+    const int threads = std::min(mode == ROWS_FULL_MAP ? 512 : kGenericMaxThreads<T>,
+                                 options().threads > 0 ? options().threads.load()
+                                                       : (smem > 113 * 1024 ? 1024 : (smem > 75 * 1024 ? 512 : 256)));
     dim3 grid((unsigned)((size_t)nbands * g.P));
     // the opt-in shared-memory limit is a per-device function attribute: raised once to the maximum (the call costs
     // several microseconds of host time, which dominated small problems when it was repeated for every launch)
@@ -342,11 +417,14 @@ static int launch_rows_generic(RowMode mode, const Geometry& g, const RowArgsT<T
         }                                                                                                  \
         k_rows<M, T><<<grid, threads, smem, st>>>(a, plan, g.H, g.W, g.Wc, R, BS, nbands);                  \
     } while (0)
-    ProfScope ps(mode == ROWS_FULL ? PROF_ROWS : PROF_OTHER, st);
+    ProfScope ps((mode == ROWS_FULL || mode == ROWS_FULL_MAP) ? PROF_ROWS : PROF_OTHER, st);
     switch (mode) {
         case ROWS_R2C: ADMM_LAUNCH_ROWS(ROWS_R2C); break;
         case ROWS_C2R: ADMM_LAUNCH_ROWS(ROWS_C2R); break;
         case ROWS_FULL: ADMM_LAUNCH_ROWS(ROWS_FULL); break;
+        case ROWS_FULL_MAP:
+            if constexpr (sizeof(T) == 4) ADMM_LAUNCH_ROWS(ROWS_FULL_MAP);
+            break;
         default: break;
     }
 #undef ADMM_LAUNCH_ROWS
@@ -355,11 +433,17 @@ static int launch_rows_generic(RowMode mode, const Geometry& g, const RowArgsT<T
 }
 
 int launch_rows(RowMode mode, const Geometry& g, const RowArgs& a, cudaStream_t st) {
+    // a threshold map: the power-of-two kernel at its widths, else the generic one (also for the large-frame widths)
+    if (mode == ROWS_FULL_MAP && !rows_pow2_supported(g)) return launch_rows_generic(ROWS_FULL_MAP, g, a, st);
     if (rows_pow2_supported(g)) return launch_rows_pow2(mode, g, a, st);
     if ((mode == ROWS_FULL || mode == ROWS_FULL_U) && rows_big_supported(g)) return launch_rows_big(mode, g, a, st);
     if ((mode == ROWS_R2C || mode == ROWS_C2R) && rows_big_supported(g)) return launch_rows_big_plain(mode, g, a, st);
     return launch_rows_generic(mode, g, a, st);
 }
+
+// the generic R2C whatever the width: a checkpointed backward with a threshold map restarts a block from v recomputed
+// elementwise, and its spectrum must be the one the forward's generic row kernel formed (same FFT, same bits)
+int launch_rows_r2c_generic(const Geometry& g, const RowArgs& a, cudaStream_t st) { return launch_rows_generic(ROWS_R2C, g, a, st); }
 
 // float64: the generic engine only (no specialised double kernels)
 int launch_rows(RowMode mode, const Geometry& g, const RowArgsT<double>& a, cudaStream_t st) {
@@ -541,5 +625,8 @@ int check_generic_f64(const Geometry& g, bool full_rows) { return check_generic<
 int check_generic_f32(const Geometry& g, bool full_rows) {
     return check_generic<float>(g, !rows_pow2_supported(g) && !rows_big_supported(g), full_rows);
 }
+
+// a solve with a threshold map runs its iterations on the generic row kernel at every width
+int check_generic_f32_map(const Geometry& g, bool full_rows) { return check_generic<float>(g, true, full_rows); }
 
 }  // namespace admm

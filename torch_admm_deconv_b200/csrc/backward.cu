@@ -34,12 +34,15 @@ struct BwdWorkspace {
     float*  ck_slots;                       // K-1 slots of [q_x, q_y]
     float2* ck_A; float2* ck_S0; float2* ck_S1;
     float*  ck_v;
+    double* taubar_map;                     // threshold maps: per-element tau gradient, accumulated over the sweep
     size_t total;
 };
 
 static inline size_t align_up_b(size_t x) { return (x + 255) & ~(size_t)255; }
 
-static size_t carve_backward(const Geometry& g, int ksize, int ckpt, char* base, BwdWorkspace* out) {
+// tau_map_planes > 0: a solve with a threshold map; its tau-gradient accumulator (one double per element of the sweep's
+// terms: P x H x W for iso = 0, H x W for iso = 1) is carved after everything else, so the scalar layout is unchanged
+static size_t carve_backward(const Geometry& g, int ksize, int ckpt, char* base, BwdWorkspace* out, int tau_map_planes = 0) {
     size_t off = 0;
     auto take = [&](size_t bytes) { char* p = base ? base + off : nullptr; off += align_up_b(bytes); return p; };
     BwdWorkspace w;
@@ -71,6 +74,9 @@ static size_t carve_backward(const Geometry& g, int ksize, int ckpt, char* base,
         w.ck_S1 = (float2*)take(g.spec_bytes);
         w.ck_v = (float*)take(g.field_bytes);
     }
+    w.taubar_map = nullptr;
+    if (tau_map_planes > 0)
+        w.taubar_map = (double*)take((g.iso ? (size_t)g.H * g.W : (size_t)g.P * g.H * g.W) * sizeof(double));
     w.total = off;
     if (out) *out = w;
     return off;
@@ -146,6 +152,75 @@ __global__ void k_bwd_recompute_v(const T* __restrict__ qx, const T* __restrict_
         auto wf = [tau](T q) { return xfma(T(-2), dual_any(q, tau), q); };
         const size_t i00 = pl + (size_t)r * W + c;
         v[i00] = wf(qx[i00]) - wf(qx[pl + (size_t)r * W + cr]) + wf(qy[i00]) - wf(qy[pl + (size_t)rd * W + c]);
+    }
+}
+
+// ---- threshold maps (lambda maps, DESIGN section 11): the two kernels above with tau read per element.  tau of element
+// i of plane p is tau_map[(tmp > 1 ? p : 0) H W + pixel]; the tau gradient of element i is added into taubar[i]
+// (P x H x W doubles: one writer per element and launch, so the sums are deterministic).  float only.
+__device__ __forceinline__ size_t tau_index(size_t i, size_t HW, int tmp) { return tmp > 1 ? i : i % HW; }
+
+__global__ void k_bwd_spatial_map(const float* __restrict__ vb, const float* __restrict__ ubx_in,
+                                  const float* __restrict__ uby_in, const float* __restrict__ qx,
+                                  const float* __restrict__ qy, float* __restrict__ ubx_out, float* __restrict__ uby_out,
+                                  float* __restrict__ xb, const float* __restrict__ tau_map, int tmp,
+                                  double* __restrict__ taubar, int H, int W, size_t total) {
+    const size_t HW = (size_t)H * W;
+    for (size_t idx = blockIdx.x * (size_t)blockDim.x + threadIdx.x; idx < total; idx += (size_t)gridDim.x * blockDim.x) {
+        const int c = (int)(idx % W);
+        const size_t rowi = idx / W;
+        const int r = (int)(rowi % H);
+        const size_t pl = (rowi / H) * HW;
+        const int cl = c == 0 ? W - 1 : c - 1, cr = c == W - 1 ? 0 : c + 1;
+        const int ru = r == 0 ? H - 1 : r - 1, rd = r == H - 1 ? 0 : r + 1;
+        const float* V = vb + pl;
+        const float v00 = V[(size_t)r * W + c];
+        const float wbx = v00 - V[(size_t)r * W + cl];
+        const float wby = v00 - V[(size_t)ru * W + c];
+        const float wbx_r = V[(size_t)r * W + cr] - v00;
+        const float wby_d = V[(size_t)rd * W + c] - v00;
+        const size_t i00 = pl + (size_t)r * W + c, i0r = pl + (size_t)r * W + cr, id0 = pl + (size_t)rd * W + c;
+        const float t00 = tau_map[tau_index(i00, HW, tmp)], t0r = tau_map[tau_index(i0r, HW, tmp)];
+        const float td0 = tau_map[tau_index(id0, HW, tmp)];
+        const float ubx = ubx_in ? ubx_in[i00] : 0.f, uby = uby_in ? uby_in[i00] : 0.f;
+        const float ubx_r = ubx_in ? ubx_in[i0r] : 0.f, uby_d = uby_in ? uby_in[id0] : 0.f;
+        const float qx0 = qx[i00], qy0 = qy[i00];
+        const float qbx = qbar_of(wbx, ubx, qx0, t00), qby = qbar_of(wby, uby, qy0, t00);
+        const float qbx_r = qbar_of(wbx_r, ubx_r, qx[i0r], t0r), qby_d = qbar_of(wby_d, uby_d, qy[id0], td0);
+        ubx_out[i00] = qbx; uby_out[i00] = qby;
+        xb[i00] = (qbx - qbx_r) + (qby - qby_d);
+        double t = 0.0;
+        if (fabsf(qx0) >= t00) t += (double)((ubx - 2.f * wbx) * (qx0 > 0.f ? 1.f : (qx0 < 0.f ? -1.f : 0.f)));
+        if (fabsf(qy0) >= t00) t += (double)((uby - 2.f * wby) * (qy0 > 0.f ? 1.f : (qy0 < 0.f ? -1.f : 0.f)));
+        taubar[idx] += t;
+    }
+}
+
+__global__ void k_bwd_recompute_v_map(const float* __restrict__ qx, const float* __restrict__ qy, float* __restrict__ v,
+                                      const float* __restrict__ tau_map, int tmp, int H, int W, size_t total) {
+    const size_t HW = (size_t)H * W;
+    for (size_t idx = blockIdx.x * (size_t)blockDim.x + threadIdx.x; idx < total; idx += (size_t)gridDim.x * blockDim.x) {
+        const int c = (int)(idx % W);
+        const size_t rowi = idx / W;
+        const int r = (int)(rowi % H);
+        const size_t pl = (rowi / H) * HW;
+        const int cr = c == W - 1 ? 0 : c + 1, rd = r == H - 1 ? 0 : r + 1;
+        // the operations and order of k_rows<ROWS_FULL_MAP> (admm_kernels.cu), so a checkpointed re-run matches the forward
+        const size_t i00 = pl + (size_t)r * W + c, i0r = pl + (size_t)r * W + cr, id0 = pl + (size_t)rd * W + c;
+        const float t00 = tau_map[tau_index(i00, HW, tmp)], t0r = tau_map[tau_index(i0r, HW, tmp)];
+        const float td0 = tau_map[tau_index(id0, HW, tmp)];
+        auto wf = [](float q, float tau) { return fmaf(-2.f, dual_any(q, tau), q); };
+        v[i00] = wf(qx[i00], t00) - wf(qx[i0r], t0r) + wf(qy[i00], t00) - wf(qy[id0], td0);
+    }
+}
+
+// grad_tau in the map's layout: tmp == P copies the per-element sums; a shared map (tmp == 1, n = H x W) adds the planes
+// of each pixel in plane order (iso = 1 accumulates per pixel already: nplanes = 1)
+__global__ void k_tau_map_grad(const double* __restrict__ taubar, int nplanes, size_t n, float* __restrict__ grad_tau) {
+    for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
+        double s = 0.0;
+        for (int p = 0; p < nplanes; ++p) s += taubar[(size_t)p * n + i];
+        grad_tau[i] = (float)s;
     }
 }
 
@@ -325,6 +400,15 @@ k_bwd_scalars(const double* __restrict__ tau_part, size_t n_tau, const double* _
     }
 }
 
+// threshold maps: the rho gradient at fixed tau is the spectral part alone (the tau term goes back through lmbd / rho in
+// the caller's autograd)
+__global__ void __launch_bounds__(256)
+k_bwd_rho_spectral(const double* __restrict__ rho_part, size_t n_rho, float* __restrict__ grad_rho) {
+    __shared__ double red[256];
+    const double rhospec = block_sum_256(rho_part, n_rho, red);
+    if (threadIdx.x == 0) grad_rho[0] = (float)rhospec;
+}
+
 static int ew_grid(size_t total) { return (int)std::min<size_t>((total + 255) / 256, 148 * 16); }
 
 // ---- the same kernels in double, for the float64 backward (f64.cu); launch shapes as in run_backward below
@@ -386,7 +470,11 @@ int launch_bwd_scalars(const double* tau_part, size_t n_tau, const double* rho_p
 int run_backward(const Geometry& g, const Workspace& ws, const BwdWorkspace& bw, const float* y, const float* grad_out,
                  const float* kern, int ksize, const float* lmbd, const float* rho, int maxit, const float* saved,
                  const float* saved_nmaps, int ckpt,
-                 float* grad_y, float* grad_kern, float* grad_lmbd, float* grad_rho, cudaStream_t st) {
+                 float* grad_y, float* grad_kern, float* grad_lmbd, float* grad_rho, cudaStream_t st,
+                 const float* tau_map = nullptr, int tmp = 0, float* grad_tau = nullptr) {
+    // tau_map != NULL (lambda maps, DESIGN section 11): tau per element, grad_tau in the map's layout instead of grad_lmbd,
+    // grad_rho at fixed tau.  The iterations re-run on the row kernel the forward ran (power-of-two, else generic); the
+    // power-of-two widths take the fused adjoint ROWS_ADJ_MAP, the others the elementwise adjoint kernels.
     const size_t fe = (size_t)g.P * g.H * g.W;
     // ---- saved state.  Slot i holds [q_x, q_y] after forward iteration i + 1 (slots 0 .. maxit-2).  Full mode: every
     // slot is in `saved`.  Checkpointed (K = ckpt >= 2): `saved` keeps the slots with (i + 1) % K == 0; the others of a
@@ -404,7 +492,7 @@ int run_backward(const Geometry& g, const Workspace& ws, const BwdWorkspace& bw,
     // The re-run uses the forward's kernels and layouts (abi.cu, solve_planes).  Large-frame row kernel: v is formed inside
     // its R2C from the checkpoint (r2c_div = 2) with the march's operation order; with both large-frame kernels the
     // spectra between them are tile-major and A is item-major (the layout COLS_INIT of cols_big.cu writes and COLS_ITER reads).
-    const bool big_rows = rows_big_supported(g);
+    const bool big_rows = rows_big_supported(g) && !tau_map;
     const int tiled = (big_rows && cols_big_supported(g)) ? 1 : 0;
     auto regen_block = [&](int b) -> int {
         RowArgs rr; std::memset(&rr, 0, sizeof(rr));
@@ -430,11 +518,17 @@ int run_backward(const Geometry& g, const Workspace& ws, const BwdWorkspace& bw,
             } else {
                 {
                     ProfScope ps(PROF_OTHER, st);
-                    k_bwd_recompute_v<<<ew_grid(fe), 256, 0, st>>>(qprev, qprev + fe, bw.ck_v, lmbd, rho, g.H, g.W, fe);
+                    if (tau_map)
+                        k_bwd_recompute_v_map<<<ew_grid(fe), 256, 0, st>>>(qprev, qprev + fe, bw.ck_v, tau_map, tmp, g.H, g.W, fe);
+                    else
+                        k_bwd_recompute_v<<<ew_grid(fe), 256, 0, st>>>(qprev, qprev + fe, bw.ck_v, lmbd, rho, g.H, g.W, fe);
                     ADMM_CUDA_CHECK(cudaGetLastError());
                 }
                 rr.real_in = bw.ck_v; rr.spec_out = bw.ck_S1;
-                if (int e = launch_rows(ROWS_R2C, g, rr, st)) return e;
+                // the restart's spectrum is formed by the R2C of the row kernel the forward ran (generic rows for a map at
+                // widths without a power-of-two kernel)
+                const bool gen = tau_map && !rows_pow2_supported(g);
+                if (int e = gen ? launch_rows_r2c_generic(g, rr, st) : launch_rows(ROWS_R2C, g, rr, st)) return e;
             }
             cc.spec_in = bw.ck_S1; cc.spec_out = bw.ck_S0; cc.in_tiled = tiled; cc.out_tiled = tiled;
             if (int e = launch_cols(COLS_ITER, g, cc, st)) return e;
@@ -444,7 +538,9 @@ int run_backward(const Geometry& g, const Workspace& ws, const BwdWorkspace& bw,
             float* qn = bw.ck_slots + (size_t)(i - m0) * 2 * fe;
             rr.spec_in = bw.ck_S0; rr.spec_out = bw.ck_S1;
             rr.qx_in = qprev; rr.qy_in = qprev ? qprev + fe : nullptr; rr.qx_out = qn; rr.qy_out = qn + fe;
-            if (int e = launch_rows(ROWS_FULL, g, rr, st)) return e;
+            RowArgs rf = rr;
+            if (tau_map) { rf.cmap = tau_map; rf.tau_map_planes = tmp; }
+            if (int e = launch_rows(tau_map ? ROWS_FULL_MAP : ROWS_FULL, g, rf, st)) return e;
             if (i + 1 < end) {                                           // another row pass follows: tile-major output
                 cc.spec_in = bw.ck_S1; cc.spec_out = bw.ck_S0; cc.in_tiled = tiled; cc.out_tiled = tiled;
                 if (int e = launch_cols(COLS_ITER, g, cc, st)) return e;
@@ -465,6 +561,8 @@ int run_backward(const Geometry& g, const Workspace& ws, const BwdWorkspace& bw,
     ADMM_CUDA_CHECK(cudaMemsetAsync(bw.GV, 0, (size_t)bw.nsplit * HWh * sizeof(double2), st));
     ADMM_CUDA_CHECK(cudaMemsetAsync(bw.tau_part, 0, bw.n_tau * sizeof(double), st));
     ADMM_CUDA_CHECK(cudaMemsetAsync(bw.rho_part, 0, bw.n_rho * sizeof(double), st));
+    const size_t n_taubar = g.iso ? (size_t)g.H * g.W : fe;
+    if (tau_map) ADMM_CUDA_CHECK(cudaMemsetAsync(bw.taubar_map, 0, n_taubar * sizeof(double), st));
 
     RowArgs ra; std::memset(&ra, 0, sizeof(ra));
     ColArgs ca; std::memset(&ca, 0, sizeof(ca));
@@ -505,24 +603,32 @@ int run_backward(const Geometry& g, const Workspace& ws, const BwdWorkspace& bw,
                 aa.spec_in = ws.S0; aa.spec_out = ws.S1;
                 aa.qx_in = qx; aa.qy_in = qy;
                 aa.ubx_in = ubx; aa.uby_in = uby; aa.ubx_out = nx; aa.uby_out = ny;
-                aa.taubar = bw.tau_part;
+                aa.taubar = tau_map ? bw.taubar_map : bw.tau_part;     // map: per element, else per CTA
+                if (tau_map) { aa.cmap = tau_map; aa.tau_map_planes = tmp; }
                 aa.qvx = nullptr; aa.qvy = nullptr; aa.spec_out2 = nullptr;
                 if (need_spec && k >= 1) {
                     aa.qvx = slot_ptr(k - 1); aa.qvy = aa.qvx + fe;
                     aa.spec_out2 = bw.ZV;                       // row spectrum of v_k, column-transformed in place below
                     zv_in_place = true;
                 }
-                if (int e = launch_rows(ROWS_ADJ, g, aa, st)) return e;
+                if (int e = launch_rows(tau_map ? ROWS_ADJ_MAP : ROWS_ADJ, g, aa, st)) return e;
             } else {
                 if (g.iso) {
                     const float* nm = saved_nmaps + (size_t)k * 2 * g.H * g.W;
                     // power-of-two sizes: xbar = D^T qbar is formed inside the R2C row pass (no xbar field in HBM)
-                    if (int e = launch_iso_bwd(g, bw.vb, ubx, uby, qx, qy, nm, ws.sbmap, nx, ny, iso_fused ? nullptr : bw.xb,
-                                               lmbd, rho, bw.tau_part, st)) return e;
+                    if (tau_map) {
+                        if (int e = launch_iso_bwd_map(g, bw.vb, ubx, uby, qx, qy, nm, nx, ny, iso_fused ? nullptr : bw.xb,
+                                                       tau_map, bw.taubar_map, st)) return e;
+                    } else if (int e = launch_iso_bwd(g, bw.vb, ubx, uby, qx, qy, nm, ws.sbmap, nx, ny, iso_fused ? nullptr : bw.xb,
+                                                      lmbd, rho, bw.tau_part, st)) return e;
                 } else {
                     ProfScope ps(PROF_OTHER, st);
-                    k_bwd_spatial<<<ew_grid(fe), 256, 0, st>>>(bw.vb, ubx, uby, qx, qy, nx, ny, bw.xb, lmbd, rho, bw.tau_part,
-                                                               g.H, g.W, fe);
+                    if (tau_map)
+                        k_bwd_spatial_map<<<ew_grid(fe), 256, 0, st>>>(bw.vb, ubx, uby, qx, qy, nx, ny, bw.xb, tau_map, tmp,
+                                                                       bw.taubar_map, g.H, g.W, fe);
+                    else
+                        k_bwd_spatial<<<ew_grid(fe), 256, 0, st>>>(bw.vb, ubx, uby, qx, qy, nx, ny, bw.xb, lmbd, rho, bw.tau_part,
+                                                                   g.H, g.W, fe);
                     ADMM_CUDA_CHECK(cudaGetLastError());
                 }
                 if (g.iso && iso_fused) {
@@ -544,16 +650,24 @@ int run_backward(const Geometry& g, const Workspace& ws, const BwdWorkspace& bw,
             if (g.iso && iso_fused) {
                 // v_k = D^T((2 s_k - 1) q_k): coefficient map from the saved norms, divergence inside the R2C row pass
                 const float* nm = saved_nmaps + (size_t)(k - 1) * 2 * g.H * g.W;
-                if (int e = launch_iso_cmap(g, nm, ws.sbmap, lmbd, rho, st)) return e;
+                if (tau_map) {
+                    if (int e = launch_iso_cmap_map(g, nm, ws.sbmap, tau_map, st)) return e;
+                } else if (int e = launch_iso_cmap(g, nm, ws.sbmap, lmbd, rho, st)) return e;
                 RowArgs rd = ra;
                 rd.r2c_div = 1; rd.cmap = ws.sbmap; rd.qx_in = qx; rd.qy_in = qx + fe; rd.spec_out = bw.ZV;
                 if (int e = launch_rows(ROWS_R2C, g, rd, st)) return e;
             } else if (g.iso) {
                 const float* nm = saved_nmaps + (size_t)(k - 1) * 2 * g.H * g.W;
-                if (int e = launch_iso_div(g, qx, qx + fe, nm, nullptr, bw.vb, lmbd, rho, st)) return e;
+                if (tau_map) {                                  // coefficient map first: k_iso_div then reads no tau
+                    if (int e = launch_iso_cmap_map(g, nm, ws.sbmap, tau_map, st)) return e;
+                    if (int e = launch_iso_div(g, qx, qx + fe, nm, ws.sbmap, bw.vb, lmbd, rho, st)) return e;
+                } else if (int e = launch_iso_div(g, qx, qx + fe, nm, nullptr, bw.vb, lmbd, rho, st)) return e;
             } else {
                 ProfScope ps(PROF_OTHER, st);
-                k_bwd_recompute_v<<<ew_grid(fe), 256, 0, st>>>(qx, qx + fe, bw.vb, lmbd, rho, g.H, g.W, fe);
+                if (tau_map)
+                    k_bwd_recompute_v_map<<<ew_grid(fe), 256, 0, st>>>(qx, qx + fe, bw.vb, tau_map, tmp, g.H, g.W, fe);
+                else
+                    k_bwd_recompute_v<<<ew_grid(fe), 256, 0, st>>>(qx, qx + fe, bw.vb, lmbd, rho, g.H, g.W, fe);
                 ADMM_CUDA_CHECK(cudaGetLastError());
             }
             if (!(g.iso && iso_fused)) {
@@ -620,6 +734,21 @@ int run_backward(const Geometry& g, const Workspace& ws, const BwdWorkspace& bw,
             k_bwd_kgrad_cols<<<(ksize * ksize + 63) / 64, 64, 0, st>>>(bw.Tk, grad_kern, g.H, ksize, ws.twHd);
             ADMM_CUDA_CHECK(cudaGetLastError());
         }
+    }
+    if (tau_map) {
+        ProfScope ps(PROF_OTHER, st);
+        if (grad_tau) {
+            // iso = 1 accumulated per pixel; iso = 0 per element, added over the planes here for a shared map
+            const int nplanes = (!g.iso && tmp == 1) ? g.P : 1;
+            const size_t n = n_taubar / nplanes;
+            k_tau_map_grad<<<ew_grid(n), 256, 0, st>>>(bw.taubar_map, nplanes, n, grad_tau);
+            ADMM_CUDA_CHECK(cudaGetLastError());
+        }
+        if (grad_rho) {
+            k_bwd_rho_spectral<<<1, 256, 0, st>>>(bw.rho_part, bw.n_rho, grad_rho);
+            ADMM_CUDA_CHECK(cudaGetLastError());
+        }
+        return 0;
     }
     if (grad_lmbd || grad_rho) {
         ProfScope ps(PROF_OTHER, st);
@@ -701,6 +830,64 @@ int admm_tv_backward_ex(const float* y, const float* grad_out, const float* kern
     const float* nmaps = (const float*)saved + (size_t)(maxit - 1) * 2 * ((size_t)g.P * H * W);
     return run_backward(g, ws, bw, y, grad_out, kern, ksize, lmbd, rho, maxit, (const float*)saved, nmaps, ckpt,
                         grad_y, grad_kern, grad_lmbd, grad_rho, st);
+}
+
+// ---- threshold maps (lambda maps, DESIGN section 11)
+size_t admm_query_workspace_backward_map(int planes, int H, int W, int ksize, int iso, int maxit, int ckpt_interval,
+                                         int tau_map_planes) {
+    Geometry g;
+    if (make_geometry_pub(planes, H, W, &g)) return 0;
+    if (check_kernel_pub(ksize, H, W)) return 0;
+    if (tau_map_planes != 1 && tau_map_planes != planes) return 0;
+    if (iso && tau_map_planes != 1) return 0;
+    g.iso = iso ? 1 : 0;
+    const int ckpt = ckpt_interval >= 2 ? ckpt_interval : 0;
+    if (ckpt && !ckpt_supported(g)) return 0;
+    return carve_workspace(g, ksize, maxit, nullptr, nullptr) + carve_backward(g, ksize, ckpt, nullptr, nullptr, tau_map_planes);
+}
+
+int admm_tv_backward_map(const float* y, const float* grad_out, const float* kern, int ksize,
+                         const float* tau_map, int tau_map_planes, const float* rho,
+                         int B, int C, int H, int W, int iso, int maxit,
+                         const void* saved, size_t saved_bytes, void* workspace, size_t workspace_bytes,
+                         float* grad_y, float* grad_kern, float* grad_tau, float* grad_rho, void* stream, int ckpt_interval) {
+    cudaStream_t st = (cudaStream_t)stream;
+    const int ckpt = ckpt_interval >= 2 ? ckpt_interval : 0;
+    if (!y || !grad_out || !rho) return fail(ADMM_ERR_INVALID, "NULL tensor pointer");
+    if (B < 1 || C < 1) return fail(ADMM_ERR_INVALID, "B and C must be >= 1");
+    if (maxit < 0) return fail(ADMM_ERR_INVALID, "maxit must be >= 0");
+    if (ksize > 0 && !kern) return fail(ADMM_ERR_INVALID, "kern is NULL but ksize > 0");
+    if (int e = check_tau_map(tau_map, tau_map_planes, B * C, iso)) return e;
+    Geometry g;
+    if (int e = make_geometry_pub(B * C, H, W, &g)) return e;
+    if (int e = check_kernel_pub(ksize, H, W)) return e;
+    g.iso = iso ? 1 : 0;
+    const size_t map_bytes = (size_t)tau_map_planes * H * W * sizeof(float);
+    if (maxit == 0) {
+        if (grad_y) ADMM_CUDA_CHECK(cudaMemsetAsync(grad_y, 0, g.field_bytes, st));
+        if (grad_kern && ksize > 0) ADMM_CUDA_CHECK(cudaMemsetAsync(grad_kern, 0, (size_t)ksize * ksize * sizeof(float), st));
+        if (grad_tau) ADMM_CUDA_CHECK(cudaMemsetAsync(grad_tau, 0, map_bytes, st));
+        if (grad_rho) ADMM_CUDA_CHECK(cudaMemsetAsync(grad_rho, 0, sizeof(float), st));
+        return 0;
+    }
+    if (int e = check_generic_f32_map(g, ckpt != 0)) return e;
+    if (!workspace || ((uintptr_t)workspace & 255)) return fail(ADMM_ERR_WORKSPACE, "workspace is NULL or not 256-byte aligned");
+    if (ckpt && !ckpt_supported(g)) return fail(ADMM_ERR_UNSUPPORTED, "checkpointed training is not available for this problem");
+    Workspace ws; BwdWorkspace bw;
+    const size_t n1 = carve_workspace(g, ksize, maxit, (char*)workspace, &ws);
+    const size_t n2 = carve_backward(g, ksize, ckpt, (char*)workspace + n1, &bw, tau_map_planes);
+    if (workspace_bytes < n1 + n2) return fail(ADMM_ERR_WORKSPACE, "workspace too small (use admm_query_workspace_backward_map)");
+    const size_t kept = ckpt ? (size_t)((maxit - 1) / ckpt) : (size_t)(maxit - 1);
+    const size_t need_saved = kept * 2 * g.field_bytes + (iso ? (size_t)(maxit - 1) * 2 * H * W * sizeof(float) : 0);
+    if (maxit > 1 && need_saved > 0 && (!saved || saved_bytes < need_saved)) return fail(ADMM_ERR_WORKSPACE, "saved state missing or too small");
+    if (int e = launch_twiddles(ws.twW, ws.twWd, W, st)) return e;
+    if (int e = launch_twiddles(ws.twH, ws.twHd, H, st)) return e;
+    if (int e = launch_tables(g, ws, kern, ksize, rho, st)) return e;
+    if (cols_big_supported(g))
+        if (int e = launch_bm_tiled(g, ws.Bm, ws.Bmt, st)) return e;
+    const float* nmaps = (const float*)saved + (size_t)(maxit - 1) * 2 * ((size_t)g.P * H * W);
+    return run_backward(g, ws, bw, y, grad_out, kern, ksize, nullptr, rho, maxit, (const float*)saved, nmaps, ckpt,
+                        grad_y, grad_kern, nullptr, grad_rho, st, tau_map, tau_map_planes, grad_tau);
 }
 
 }  // extern "C"

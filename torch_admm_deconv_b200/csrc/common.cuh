@@ -73,6 +73,7 @@ struct Workspace {
 
 size_t carve_workspace(const Geometry& g, int ksize, int maxit, char* base, Workspace* ws);
 bool   ckpt_supported(const Geometry& g);      // checkpointed training (admm_ext.ckpt_interval) available for this problem
+int    check_tau_map(const float* tau_map, int tau_map_planes, int planes, int iso);   // 0, or ADMM_ERR_INVALID with a message
 
 // Programmatic dependent launch: the iteration kernels may start (build their twiddle tables, set up indices) while the
 // previous kernel of the stream drains; they call pdl_wait() before touching anything the previous kernel wrote.
@@ -146,7 +147,10 @@ struct ProfScope {
 // ------------------------------------------------------------------ kernel launchers (admm_kernels.cu)
 // ROWS_FULL_U: like ROWS_FULL but the state arrays hold the clamped dual u = clamp(q) (inference: nothing is saved for a
 // backward, so the clamp on load disappears); power-of-two kernels only
-enum RowMode { ROWS_R2C = 0, ROWS_C2R = 1, ROWS_FULL = 2, ROWS_ADJ = 3, ROWS_FULL_U = 4 };
+// ROWS_FULL_MAP / ROWS_ADJ_MAP: ROWS_FULL / ROWS_ADJ with a per-pixel threshold map (lambda maps, DESIGN section 11).
+// ROWS_FULL_MAP runs on the power-of-two kernel at W in {128, 256, 512} and on the generic kernel at every other width;
+// ROWS_ADJ_MAP exists for the power-of-two widths and adds each element's tau gradient into RowArgs::taubar[element]
+enum RowMode { ROWS_R2C = 0, ROWS_C2R = 1, ROWS_FULL = 2, ROWS_ADJ = 3, ROWS_FULL_U = 4, ROWS_FULL_MAP = 5, ROWS_ADJ_MAP = 6 };
 // COLS_INIT_SPEC: like COLS_INIT but the input already is the column-transformed spectrum of y (shared by several solvers)
 enum ColMode { COLS_FFT_FWD = 0, COLS_FFT_INV = 1, COLS_INIT = 2, COLS_ITER = 3, COLS_BM_INV = 4, COLS_CMUL_INV = 5, COLS_INIT_SPEC = 6 };
 
@@ -184,8 +188,14 @@ struct RowArgsT {
     V*            spec_out2;
     const V*      tw;
     int tiled;                // large kernels: spec_in / spec_out are tile-major (see kSpecTile)
+    // ROWS_FULL_MAP (threshold map, admm_ext.tau_map): the map travels in `cmap` (which the iteration modes never read);
+    // tau of pixel (r, c) of plane p is cmap[(tau_map_planes > 1 ? p : 0) H W + r W + c], and lmbd / rho are not read.
+    // The count sits in the struct's tail padding: sizeof and every offset stay those of the scalar kernels' parameters
+    int           tau_map_planes;
 };
 using RowArgs = RowArgsT<float>;
+static_assert(sizeof(RowArgsT<float>) == 27 * 8, "RowArgs is a kernel parameter: its size and layout are part of the ABI "
+                                                 "of every row kernel");
 
 // Tile-major packed spectrum shared by the two large-frame kernels (rows_big.cu <-> cols_big.cu): per plane
 // [tile = col / 8][row pair][col % 8][row in pair] float2.  One row pair of one tile is a 128-byte run for the row kernel
@@ -213,6 +223,7 @@ int launch_twiddles(float2* tw, double2* twd, int N, cudaStream_t st);
 int launch_tables(const Geometry& g, const Workspace& ws, const float* kern, int ksize,
                   const float* rho, cudaStream_t st);
 int launch_rows(RowMode mode, const Geometry& g, const RowArgs& a, cudaStream_t st);
+int launch_rows_r2c_generic(const Geometry& g, const RowArgs& a, cudaStream_t st);
 int launch_cols(ColMode mode, const Geometry& g, const ColArgs& a, cudaStream_t st);
 
 // fused backward column pass (cols_pow2.cu)
@@ -225,6 +236,14 @@ int launch_iso_prox(const Geometry& g, const float* x, const float* qx_prev, con
                     float* qx_new, float* qy_new, float* n_new, float* c_new, const float* lmbd, const float* rho,
                     cudaStream_t st);
 int launch_iso_cmap(const Geometry& g, const float* nmap, float* cmap, const float* lmbd, const float* rho, cudaStream_t st);
+// the same with an H x W threshold map (lambda maps, iso = 1: one tau per pixel shared by every plane); the backward adds
+// each pixel's tau gradient into taubar_map[pixel] (double, one writer per pixel and launch)
+int launch_iso_prox_map(const Geometry& g, const float* x, const float* qx_prev, const float* qy_prev, const float* n_prev,
+                        float* qx_new, float* qy_new, float* n_new, float* c_new, const float* tau_map, cudaStream_t st);
+int launch_iso_cmap_map(const Geometry& g, const float* nmap, float* cmap, const float* tau_map, cudaStream_t st);
+int launch_iso_bwd_map(const Geometry& g, const float* vb, const float* ubx_in, const float* uby_in, const float* qx,
+                       const float* qy, const float* nmap, float* ubx_out, float* uby_out, float* xb, const float* tau_map,
+                       double* taubar_map, cudaStream_t st);
 int launch_iso_div(const Geometry& g, const float* qx, const float* qy, const float* nmap, const float* cmap, float* v,
                    const float* lmbd, const float* rho, cudaStream_t st);
 int launch_iso_bwd(const Geometry& g, const float* vb, const float* ubx_in, const float* uby_in, const float* qx,
@@ -239,6 +258,7 @@ int launch_rows(RowMode mode, const Geometry& g, const RowArgsT<double>& a, cuda
 int launch_cols(ColMode mode, const Geometry& g, const ColArgsT<double>& a, cudaStream_t st);
 int check_generic_f64(const Geometry& g, bool full_rows);       // 0, or ADMM_ERR_UNSUPPORTED with a message
 int check_generic_f32(const Geometry& g, bool full_rows);       // the same for the float32 solver's generic passes
+int check_generic_f32_map(const Geometry& g, bool full_rows);   // ... of a solve with a threshold map (generic rows always)
 int launch_iso_prox(const Geometry& g, const double* x, const double* qx_prev, const double* qy_prev, const double* n_prev,
                     double* qx_new, double* qy_new, double* n_new, double* c_new, const double* lmbd, const double* rho,
                     cudaStream_t st);

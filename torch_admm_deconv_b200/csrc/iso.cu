@@ -242,6 +242,148 @@ static int launch_iso_bwd_t(const Geometry& g, const T* vb, const T* ubx_in, con
     return 0;
 }
 
+// ---- threshold maps (lambda maps, DESIGN section 11): the kernels above with tau = tau_map[pixel].  With iso = 1 a map is
+// shared by every plane (the block threshold scales all planes of a pixel by one factor), so one thread still owns one
+// pixel; the backward adds that pixel's tau gradient into taubar_map[pixel] (one writer per launch: deterministic).
+__global__ void k_iso_prox_map(const float* __restrict__ x, const float* __restrict__ qxp, const float* __restrict__ qyp,
+                               const float* __restrict__ n_prev, float* __restrict__ qxn, float* __restrict__ qyn,
+                               float* __restrict__ n_new, float* __restrict__ c_new, const float* __restrict__ tau_map,
+                               int P, int H, int W) {
+    const int idx = blockIdx.x * blockDim.x + threadIdx.x;
+    if (idx >= H * W) return;
+    const int r = idx / W, c = idx - r * W;
+    const int cl = c == 0 ? W - 1 : c - 1, ru = r == 0 ? H - 1 : r - 1;
+    const float tau = tau_map[idx];
+    float ux_scale = 0.f, uy_scale = 0.f;
+    if (n_prev) {
+        ux_scale = 1.f - iso_scale(n_prev[idx], tau);
+        uy_scale = 1.f - iso_scale(n_prev[(size_t)H * W + idx], tau);
+    }
+    float sx = 0.f, sy = 0.f;
+    const size_t HW = (size_t)H * W;
+    for (int p = 0; p < P; ++p) {
+        const float* X = x + p * HW;
+        const float xc = X[idx];
+        float qx = xc - X[(size_t)r * W + cl];
+        float qy = xc - X[(size_t)ru * W + c];
+        if (n_prev) {
+            qx += ux_scale * qxp[p * HW + idx];
+            qy += uy_scale * qyp[p * HW + idx];
+        }
+        qxn[p * HW + idx] = qx; qyn[p * HW + idx] = qy;
+        sx = fmaf(qx, qx, sx); sy = fmaf(qy, qy, sy);
+    }
+    const float nx = sqrtf(sx + iso_eps<float>()), ny = sqrtf(sy + iso_eps<float>());
+    n_new[idx] = nx;
+    n_new[HW + idx] = ny;
+    if (c_new) {
+        c_new[idx] = 2.f * iso_scale(nx, tau) - 1.f;
+        c_new[HW + idx] = 2.f * iso_scale(ny, tau) - 1.f;
+    }
+}
+
+__global__ void k_iso_cmap_map(const float* __restrict__ nmap, float* __restrict__ cmap, const float* __restrict__ tau_map,
+                               int HW) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= 2 * HW) return;
+    cmap[i] = 2.f * iso_scale(nmap[i], tau_map[i < HW ? i : i - HW]) - 1.f;
+}
+
+template <bool HAS_U>
+__global__ void __launch_bounds__(32 * kIsoPG)
+k_iso_bwd_map(const float* __restrict__ vb, const float* __restrict__ ubx_in, const float* __restrict__ uby_in,
+              const float* __restrict__ qx, const float* __restrict__ qy, const float* __restrict__ nmap,
+              float* __restrict__ ubx_out, float* __restrict__ uby_out, const float* __restrict__ tau_map,
+              double* __restrict__ taubar_map, int P, int H, int W) {
+    __shared__ float red[kIsoPG][2][32];
+    const int tx = threadIdx.x & 31, g = threadIdx.x >> 5;
+    const size_t HW = (size_t)H * W;
+    const size_t idx = (size_t)blockIdx.x * 32 + tx;
+    const bool ok = idx < HW;
+    size_t ol = 0, ou = 0;
+    if (ok) {
+        const int r = (int)(idx / W), c = (int)(idx - (size_t)r * W);
+        ol = (size_t)r * W + (c == 0 ? W - 1 : c - 1);
+        ou = (size_t)(r == 0 ? H - 1 : r - 1) * W + c;
+    }
+    float ax = 0.f, ay = 0.f;
+    if (ok) {
+#pragma unroll 4
+        for (int p = g; p < P; p += kIsoPG) {
+            const float* V = vb + p * HW;
+            const float v0 = V[idx];
+            const float wbx = v0 - V[ol], wby = v0 - V[ou];
+            const float ux = HAS_U ? ubx_in[p * HW + idx] : 0.f, uy = HAS_U ? uby_in[p * HW + idx] : 0.f;
+            ax = fmaf(2.f * wbx - ux, qx[p * HW + idx], ax);
+            ay = fmaf(2.f * wby - uy, qy[p * HW + idx], ay);
+        }
+    }
+    red[g][0][tx] = ax; red[g][1][tx] = ay;
+    __syncthreads();
+    if (!ok) return;
+    float sbx = 0.f, sby = 0.f;
+#pragma unroll
+    for (int i = 0; i < kIsoPG; ++i) { sbx += red[i][0][tx]; sby += red[i][1][tx]; }
+    const float tau = tau_map[idx];
+    const float nx = nmap[idx], ny = nmap[HW + idx];
+    const float sx = iso_scale(nx, tau), sy = iso_scale(ny, tau);
+    const float kx = (sx > 0.f) ? sbx * tau / ((nx + iso_eps<float>()) * (nx + iso_eps<float>()) * nx) : 0.f;
+    const float ky = (sy > 0.f) ? sby * tau / ((ny + iso_eps<float>()) * (ny + iso_eps<float>()) * ny) : 0.f;
+    if (g == 0) {
+        double t = 0.0;
+        if (sx > 0.f) t -= (double)sbx / (double)(nx + iso_eps<float>());
+        if (sy > 0.f) t -= (double)sby / (double)(ny + iso_eps<float>());
+        taubar_map[idx] += t;
+    }
+#pragma unroll 4
+    for (int p = g; p < P; p += kIsoPG) {
+        const float* V = vb + p * HW;
+        const float v0 = V[idx];
+        const float wbx = v0 - V[ol], wby = v0 - V[ou];
+        const float ux = HAS_U ? ubx_in[p * HW + idx] : 0.f, uy = HAS_U ? uby_in[p * HW + idx] : 0.f;
+        ubx_out[p * HW + idx] = fmaf(sx, 2.f * wbx - ux, ux - wbx) + kx * qx[p * HW + idx];
+        uby_out[p * HW + idx] = fmaf(sy, 2.f * wby - uy, uy - wby) + ky * qy[p * HW + idx];
+    }
+}
+
+int launch_iso_prox_map(const Geometry& g, const float* x, const float* qx_prev, const float* qy_prev, const float* n_prev,
+                        float* qx_new, float* qy_new, float* n_new, float* c_new, const float* tau_map, cudaStream_t st) {
+    ProfScope ps(PROF_OTHER, st);
+    const int n = g.H * g.W;
+    k_iso_prox_map<<<(unsigned)((n + 63) / 64), 64, 0, st>>>(x, qx_prev, qy_prev, n_prev, qx_new, qy_new, n_new, c_new, tau_map,
+                                                             g.P, g.H, g.W);
+    ADMM_CUDA_CHECK(cudaGetLastError());
+    return 0;
+}
+
+int launch_iso_cmap_map(const Geometry& g, const float* nmap, float* cmap, const float* tau_map, cudaStream_t st) {
+    ProfScope ps(PROF_OTHER, st);
+    const int n = g.H * g.W;
+    k_iso_cmap_map<<<(2 * n + 255) / 256, 256, 0, st>>>(nmap, cmap, tau_map, n);
+    ADMM_CUDA_CHECK(cudaGetLastError());
+    return 0;
+}
+
+int launch_iso_bwd_map(const Geometry& g, const float* vb, const float* ubx_in, const float* uby_in, const float* qx,
+                       const float* qy, const float* nmap, float* ubx_out, float* uby_out, float* xb, const float* tau_map,
+                       double* taubar_map, cudaStream_t st) {
+    ProfScope ps(PROF_OTHER, st);
+    const size_t total = (size_t)g.P * g.H * g.W;
+    const unsigned nb = (unsigned)(((size_t)g.H * g.W + 31) / 32);
+    if (ubx_in && uby_in)
+        k_iso_bwd_map<true><<<nb, 32 * kIsoPG, 0, st>>>(vb, ubx_in, uby_in, qx, qy, nmap, ubx_out, uby_out, tau_map, taubar_map,
+                                                        g.P, g.H, g.W);
+    else
+        k_iso_bwd_map<false><<<nb, 32 * kIsoPG, 0, st>>>(vb, nullptr, nullptr, qx, qy, nmap, ubx_out, uby_out, tau_map, taubar_map,
+                                                         g.P, g.H, g.W);
+    ADMM_CUDA_CHECK(cudaGetLastError());
+    if (xb) {
+        k_div_adjoint<<<ew_grid(total), 256, 0, st>>>(ubx_out, uby_out, xb, g.H, g.W, total);
+        ADMM_CUDA_CHECK(cudaGetLastError());
+    }
+    return 0;
+}
+
 // float (the solver) and double (the float64 solve, f64.cu) entry points
 #define ADMM_ISO_LAUNCHERS(T)                                                                                              \
     int launch_iso_prox(const Geometry& g, const T* x, const T* qx_prev, const T* qy_prev, const T* n_prev, T* qx_new,     \

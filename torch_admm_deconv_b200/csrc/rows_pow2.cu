@@ -15,8 +15,15 @@
 
 namespace admm {
 
+// the marching modes: ROWS_FULL, ROWS_FULL_U, ROWS_ADJ and their threshold-map variants (one halo row above and below)
+template <int MODE> constexpr bool kRowsIter = (MODE == ROWS_FULL || MODE == ROWS_FULL_U || MODE == ROWS_ADJ ||
+                                                MODE == ROWS_FULL_MAP || MODE == ROWS_ADJ_MAP);
+// CTAs per SM the kernel is built for: 4, the adjoint ROWS_ADJ_OCC; the map modes carry the map's values on top of the
+// state and are built for 3 (no spills)
+template <int MODE> constexpr int kRowsOcc = (MODE == ROWS_ADJ) ? ROWS_ADJ_OCC : (MODE == ROWS_FULL_MAP || MODE == ROWS_ADJ_MAP) ? 3 : 4;
+
 template <int W, int MODE, int HT>
-__global__ void __launch_bounds__(256, MODE == ROWS_ADJ ? ROWS_ADJ_OCC : 4)
+__global__ void __launch_bounds__(256, kRowsOcc<MODE>)
 k_rows_pow2(RowArgs a, int H, int nbands, int pdl) {
     extern __shared__ float2 smem[];
     rows_pow2_body<W, MODE, false, HT>(a, H, nbands, pdl, blockIdx.x, smem);
@@ -27,7 +34,7 @@ k_rows_pow2(RowArgs a, int H, int nbands, int pdl) {
 template <int W, int MODE, int HT>
 static int launch_rows_pow2_h(const Geometry& g, const RowArgs& a, cudaStream_t st) {
     using S = RowSmem<W>;
-    constexpr int rmax = (MODE == ROWS_FULL || MODE == ROWS_FULL_U || MODE == ROWS_ADJ) ? S::RMAX : 2 * S::NPAIR;
+    constexpr int rmax = kRowsIter<MODE> ? S::RMAX : 2 * S::NPAIR;
     int nbands = (g.H + rmax - 1) / rmax;
     // few planes (latency-bound problems such as a single image): cut thinner bands so that every SM gets a CTA
     const int want = (2 * 148 + g.P - 1) / g.P;
@@ -36,8 +43,8 @@ static int launch_rows_pow2_h(const Geometry& g, const RowArgs& a, cudaStream_t 
         // wave balance (rows_per_band = -1 switches it off): with a few hundred to a few thousand CTAs the last, partly
         // filled wave costs as much as a full one; thinner bands (more CTAs, one more halo pair each in the marching
         // modes) can fill it.  Model: waves x (rows per band + halo).
-        constexpr int halo = (MODE == ROWS_FULL || MODE == ROWS_FULL_U || MODE == ROWS_ADJ) ? 2 : 0;
-        const long slots = 148L * (MODE == ROWS_ADJ ? ROWS_ADJ_OCC : 4);
+        constexpr int halo = kRowsIter<MODE> ? 2 : 0;
+        const long slots = 148L * kRowsOcc<MODE>;
         auto cost = [&](int nb) { return ((long)nb * g.P + slots - 1) / slots * ((g.H + nb - 1) / nb + halo); };
         int best = nbands;
         for (int nb = nbands + 1; nb <= std::min(g.H / 2, 2 * nbands); ++nb)
@@ -55,7 +62,7 @@ static int launch_rows_pow2_h(const Geometry& g, const RowArgs& a, cudaStream_t 
         ADMM_CUDA_CHECK(cudaFuncSetAttribute(k_rows_pow2<W, MODE, HT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S::bytes));
         attr_set = true;
     }
-    ProfScope ps((MODE == ROWS_FULL || MODE == ROWS_FULL_U) ? PROF_ROWS : PROF_OTHER, st);
+    ProfScope ps((MODE == ROWS_FULL || MODE == ROWS_FULL_U || MODE == ROWS_FULL_MAP) ? PROF_ROWS : PROF_OTHER, st);
     // programmatic dependent launch pays off when a kernel is a wave or two (launch / drain latency dominates)
     const size_t nctas = (size_t)nbands * g.P;
     if (options().use_pdl && nctas <= 148 * 8) {
@@ -69,7 +76,7 @@ static int launch_rows_pow2_h(const Geometry& g, const RowArgs& a, cudaStream_t 
 
 template <int W, int MODE>
 static int launch_rows_pow2_m(const Geometry& g, const RowArgs& a, cudaStream_t st) {
-    constexpr bool iter = (MODE == ROWS_FULL || MODE == ROWS_FULL_U || MODE == ROWS_ADJ);
+    constexpr bool iter = kRowsIter<MODE>;
     if (iter && g.H == W) return launch_rows_pow2_h<W, MODE, (iter ? W : 0)>(g, a, st);
     return launch_rows_pow2_h<W, MODE, 0>(g, a, st);
 }
@@ -82,6 +89,8 @@ static int launch_rows_pow2_t(RowMode mode, const Geometry& g, const RowArgs& a,
         case ROWS_C2R: return launch_rows_pow2_m<W, ROWS_C2R>(g, a, st);
         case ROWS_ADJ: return launch_rows_pow2_m<W, ROWS_ADJ>(g, a, st);
         case ROWS_FULL_U: return launch_rows_pow2_m<W, ROWS_FULL_U>(g, a, st);
+        case ROWS_FULL_MAP: return launch_rows_pow2_m<W, ROWS_FULL_MAP>(g, a, st);
+        case ROWS_ADJ_MAP: return launch_rows_pow2_m<W, ROWS_ADJ_MAP>(g, a, st);
     }
     return fail(4, "rows_pow2: bad mode");
 }

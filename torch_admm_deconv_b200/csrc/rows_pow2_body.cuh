@@ -44,7 +44,8 @@ __device__ __forceinline__ void rows_pow2_body(const RowArgs& a, int H_dyn, int 
     float2* regX = smem;                                    // NPAIR regions
     // v pair m is written over x pair m+1 once every thread has loaded that pair (one barrier per march step),
     // so the divergence needs no second tile and four CTAs fit on an SM
-    float2* regV = (MODE == ROWS_FULL || MODE == ROWS_FULL_U || MODE == ROWS_ADJ) ? regX + REGION : regX;
+    float2* regV = (MODE == ROWS_FULL || MODE == ROWS_FULL_U || MODE == ROWS_ADJ || MODE == ROWS_FULL_MAP || MODE == ROWS_ADJ_MAP)
+                 ? regX + REGION : regX;
     float2* tabs = regX + NPAIR * REGION;
     float2* side = tabs + S::TAB_END;
     const RowMapObj map;
@@ -59,9 +60,10 @@ __device__ __forceinline__ void rows_pow2_body(const RowArgs& a, int H_dyn, int 
     const int r0 = 2 * ((band * hh) / nbands);
     const int r1 = 2 * (((band + 1) * hh) / nbands);
     const int Rb = r1 - r0;                   // even, <= RMAX (FULL) or 2*NPAIR (plain modes)
-    constexpr bool kFull = (MODE == ROWS_FULL || MODE == ROWS_FULL_U);
+    constexpr bool kFull = (MODE == ROWS_FULL || MODE == ROWS_FULL_U || MODE == ROWS_FULL_MAP);
     constexpr bool kStateU = (MODE == ROWS_FULL_U);
-    constexpr bool kHalo = (kFull || MODE == ROWS_ADJ);
+    constexpr bool kMap = (MODE == ROWS_FULL_MAP || MODE == ROWS_ADJ_MAP);   // tau per pixel from a.cmap (DESIGN section 11)
+    constexpr bool kHalo = (kFull || MODE == ROWS_ADJ || MODE == ROWS_ADJ_MAP);
     const int npx = kHalo ? Rb / 2 + 1 : Rb / 2;   // x pairs (halo modes: rows r0-1 .. r0+Rb)
     const int npv = Rb / 2;                   // v pairs (rows r0 .. r0+Rb-1)
     const int rowbase = kHalo ? r0 - 1 : r0;
@@ -248,7 +250,7 @@ __device__ __forceinline__ void rows_pow2_body(const RowArgs& a, int H_dyn, int 
         const int g = tid / CP;
         const int c = 2 * (tid % CP);
         const int m_lo = (g * npv) / NG, m_hi = ((g + 1) * npv) / NG;
-        const float tau = __ldg(a.lmbd) / __ldg(a.rho);                 // deconv.py:44
+        const float tau = kMap ? 0.f : __ldg(a.lmbd) / __ldg(a.rho);   // deconv.py:44 (maps: read per pixel below)
         const bool have_q = (a.qx_in != nullptr);
         const float* __restrict__ qxi = a.qx_in + plane_real + c;
         const float* __restrict__ qyi = a.qy_in + plane_real + c;
@@ -364,7 +366,68 @@ __device__ __forceinline__ void rows_pow2_body(const RowArgs& a, int H_dyn, int 
                 qy0 = qyc0; qy1 = qyc1; wy0 = wyc0; wy1 = wyc1;
             }
         };
-        if (tau < 0.f) march(TauNeg{}); else march(TauPos{});
+        // the march with a threshold map: tau of every element read from the map (rows a, b at columns c, c+1, c+2 and
+        // the row below at c, c+1; a shared map stays in L2), the dual per element with dual_any (the sign varies)
+        auto march_map = [&]() {
+            const float* __restrict__ tm = a.cmap + (a.tau_map_planes > 1 ? plane_real : 0) + c;
+            auto du = [](float q_, float t_) { return dual_any(q_, t_); };
+            auto wf = [](float q_, float t_) { return fmaf(-2.0f, dual_any(q_, t_), q_); };
+            const float2* X = regX + m_lo * REGION;
+            float2 Pl = baseL[0], P0 = X[pc], P1 = X[pc1], P2 = baseR[0];
+            __syncthreads();
+            float qy0 = 0.f, qy1 = 0.f, wy0 = 0.f, wy1 = 0.f;
+            if (m_lo < m_hi) {
+                const float2 t0_ = ldg_f2(tm + (size_t)(r0 + 2 * m_lo) * W);
+                qy0 = P0.y - P0.x + du(qya.x, t0_.x);
+                qy1 = P1.y - P1.x + du(qya.y, t0_.y);
+                wy0 = wf(qy0, t0_.x); wy1 = wf(qy1, t0_.y);
+            }
+            for (int it = 0; it < steps; ++it) {
+                const int m = m_lo + it;
+                if (m >= m_hi) break;
+                const QRegs q = q0;
+                q0 = q1;
+                if (have_q && m + 2 < m_hi) load_q(m + 2, q1);
+                X += REGION;
+                const float2 Nl = baseL[(it + 1) * strideL], N0 = X[pc], N1 = X[pc1], N2 = baseR[(it + 1) * strideR];
+                __syncwarp();
+                const int ra = r0 + 2 * m;
+                int rc = ra + 2; if (rc >= H) rc -= H;
+                const float* ta_ = tm + (size_t)ra * W;
+                const float2 ta = ldg_f2(ta_), tb = ldg_f2(ta_ + W), tc = ldg_f2(tm + (size_t)rc * W);
+                const float ta2 = ldg_f(ta_ + c2), tb2 = ldg_f(ta_ + W + c2);
+                const float qxa0 = P0.y - Pl.y + du(q.qxa.x, ta.x);
+                const float qxa1 = P1.y - P0.y + du(q.qxa.y, ta.y);
+                const float qxa2 = P2.y - P1.y + du(q.qxa2, ta2);
+                const float wxa0 = wf(qxa0, ta.x), wxa1 = wf(qxa1, ta.y), wxa2 = wf(qxa2, ta2);
+                const float qyb0 = N0.x - P0.y + du(q.qyb.x, tb.x);
+                const float qyb1 = N1.x - P1.y + du(q.qyb.y, tb.y);
+                const float wyb0 = wf(qyb0, tb.x), wyb1 = wf(qyb1, tb.y);
+                const float qxb0 = N0.x - Nl.x + du(q.qxb.x, tb.x);
+                const float qxb1 = N1.x - N0.x + du(q.qxb.y, tb.y);
+                const float qxb2 = N2.x - N1.x + du(q.qxb2, tb2);
+                const float wxb0 = wf(qxb0, tb.x), wxb1 = wf(qxb1, tb.y), wxb2 = wf(qxb2, tb2);
+                const float qyc0 = N0.y - N0.x + du(q.qyc.x, tc.x);
+                const float qyc1 = N1.y - N1.x + du(q.qyc.y, tc.y);
+                const float wyc0 = wf(qyc0, tc.x), wyc1 = wf(qyc1, tc.y);
+                const float va0 = wxa0 - wxa1 + wy0 - wyb0;
+                const float va1 = wxa1 - wxa2 + wy1 - wyb1;
+                const float vb0 = wxb0 - wxb1 + wyb0 - wyc0;
+                const float vb1 = wxb1 - wxb2 + wyb1 - wyc1;
+                const size_t oa = (size_t)ra * W;
+                *reinterpret_cast<float2*>(qxo + oa) = make_float2(qxa0, qxa1);
+                *reinterpret_cast<float2*>(qyo + oa) = make_float2(qy0, qy1);
+                *reinterpret_cast<float2*>(qxo + oa + W) = make_float2(qxb0, qxb1);
+                *reinterpret_cast<float2*>(qyo + oa + W) = make_float2(qyb0, qyb1);
+                float2* V = regV + m * REGION;
+                V[pc] = make_float2(va0, vb0);
+                V[pc1] = make_float2(va1, vb1);
+                Pl = Nl; P0 = N0; P1 = N1; P2 = N2;
+                qy0 = qyc0; qy1 = qyc1; wy0 = wyc0; wy1 = wyc1;
+            }
+        };
+        if constexpr (kMap) march_map();
+        else if (tau < 0.f) march(TauNeg{}); else march(TauPos{});
     }
     // ------------------------------------------------------------------ backward: adjoint of prox / dual / gradient
     // qbar = wbar + 1[|q| < tau] (ubar - 2 wbar) with wbar = D vbar;  xbar = D^T qbar;  new ubar = qbar;
@@ -489,6 +552,95 @@ __device__ __forceinline__ void rows_pow2_body(const RowArgs& a, int H_dyn, int 
             a.taubar[bid] += s;
         }
     }
+    // the adjoint with a threshold map: masks per element, and each element's tau gradient (its x and y terms) added into
+    // a.taubar[plane element] (double, one writer per element and launch: deterministic)
+    if constexpr (MODE == ROWS_ADJ_MAP) {
+        constexpr int CP = W / 2;
+        constexpr int NG = S::kThreads / CP;
+        const int g = tid / CP;
+        const int c = 2 * (tid % CP);
+        const int m_lo = (g * npv) / NG, m_hi = ((g + 1) * npv) / NG;
+        const bool have_u = (a.ubx_in != nullptr);
+        const float* __restrict__ uxi = a.ubx_in + plane_real + c;
+        const float* __restrict__ uyi = a.uby_in + plane_real + c;
+        const float* __restrict__ qxs = a.qx_in + plane_real + c;
+        const float* __restrict__ qys = a.qy_in + plane_real + c;
+        const float* __restrict__ tm = a.cmap + (a.tau_map_planes > 1 ? plane_real : 0) + c;
+        float* __restrict__ uxo = a.ubx_out + plane_real + c;
+        float* __restrict__ uyo = a.uby_out + plane_real + c;
+        double* __restrict__ tbo = a.taubar + plane_real + c;
+        const int c2 = (c + 2 == W) ? (2 - W) : 2;
+        const int cl = (c == 0) ? W - 1 : c - 1;
+        const int pl = map.at(cl), pc = map.at(c), pr2 = map.at((c + 2) & (W - 1));
+        const int pc1 = pc + 1;
+        auto ld2 = [&](const float* p_, bool ok) { return ok ? ldg_f2(p_) : make_float2(0.f, 0.f); };
+        auto qbar = [](float wb, float ub, float q, float t) { return (fabsf(q) < t) ? (ub - wb) : wb; };
+        auto tterm = [](float wb, float ub, float q, float t) {
+            return (fabsf(q) >= t) ? (ub - 2.f * wb) * (q > 0.f ? 1.f : (q < 0.f ? -1.f : 0.f)) : 0.f;
+        };
+        float2 tya = make_float2(0.f, 0.f);                        // y terms of row a, carried from the row above
+        float qby0 = 0.f, qby1 = 0.f;
+        __syncthreads();                                             // vbar rows of every pair are in shared memory
+        const float2* X = regX + m_lo * REGION;
+        float2 Pl = X[pl], P0 = X[pc], P1 = X[pc1], P2 = X[pr2];
+        if (m_lo < m_hi) {
+            const size_t o0 = (size_t)(r0 + 2 * m_lo) * W;
+            const float2 qya = ldg_f2(qys + o0), uya = ld2(uyi + o0, have_u), t0_ = ldg_f2(tm + o0);
+            qby0 = qbar(P0.y - P0.x, uya.x, qya.x, t0_.x);
+            qby1 = qbar(P1.y - P1.x, uya.y, qya.y, t0_.y);
+            tya = make_float2(tterm(P0.y - P0.x, uya.x, qya.x, t0_.x), tterm(P1.y - P1.x, uya.y, qya.y, t0_.y));
+        }
+        const int steps = (npv + NG - 1) / NG;
+        for (int it = 0; it < steps; ++it) {
+            const int m = m_lo + it;
+            const bool active = (m < m_hi);
+            X += REGION;
+            float2 Nl = Pl, N0 = P0, N1 = P1, N2 = P2;
+            if (active) { Nl = X[pl]; N0 = X[pc]; N1 = X[pc1]; N2 = X[pr2]; }
+            __syncthreads();                                         // every thread holds pair m+1 in registers
+            if (!active) continue;
+            const int ra = r0 + 2 * m;
+            int rc = ra + 2; if (rc >= H) rc -= H;
+            const size_t oa = (size_t)ra * W, oc = (size_t)rc * W;
+            const float2 qxa = ldg_f2(qxs + oa), qxb = ldg_f2(qxs + oa + W), qyb = ldg_f2(qys + oa + W), qyc = ldg_f2(qys + oc);
+            const float qxa2 = ldg_f(qxs + oa + c2), qxb2 = ldg_f(qxs + oa + W + c2);
+            const float2 uxa = ld2(uxi + oa, have_u), uxb = ld2(uxi + oa + W, have_u);
+            const float2 uyb = ld2(uyi + oa + W, have_u), uyc = ld2(uyi + oc, have_u);
+            const float uxa2 = have_u ? ldg_f(uxi + oa + c2) : 0.f, uxb2 = have_u ? ldg_f(uxi + oa + W + c2) : 0.f;
+            const float2 ta = ldg_f2(tm + oa), tb = ldg_f2(tm + oa + W), tc = ldg_f2(tm + oc);
+            const float ta2 = ldg_f(tm + oa + c2), tb2 = ldg_f(tm + oa + W + c2);
+            // row a: vbar = P.y
+            const float wxa0 = P0.y - Pl.y, wxa1 = P1.y - P0.y, wxa2 = P2.y - P1.y;
+            const float bxa0 = qbar(wxa0, uxa.x, qxa.x, ta.x), bxa1 = qbar(wxa1, uxa.y, qxa.y, ta.y), bxa2 = qbar(wxa2, uxa2, qxa2, ta2);
+            const double ga0 = (double)tterm(wxa0, uxa.x, qxa.x, ta.x) + (double)tya.x;
+            const double ga1 = (double)tterm(wxa1, uxa.y, qxa.y, ta.y) + (double)tya.y;
+            // row b: vbar = N.x
+            const float wyb0 = N0.x - P0.y, wyb1 = N1.x - P1.y;
+            const float byb0 = qbar(wyb0, uyb.x, qyb.x, tb.x), byb1 = qbar(wyb1, uyb.y, qyb.y, tb.y);
+            const float wxb0 = N0.x - Nl.x, wxb1 = N1.x - N0.x, wxb2 = N2.x - N1.x;
+            const float bxb0 = qbar(wxb0, uxb.x, qxb.x, tb.x), bxb1 = qbar(wxb1, uxb.y, qxb.y, tb.y), bxb2 = qbar(wxb2, uxb2, qxb2, tb2);
+            const double gb0 = (double)tterm(wyb0, uyb.x, qyb.x, tb.x) + (double)tterm(wxb0, uxb.x, qxb.x, tb.x);
+            const double gb1 = (double)tterm(wyb1, uyb.y, qyb.y, tb.y) + (double)tterm(wxb1, uxb.y, qxb.y, tb.y);
+            // row below b: vbar = N.y; its y terms belong to row a of the next pair (the next group's first row is its own)
+            const float wyc0 = N0.y - N0.x, wyc1 = N1.y - N1.x;
+            const float byc0 = qbar(wyc0, uyc.x, qyc.x, tc.x), byc1 = qbar(wyc1, uyc.y, qyc.y, tc.y);
+            tya = (m + 1 < m_hi) ? make_float2(tterm(wyc0, uyc.x, qyc.x, tc.x), tterm(wyc1, uyc.y, qyc.y, tc.y)) : make_float2(0.f, 0.f);
+            const float xa0 = bxa0 - bxa1 + qby0 - byb0;
+            const float xa1 = bxa1 - bxa2 + qby1 - byb1;
+            const float xb0 = bxb0 - bxb1 + byb0 - byc0;
+            const float xb1 = bxb1 - bxb2 + byb1 - byc1;
+            *reinterpret_cast<float2*>(uxo + oa) = make_float2(bxa0, bxa1);
+            *reinterpret_cast<float2*>(uyo + oa) = make_float2(qby0, qby1);
+            *reinterpret_cast<float2*>(uxo + oa + W) = make_float2(bxb0, bxb1);
+            *reinterpret_cast<float2*>(uyo + oa + W) = make_float2(byb0, byb1);
+            tbo[oa] += ga0; tbo[oa + 1] += ga1; tbo[oa + W] += gb0; tbo[oa + W + 1] += gb1;
+            float2* V = regV + m * REGION;
+            V[pc] = make_float2(xa0, xb0);
+            V[pc1] = make_float2(xa1, xb1);
+            Pl = Nl; P0 = N0; P1 = N1; P2 = N2;
+            qby0 = byc0; qby1 = byc1;
+        }
+    }
     __syncthreads();
     ROWS_ST(3);
 
@@ -555,7 +707,7 @@ __device__ __forceinline__ void rows_pow2_body(const RowArgs& a, int H_dyn, int 
                st[3] - st[2], st[4] - st[3], st[4] - st[0]);
 #endif
 
-    if (MODE == ROWS_ADJ) {
+    if (MODE == ROWS_ADJ || MODE == ROWS_ADJ_MAP) {
         // optional second output: v_k = D^T w(q_k) recomputed from the saved pre-clamp state, and its row spectrum
         if (a.qvx != nullptr) {
             constexpr int CP = W / 2;
@@ -563,7 +715,9 @@ __device__ __forceinline__ void rows_pow2_body(const RowArgs& a, int H_dyn, int 
             const int g = tid / CP;
             const int c = 2 * (tid % CP);
             const int m_lo = (g * npv) / NG, m_hi = ((g + 1) * npv) / NG;
-            const float tau = __ldg(a.lmbd) / __ldg(a.rho);
+            const float tau = kMap ? 0.f : __ldg(a.lmbd) / __ldg(a.rho);
+            const float* __restrict__ tm = kMap ? a.cmap + (a.tau_map_planes > 1 ? plane_real : 0) + c : nullptr;
+            (void)tm;
             const float* __restrict__ qx = a.qvx + plane_real + c;
             const float* __restrict__ qy = a.qvy + plane_real + c;
             const int c2 = (c + 2 == W) ? (2 - W) : 2;
@@ -577,6 +731,19 @@ __device__ __forceinline__ void rows_pow2_body(const RowArgs& a, int H_dyn, int 
                 const float xa2 = ldg_f(xa + c2), xb2 = ldg_f(xa + W + c2);
                 const float2 ya = ldg_f2(qy + (size_t)ra * W), yb = ldg_f2(qy + (size_t)ra * W + W), yc = ldg_f2(qy + (size_t)rc * W);
                 auto wfun2 = [](float q_, float tau_) { return fmaf(-2.0f, dual_any(q_, tau_), q_); };
+                if constexpr (kMap) {
+                    // the threshold of each element from the map: rows a, b at columns c, c+1, c+2 and the row below
+                    const float* t_ = tm + (size_t)ra * W;
+                    const float2 ta = ldg_f2(t_), tb = ldg_f2(t_ + W), tc = ldg_f2(tm + (size_t)rc * W);
+                    const float ta2 = ldg_f(t_ + c2), tb2 = ldg_f(t_ + W + c2);
+                    const float wxa0 = wfun2(xa01.x, ta.x), wxa1 = wfun2(xa01.y, ta.y), wxa2 = wfun2(xa2, ta2);
+                    const float wxb0 = wfun2(xb01.x, tb.x), wxb1 = wfun2(xb01.y, tb.y), wxb2 = wfun2(xb2, tb2);
+                    const float wya0 = wfun2(ya.x, ta.x), wya1 = wfun2(ya.y, ta.y);
+                    const float wyb0 = wfun2(yb.x, tb.x), wyb1 = wfun2(yb.y, tb.y);
+                    const float wyc0 = wfun2(yc.x, tc.x), wyc1 = wfun2(yc.y, tc.y);
+                    regX[m * REGION + pc] = make_float2(wxa0 - wxa1 + wya0 - wyb0, wxb0 - wxb1 + wyb0 - wyc0);
+                    regX[m * REGION + pc + 1] = make_float2(wxa1 - wxa2 + wya1 - wyb1, wxb1 - wxb2 + wyb1 - wyc1);
+                } else {
                 const float wxa0 = wfun2(xa01.x, tau), wxa1 = wfun2(xa01.y, tau), wxa2 = wfun2(xa2, tau);
                 const float wxb0 = wfun2(xb01.x, tau), wxb1 = wfun2(xb01.y, tau), wxb2 = wfun2(xb2, tau);
                 const float wya0 = wfun2(ya.x, tau), wya1 = wfun2(ya.y, tau);
@@ -584,6 +751,7 @@ __device__ __forceinline__ void rows_pow2_body(const RowArgs& a, int H_dyn, int 
                 const float wyc0 = wfun2(yc.x, tau), wyc1 = wfun2(yc.y, tau);
                 regX[m * REGION + pc] = make_float2(wxa0 - wxa1 + wya0 - wyb0, wxb0 - wxb1 + wyb0 - wyc0);
                 regX[m * REGION + pc + 1] = make_float2(wxa1 - wxa2 + wya1 - wyb1, wxb1 - wxb2 + wyb1 - wyc1);
+                }
             }
             __syncthreads();
             r2c(regX, a.spec_out2 + plane_spec);

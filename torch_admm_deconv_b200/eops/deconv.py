@@ -94,6 +94,45 @@ def _scalar_param(v, device, name):
     return v
 
 
+def _is_map(lmbd) -> bool:
+    """A `lmbd` that is a tensor of more than one element: a regularisation map (DESIGN.md section 11)."""
+    return torch.is_tensor(lmbd) and lmbd.numel() != 1
+
+
+def _tau_map(lmbd: torch.Tensor, rho, shape, iso: bool, device):
+    """tau = lmbd / rho for a λ map, as the reference forms it (deconv.py:44) and applies it element by element.
+
+    `lmbd` is a float tensor whose shape broadcasts to `shape` = (B, C, H, W); `rho` holds one element (it enters the
+    Fourier-domain denominator, so a ρ map is not possible).  The division runs in float32 and is tracked by autograd, so
+    the gradient the solve returns for tau reaches λ and ρ through it, summed over broadcast dimensions.  Returns
+    (tau, planes): a contiguous (1, 1, H, W) map when λ is constant over B and C (planes = 1), else the expanded
+    (B, C, H, W) map (planes = B*C).  iso=True takes the first form only: the block threshold scales every plane of a
+    pixel by one factor.  Raises ValueError before anything runs on the GPU."""
+    B, C, H, W = (int(v) for v in shape)
+    if not lmbd.is_floating_point():
+        raise ValueError("a lmbd map must be a floating-point tensor, got %s" % lmbd.dtype)
+    if torch.is_tensor(rho) and rho.numel() != 1:
+        raise ValueError("rho must hold exactly one element, got shape %s: it enters the Fourier-domain denominator, so "
+                         "a rho map is not possible (pass a lmbd map instead)" % (tuple(rho.shape),))
+    if lmbd.dim() > 4:
+        raise ValueError("lmbd of shape %s does not broadcast to the image shape %s" % (tuple(lmbd.shape), (B, C, H, W)))
+    lshape = (1,) * (4 - lmbd.dim()) + tuple(lmbd.shape)
+    if any(l not in (1, n) for l, n in zip(lshape, (B, C, H, W))):
+        raise ValueError("lmbd of shape %s does not broadcast to the image shape %s" % (tuple(lmbd.shape), (B, C, H, W)))
+    shared = lshape[0] == 1 and lshape[1] == 1
+    if iso and not shared:
+        raise ValueError("iso=True takes a lmbd map that is constant over batch and channel (shape (1, 1, H, W) or "
+                         "smaller), got %s: the block threshold scales every plane of a pixel by one factor"
+                         % (tuple(lmbd.shape),))
+    # a Python rho is uploaded once per value and cached (_scalar_param): no copy per call, and CUDA-graph capture works
+    rho_t = _scalar_param(rho, device, "rho").to(device=device, dtype=torch.float32).reshape(())
+    tau = lmbd.to(device=device, dtype=torch.float32).reshape(lshape) / rho_t
+    tau = tau.expand((1, 1, H, W) if shared else (B, C, H, W)).contiguous()
+    if tau.data_ptr() % 16:                            # the library reads the map through 16-byte aligned pointers
+        tau = tau.clone()
+    return tau, (1 if shared else B * C)
+
+
 def _prep_kernel(kern: torch.Tensor):
     """Returns (ksize, contiguous fp32 (k,k) tensor or None).  Empty kernel = TV denoise (deconv.py:46,86)."""
     if kern is None or kern.numel() == 0:
@@ -140,13 +179,19 @@ def _act_grad(act: int, out: torch.Tensor, g: torch.Tensor) -> torch.Tensor:
 
 class _AdmmTV(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, xin, lmbd, rho, kern, bias, iso, maxit, need_grad, act, out_view, yhat=None, ckpt=0, resid=None):
+    def forward(ctx, xin, lmbd, rho, kern, bias, iso, maxit, need_grad, act, out_view, yhat=None, ckpt=0, resid=None,
+                tau_planes=0):
+        # tau_planes > 0: `lmbd` is a threshold map tau = lambda / rho, (tau_planes, H, W) contiguous float32 on xin's
+        # device (_tau_map); the backward returns its gradient and the gradient of rho at fixed tau
         lib = _lib.load()
         B, C, H, W = xin.shape
         dev = xin.device
         ksize = _prep_kernel(kern)
         x = xin.contiguous()
-        lam_d = lmbd.detach().to(device=dev, dtype=torch.float32, non_blocking=True).reshape(1).contiguous()
+        if tau_planes:
+            lam_d = lmbd.detach()
+        else:
+            lam_d = lmbd.detach().to(device=dev, dtype=torch.float32, non_blocking=True).reshape(1).contiguous()
         rho_d = rho.detach().to(device=dev, dtype=torch.float32, non_blocking=True).reshape(1).contiguous()
         kern_d = kern.detach().to(device=dev, dtype=torch.float32).contiguous() if ksize else None
         bias_d = bias.detach().to(device=dev, dtype=torch.float32).reshape(1).contiguous() if bias is not None else None
@@ -160,6 +205,9 @@ class _AdmmTV(torch.autograd.Function):
         ext.out_batch_stride = int(out.stride(0))
         if yhat is not None:                           # F(y) shared by several solvers on the same input (shared_spectrum)
             ext.yhat_in = yhat.data_ptr()
+        if tau_planes:
+            ext.tau_map = lam_d.data_ptr()
+            ext.tau_map_planes = int(tau_planes)
         with torch.cuda.device(dev):
             ws_bytes = lib.admm_query_workspace(B * C, H, W, ksize, int(iso), maxit)
             if ws_bytes == 0:
@@ -187,7 +235,8 @@ class _AdmmTV(torch.autograd.Function):
                     ext.host_flag = _host_flag(dev).data_ptr()
                 ext.iters_out = ctypes.addressof(resid.iters)
             stream = torch.cuda.current_stream(dev).cuda_stream
-            st = lib.admm_tv_forward_ex(_ptr(x), _ptr(out), _ptr(kern_d), ksize, _ptr(lam_d), _ptr(rho_d), _ptr(bias_d),
+            st = lib.admm_tv_forward_ex(_ptr(x), _ptr(out), _ptr(kern_d), ksize, _ptr(None if tau_planes else lam_d),
+                                        _ptr(rho_d), _ptr(bias_d),
                                         B, C, H, W, int(iso), maxit, _ptr(ws), ws.numel(),
                                         _ptr(saved), saved_bytes, ctypes.c_void_p(stream), ctypes.byref(ext))
             _lib.check(st, "admm_tv_forward_ex")
@@ -196,7 +245,7 @@ class _AdmmTV(torch.autograd.Function):
                                   out if act != _lib.ACT_NONE else x.new_empty(0, dtype=torch.float32))
             ctx.cfg = (ksize, bool(iso), int(maxit), bias is not None,
                        tuple(kern.shape) if kern is not None else (0,), tuple(lmbd.shape), tuple(rho.shape),
-                       tuple(bias.shape) if bias is not None else None, int(act), int(ckpt))
+                       tuple(bias.shape) if bias is not None else None, int(act), int(ckpt), int(tau_planes))
         return out
 
     @staticmethod
@@ -204,7 +253,7 @@ class _AdmmTV(torch.autograd.Function):
     def backward(ctx, grad_out):
         lib = _lib.load()
         x, lam_d, rho_d, kern_d, saved, out_saved = ctx.saved_tensors
-        ksize, iso, maxit, has_bias, kshape, lshape, rshape, bshape, act, ckpt = ctx.cfg
+        ksize, iso, maxit, has_bias, kshape, lshape, rshape, bshape, act, ckpt, tau_planes = ctx.cfg
         B, C, H, W = x.shape
         dev = x.device
         g = grad_out.to(torch.float32)
@@ -214,11 +263,22 @@ class _AdmmTV(torch.autograd.Function):
         need_x, need_l, need_r, need_k, need_b = ctx.needs_input_grad[:5]
         need_x = need_x and x.dtype == torch.float32
         gx = torch.empty_like(x) if need_x else None
-        gl = torch.zeros(1, dtype=torch.float32, device=dev) if need_l else None
+        gl = (torch.empty_like(lam_d) if tau_planes else torch.zeros(1, dtype=torch.float32, device=dev)) if need_l else None
         gr = torch.zeros(1, dtype=torch.float32, device=dev) if need_r else None
         gk = torch.zeros(ksize, ksize, dtype=torch.float32, device=dev) if (need_k and ksize) else None
         y = x if x.dtype == torch.float32 else x.to(torch.float32) / 255.0
         with torch.cuda.device(dev):
+            if tau_planes:
+                ws = _workspace(lib.admm_query_workspace_backward_map(B * C, H, W, ksize, int(iso), maxit, ckpt, tau_planes), dev)
+                st = lib.admm_tv_backward_map(_ptr(y), _ptr(g), _ptr(kern_d if ksize else None), ksize, _ptr(lam_d), tau_planes,
+                                              _ptr(rho_d), B, C, H, W, int(iso), maxit, _ptr(saved), saved.numel(),
+                                              _ptr(ws), ws.numel(), _ptr(gx), _ptr(gk), _ptr(gl), _ptr(gr),
+                                              ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream), ckpt)
+                _lib.check(st, "admm_tv_backward_map")
+                return (gx, gl, gr.reshape(rshape) if gr is not None else None,
+                        gk.reshape(kshape) if gk is not None else None,
+                        g.sum().reshape(bshape) if (has_bias and need_b) else None,
+                        None, None, None, None, None, None, None, None, None)
             ws_bytes = lib.admm_query_workspace_backward_ex(B * C, H, W, ksize, int(iso), maxit, ckpt)
             ws = _workspace(ws_bytes, dev)
             stream = torch.cuda.current_stream(dev).cuda_stream
@@ -232,7 +292,7 @@ class _AdmmTV(torch.autograd.Function):
                 gl.reshape(lshape) if gl is not None else None,
                 gr.reshape(rshape) if gr is not None else None,
                 gk.reshape(kshape) if gk is not None else None,
-                gb, None, None, None, None, None, None, None, None)
+                gb, None, None, None, None, None, None, None, None, None)
 
 
 def shared_spectrum(xin: torch.Tensor) -> Optional[torch.Tensor]:
@@ -309,7 +369,10 @@ def admm_solve(xin: torch.Tensor, lmbd, rho, kern, iso: bool = False, maxit: int
     `ckpt_interval` (training, iso=False): K >= 2 keeps the per-iteration state of every K-th iteration only and lets the
     backward re-run each block of K iterations from its checkpoint (about one extra forward): saved memory drops from
     maxit-1 to (maxit-1)//K + K-1 fields pairs -- 99 -> 19 for 100 iterations at K = 10 (cfg2: 38 GB -> 7.6 GB).
-    -1 picks K = ceil(sqrt(maxit - 1)).  0 keeps every iteration (stock-autograd-like memory, fastest backward)."""
+    -1 picks K = ceil(sqrt(maxit - 1)).  0 keeps every iteration (stock-autograd-like memory, fastest backward).
+
+    `lmbd` may be a λ map (a float tensor that broadcasts to xin's shape): tau = lmbd / rho is formed here in float32 under
+    autograd and the solve thresholds element by element (DESIGN.md section 11); `rho` stays one element."""
     ckpt_interval = int(ckpt_interval)
     if ckpt_interval < 0:
         ckpt_interval = int(math.ceil(math.sqrt(max(int(maxit) - 1, 1))))
@@ -324,7 +387,11 @@ def admm_solve(xin: torch.Tensor, lmbd, rho, kern, iso: bool = False, maxit: int
         raise TypeError("float32 inputs (or uint8 images, read as x / 255) are supported by the sm_100a kernels (got %s); "
                         "fft_admm_tv_cast is the explicit float32 shim for other floating dtypes" % xin.dtype)
     maxit = int(maxit)
-    lmbd = _scalar_param(lmbd, xin.device, "lmbd")
+    tau_planes = 0
+    if _is_map(lmbd):                                  # spatially varying regularisation: the solve takes tau = lmbd / rho
+        lmbd, tau_planes = _tau_map(lmbd, rho, xin.shape, bool(iso), xin.device)
+    else:
+        lmbd = _scalar_param(lmbd, xin.device, "lmbd")
     rho = _scalar_param(rho, xin.device, "rho")
     if kern is None:
         kern = xin.new_empty(0, dtype=torch.float32)
@@ -338,16 +405,19 @@ def admm_solve(xin: torch.Tensor, lmbd, rho, kern, iso: bool = False, maxit: int
     need_grad = torch.is_grad_enabled() and any(
         torch.is_tensor(t) and t.requires_grad for t in (xin, lmbd, rho, kern, bias))
     code = act if act is not None else _lib.ACT_NONE
-    if (SPLIT_STREAMS >= 2 and not need_grad and not iso and act is not None and yhat is None and xin.shape[0] >= 2
+    if (SPLIT_STREAMS >= 2 and not need_grad and not iso and not tau_planes and act is not None and yhat is None
+            and xin.shape[0] >= 2
             and xin.numel() >= SPLIT_MIN_ELEMENTS and maxit >= 2 and not torch.cuda.is_current_stream_capturing()):
         return _solve_split(xin, lmbd, rho, kern, bias, iso, maxit, code, out)
     if out is not None and (need_grad or act is None):
         # training, or an activation the kernels do not know: solve into a fresh tensor and let autograd track the copy
         # into the slice (plain torch semantics); inference with a known activation writes the slice directly
-        res = _AdmmTV.apply(xin, lmbd, rho, kern, bias, bool(iso), maxit, need_grad, code, None, yhat, ckpt_interval)
+        res = _AdmmTV.apply(xin, lmbd, rho, kern, bias, bool(iso), maxit, need_grad, code, None, yhat, ckpt_interval, None,
+                            tau_planes)
         out.copy_(res if act is not None else activation(res))
         return out
-    res = _AdmmTV.apply(xin, lmbd, rho, kern, bias, bool(iso), maxit, need_grad, code, out, yhat, ckpt_interval)
+    res = _AdmmTV.apply(xin, lmbd, rho, kern, bias, bool(iso), maxit, need_grad, code, out, yhat, ckpt_interval, None,
+                        tau_planes)
     return res if act is not None else activation(res)
 
 
@@ -412,6 +482,9 @@ def admm_solve_tol(xin: torch.Tensor, lmbd, rho, kern, iso: bool = False, maxit:
     rtol, atol, check_every, maxit = float(rtol), float(atol), int(check_every), int(maxit)
     if not (rtol >= 0 and atol >= 0):
         raise ValueError("rtol and atol must be >= 0 (got %r, %r)" % (rtol, atol))
+    if _is_map(lmbd):
+        raise ValueError("admm_solve_tol takes a scalar lmbd: the residual kernels have no lmbd map (got shape %s); "
+                         "admm_solve takes the map" % (tuple(lmbd.shape),))
     if check_every < 1:
         raise ValueError("check_every must be >= 1 (got %d)" % check_every)
     ckpt_interval = int(ckpt_interval)
@@ -468,7 +541,9 @@ def fft_admm_tv(xin: torch.Tensor,
     """ADMM total-variation deconvolution / denoising, drop-in for reference deconv.py:35-117.
 
     xin   (B, C, H, W) float32 CUDA tensor (blurred / noisy image batch)
-    lmbd  (1,) tensor, TV weight          rho (1,) tensor, ADMM penalty          tau = lmbd / rho
+    lmbd  (1,) tensor, TV weight, or a λ map: a float tensor that broadcasts to (B, C, H, W) (per pixel, per plane or
+          per element; iso=True: constant over B and C), applied element by element as in the reference
+    rho   (1,) tensor, ADMM penalty          tau = lmbd / rho
     kern  (1, 1, k, k) square PSF, or an empty tensor for pure TV denoising (deconv.py:46-47, 86-87)
     iso   False: anisotropic soft threshold; True: block threshold over (batch, channel) (deconv.py:19-24)
     maxit number of ADMM iterations; 0 returns zeros (deconv.py:61, 103, 117)
