@@ -476,9 +476,7 @@ def test_inference_map_solve(shape, opts, kind):
 
 
 # d. training ----------------------------------------------------------------------------------------------------------
-# (an odd-height generic frame such as 33 x 45 is left out: there the scalar solve's own checkpointed rho and kernel
-# gradients already differ from full-state training in the last bits, DESIGN.md section 11)
-@pytest.mark.parametrize("shape,k,maxit", [((2, 2, 256, 256), 5, 10), ((1, 1, 1080, 1920), 3, 7)],
+@pytest.mark.parametrize("shape,k,maxit", [((2, 2, 256, 256), 5, 10), ((1, 1, 1080, 1920), 3, 7), ((1, 2, 33, 45), 3, 10)],
                          ids=lambda v: "x".join(map(str, v)) if isinstance(v, tuple) else None)
 @pytest.mark.parametrize("kind", ["shared", "full"])
 def test_checkpointed_training_is_bit_identical(shape, k, maxit, kind):

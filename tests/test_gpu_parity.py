@@ -777,7 +777,11 @@ def test_maxit_zero_with_bias_returns_bias():
 
 
 @pytest.mark.parametrize("shape,k,maxit,K", [((2, 3, 64, 64), 5, 11, 3), ((1, 2, 128, 256), 0, 10, 4), ((2, 1, 60, 90), 3, 9, 2),
-                                             ((2, 2, 256, 256), 7, 26, -1), ((1, 1, 48, 40), 3, 7, 10)])
+                                             ((2, 2, 256, 256), 7, 26, -1), ((1, 1, 48, 40), 3, 7, 10),
+                                             # odd heights (generic rows, the last band's halo wraps to row 0); K = 6 of 7
+                                             # slots re-runs a one-slot block, K = 8 of 8 slots keeps only the last one
+                                             ((1, 2, 33, 45), 5, 10, 3), ((2, 3, 31, 37), 3, 9, -1), ((1, 1, 45, 63), 5, 8, 6),
+                                             ((1, 2, 33, 45), 3, 9, 8), ((1, 1, 45, 256), 5, 6, 2)])
 def test_checkpointed_training_matches_full_state(shape, k, maxit, K):
     """Memory-saving training (admm_ext.ckpt_interval): the forward keeps every K-th iteration's state, the backward re-runs
     each block from its checkpoint.  Gradients must equal those of the run that keeps every iteration and the saved buffer

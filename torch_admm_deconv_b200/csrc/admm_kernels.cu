@@ -127,17 +127,22 @@ __device__ __forceinline__ double act_out(double v, int) { return v; }
 
 // Two real rows <-> one complex FFT (z = row_a + i row_b).  Merge builds the full complex spectrum of z
 // from the two packed half spectra; split is the inverse.
-template <typename V>
+// WRAP (the halo bands of ROWS_FULL): a last pair without a partner row -- the bottom halo row 0 of the last band when H
+// is odd -- is merged as (row H-1, row 0) instead of (row 0, zero), the pair band 0 holds as its top halo, so that both
+// bands compute row 0 and row H-1 with the same bits.
+template <typename V, bool WRAP = false>
 __device__ __forceinline__ void merge_pairs(const V* __restrict__ S, int H, int W, int Wc, int BS,
                                             int rfirst, int nrows, int NP, V* __restrict__ buf) {
     using T = real_t<V>;
     const bool even = (W & 1) == 0;
     for (int w = threadIdx.x; w < NP * Wc; w += blockDim.x) {
         const int m = w / Wc, c = w - m * Wc;
-        int ra = rfirst + 2 * m; ra %= H; if (ra < 0) ra += H;
+        int ra = rfirst + 2 * m;
+        if constexpr (WRAP) { if (2 * m + 1 >= nrows) ra -= 1; }
+        ra %= H; if (ra < 0) ra += H;
         V a = S[(size_t)ra * Wc + c];
         V b = make_cplx(T(0), T(0));
-        if (2 * m + 1 < nrows) {
+        if (WRAP || 2 * m + 1 < nrows) {
             int rb = ra + 1; if (rb >= H) rb -= H;
             b = S[(size_t)rb * Wc + c];
         }
@@ -235,7 +240,7 @@ k_rows(RowArgsT<T> a, FftPlan plan, int H, int W, int Wc, int R, int BS, int nba
         // rows r0-1 .. r0+Rb  (Rb + 2 rows, circular), as pairs (i = 2m, 2m+1)
         const int nrows = Rb + 2;
         const int NP = (nrows + 1) / 2;
-        merge_pairs(a.spec_in + plane_spec, H, W, Wc, BS, r0 - 1, nrows, NP, bufA);
+        merge_pairs<V, true>(a.spec_in + plane_spec, H, W, Wc, BS, r0 - 1, nrows, NP, bufA);
         __syncthreads();
         V* res = fft_batched<+1>(bufA, bufB, plan, NP, BS, tw);
         V* zb = (res == bufA) ? bufB : bufA;
@@ -276,7 +281,8 @@ k_rows(RowArgsT<T> a, FftPlan plan, int H, int W, int Wc, int R, int BS, int nba
             const T qx_a  = xa_c - xa_l + uxa;                   // deconv.py:108,111,114
             const T qx_ar = xa_r - xa_c + uxar;
             const T qy_a  = xa_c - xu + uya;                     // deconv.py:109,112,115
-            const T qy_b  = xb_c - xa_c + uyb;
+            // no row ra+1 in the band (ra = H-1, H odd): q_y of row 0 from the pair (H-1, 0), as band 0 forms its qy_a
+            const T qy_b  = (hasb ? xb_c : P1c.y) - (hasb ? xa_c : P1c.x) + uyb;
             const T va = wfun(qx_a, tau) - wfun(qx_ar, tau) + wfun(qy_a, tau) - wfun(qy_b, tau);   // deconv.py:104
             qxo[(size_t)ra * W + c] = qx_a;
             qyo[(size_t)ra * W + c] = qy_a;
@@ -303,7 +309,7 @@ k_rows(RowArgsT<T> a, FftPlan plan, int H, int W, int Wc, int R, int BS, int nba
         // deconv.py:111-112 with a broadcast tensor lmbd).  The sign of tau varies inside a map: dual_any per element.
         const int nrows = Rb + 2;
         const int NP = (nrows + 1) / 2;
-        merge_pairs(a.spec_in + plane_spec, H, W, Wc, BS, r0 - 1, nrows, NP, bufA);
+        merge_pairs<V, true>(a.spec_in + plane_spec, H, W, Wc, BS, r0 - 1, nrows, NP, bufA);
         __syncthreads();
         V* res = fft_batched<+1>(bufA, bufB, plan, NP, BS, tw);
         V* zb = (res == bufA) ? bufB : bufA;
@@ -346,7 +352,7 @@ k_rows(RowArgsT<T> a, FftPlan plan, int H, int W, int Wc, int R, int BS, int nba
             const T qx_a  = xa_c - xa_l + uxa;
             const T qx_ar = xa_r - xa_c + uxar;
             const T qy_a  = xa_c - xu + uya;
-            const T qy_b  = xb_c - xa_c + uyb;
+            const T qy_b  = (hasb ? xb_c : P1c.y) - (hasb ? xa_c : P1c.x) + uyb;
             const T va = wfun(qx_a, t_ac) - wfun(qx_ar, t_ar) + wfun(qy_a, t_ac) - wfun(qy_b, t_bc);
             qxo[(size_t)ra * W + c] = qx_a;
             qyo[(size_t)ra * W + c] = qy_a;
